@@ -2,7 +2,7 @@
 """bench.py — Vamana search throughput on the BASELINE.json configs on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload c2|c3|c4|c5b|c5a] [--extra auto|none|c3,c5b,...]
+                    [--workload c2|c3|c4|c5b|c5a] [--extra auto|none|c3,c5b,...] [--dump-outputs DIR]
 
 The default line (what the driver runs) is C2, the config the metric is quoted on: a "step" is
 one pass of the hot path over one 10k-query batch — batched greedy beam search (K1) over a
@@ -35,6 +35,13 @@ NVLink + flag barrier) and the merge kernel (K6).
 Nothing on a timed GPU path touches oracle/: it builds the C2 graph during untimed input
 preparation ("searching the reference-built graph"), serves as the parity checker in the
 untimed tail and as the CPU baseline.
+
+--dump-outputs DIR writes what the headline's last timed step returned to its caller as DIR/<name>.npy
+(float32 / float64, under 64 MB in all: past that a seeded sample of rows, listed in rows.npy), for comparing
+two builds output for output. Every input of the timed path is the same in every run with the same
+arguments: points and queries are seeded, and the reference-built C2 graph is inserted on all host cores
+in rounds of at most ORACLE_ROUND points (OracleIndex.insert max_round), which make it independent of
+the core count and of thread timing. The bench writes nothing into the repository tree.
 """
 from __future__ import annotations
 
@@ -53,6 +60,10 @@ ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
 
 L, R, ALPHA, K = 75, 64, 1.2, 10
+# points per round of the reference-built graph: a few times the reference's concurrent workers in
+# flight, same recall and hop count as their graph at 100k points
+ORACLE_ROUND = 64
+DUMP_BYTES = 60_000_000  # array bytes of --dump-outputs: with the .npy headers, under 64 MB
 _OUT = sys.stdout
 _T0 = time.time()
 
@@ -83,6 +94,29 @@ PQ_WORKLOADS = ("c4", "c4cos")
 
 def log(*a):
     print(f"[{time.time() - _T0:7.1f}s]", *a, file=sys.stderr, flush=True)
+
+
+def dump_rows(n, row_bytes):
+    """Rows of an n-row output that --dump-outputs keeps: None (all of them) up to DUMP_BYTES,
+    else a fixed seeded sample, sized to leave room for its own float64 index."""
+    if n * row_bytes <= DUMP_BYTES:
+        return None
+    return np.sort(np.random.default_rng(0).choice(n, DUMP_BYTES // (row_bytes + 8), replace=False))
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each array (same number of rows, float32 / float64) as out_dir/<name>.npy; a sample
+    of rows (dump_rows) is listed in rows.npy."""
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    n = len(next(iter(arrays.values())))
+    keep = dump_rows(n, sum(a.nbytes for a in arrays.values()) // max(1, n))
+    if keep is not None:
+        arrays = {k: a[keep] for k, a in arrays.items()}
+        arrays["rows"] = keep.astype(np.float64)
+    for k, a in arrays.items():
+        np.save(out_dir / f"{k}.npy", np.ascontiguousarray(a))
+    log(f"outputs written to {out_dir}: " + ", ".join(f"{k} {a.shape} {a.dtype}" for k, a in arrays.items()))
 
 
 def measured_peaks():
@@ -198,7 +232,7 @@ def build_oracle_index(X, start, threads, dim=128, metric="euclidean"):
     oix.set_start(start)
     ids = np.arange(2, len(X) + 2, dtype=np.uint32)
     t = time.time()
-    oix.insert(ids, X, threads=threads)
+    oix.insert(ids, X, threads=threads, max_round=ORACLE_ROUND)
     return oix, ids, time.time() - t
 
 
@@ -669,6 +703,8 @@ def run_search(cx, name, n, B, steps, warmup, graph, headline):
         "parity": parity, "parity_merged": parity_merged, "oracle_recall": oracle_recall, "k_ids": k_ids, "k_d": k_d,
         "pq_fit": fit_cpu,
         "exchange": searcher.exchange, "searcher": searcher, "launch_queries": launch_queries, "pipelined": pipelined,
+        "outputs": {"ids": m_ids.cpu().numpy().astype(np.float64), "dists": m_d.cpu().numpy().astype(np.float32),
+                    "counts": m_c.cpu().numpy().astype(np.float32)} if headline else None,
     })
     return out
 
@@ -749,10 +785,12 @@ def run_flat(cx, g, Q, n, reps=7):
                          "note": "useful FLOP (2 x queries x points x dim) / whole call incl. copies, sample pass and re-score"}}
 
 
-def run_build(cx, n, steps, warmup, stat="mean"):
+def run_build(cx, n, steps, warmup, stat="mean", outputs=False):
     """C5a: batched graph build (K8) of one n x 128 shard per GPU from empty; points/s over all GPUs.
     stat: how the timed builds are summarised — "mean" (the headline contract) or "median" (the
-    extra block: one build in a few runs long on some hosts, DESIGN.md K8; every time is listed)."""
+    extra block: one build in a few runs long on some hosts, DESIGN.md K8; every time is listed).
+    outputs: also return the graph of the last timed build (degree and edge list of nodes 1..n+1,
+    unused slots -1)."""
     torch = cx.torch
     from semadb_b200 import synth
     X = synth.sift_shaped(n, 128, seed=3 + 1000 * cx.rank, w_seed=3)
@@ -776,6 +814,15 @@ def run_build(cx, n, steps, warmup, stat="mean"):
             times.append(dt)
             stats = g.insert_stats()
     dt = float(np.median(times)) if stat == "median" else float(np.mean(times))
+    graph = None
+    if outputs:
+        keep = dump_rows(n + 1, 4 + R * 8)
+        rows = np.arange(n + 1) if keep is None else keep
+        deg, edges = g.get_edges((rows + 1).astype(np.uint64))
+        edges = np.where(np.arange(R)[None, :] < deg[:, None], edges.astype(np.float64), -1.0)
+        graph = {"degree": deg.astype(np.float32), "edges": edges}
+        if keep is not None:
+            graph["rows"] = keep.astype(np.float64)
     # algorithmic bytes of the build (DESIGN.md K8): the searches' gathers, the candidate rows of
     # robustPrune(new), the adjacency rows of the back-edge targets (read + write) and the
     # candidate rows of robustPrune(B) on saturated targets
@@ -788,14 +835,17 @@ def run_build(cx, n, steps, warmup, stat="mean"):
     fi, fd, _ = g.flat_search_batch(Q, K)
     rec = float(np.mean([len(set(ids_[b].tolist()) & set(fi[b].tolist())) / K for b in range(len(Q))]))
     g.close()
-    return {"workload": f"C5a: batched graph build from empty, {n}x128 f32 L2 per GPU (greedySearch + robustPrune + "
-                        f"back-edges, K8), vectors resident in HBM",
-            "points_per_s": cx.world * n / dt, "build_s": dt, "build_s_is": stat + f" of {len(times)} builds",
-            "builds_timed": len(times), "build_s_each": [round(t, 4) for t in times],
-            "n_gpus": cx.world,
-            "recall_at_10_of_built_graph": rec, "insert_stats": stats,
-            "roofline": {"bound": "hbm", "achieved": by / dt / 1e9, "peak": peak, "unit": "GB/s", "frac": by / dt / 1e9 / peak,
-                         "algorithmic_bytes_per_point": by / max(1, stats["points"]), "per": "GPU"}}
+    res = {"workload": f"C5a: batched graph build from empty, {n}x128 f32 L2 per GPU (greedySearch + robustPrune + "
+                       f"back-edges, K8), vectors resident in HBM",
+           "points_per_s": cx.world * n / dt, "build_s": dt, "build_s_is": stat + f" of {len(times)} builds",
+           "builds_timed": len(times), "build_s_each": [round(t, 4) for t in times],
+           "n_gpus": cx.world,
+           "recall_at_10_of_built_graph": rec, "insert_stats": stats,
+           "roofline": {"bound": "hbm", "achieved": by / dt / 1e9, "peak": peak, "unit": "GB/s", "frac": by / dt / 1e9 / peak,
+                        "algorithmic_bytes_per_point": by / max(1, stats["points"]), "per": "GPU"}}
+    if graph is not None:
+        res["outputs"] = graph
+    return res
 
 
 def main():
@@ -824,7 +874,11 @@ def main():
     ap.add_argument("--probe-queries", type=int, default=1000)
     ap.add_argument("--extra-budget-s", type=float, default=560.0,
                     help="no further extra workload is started once this much wall time has passed")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the headline's last timed step returned as DIR/<name>.npy (float32/float64, < 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     if args.graph == "auto":
@@ -837,7 +891,9 @@ def main():
 
     if args.workload == "c5a":
         n = args.n or 1_000_000
-        r = run_build(cx, n, max(1, min(args.steps, 5)), min(args.warmup, 1))
+        r = run_build(cx, n, args.steps, min(args.warmup, 1), outputs=args.dump_outputs is not None)
+        if rank == 0 and args.dump_outputs:
+            dump_outputs(args.dump_outputs, r["outputs"])
         if rank == 0:
             out = {"metric": "vamana_build_points_per_s", "value": r["points_per_s"], "unit": "points/s", "n_gpus": world,
                    "steps": r["builds_timed"], "warmup": min(args.warmup, 1), "ms_per_step": r["build_s"] * 1e3,
@@ -863,6 +919,8 @@ def main():
     n = args.n or WORKLOADS[name]["n"]
     h = run_search(cx, name, n, B, args.steps, max(3, args.warmup), args.graph, headline=True)
     h["n"] = n
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, h["outputs"])
 
     # ---- cpu baseline (untimed, rank 0, N = 1, C2)
     cpu = None

@@ -614,8 +614,9 @@ int robust_prune(const Index* ix, uint32_t node, std::vector<Elem>& cand, uint32
   return cnt;
 }
 
-// insertSinglePoint (shard/index/vamana/insert.go:16-68)
-int insert_single(Index* ix, uint32_t id, const float* v, SearchScratch& sc, SearchOut& so, bool locked) {
+// insertSinglePoint, first half (insert.go:16-36): greedySearch from the start node and
+// robustPrune of the visited set become the new point's edges.
+int insert_link(Index* ix, uint32_t id, const float* v, SearchScratch& sc, SearchOut& so, bool locked) {
   // vecStore.Set happened already (capacity must not move under concurrent workers)
   int rc = greedy_search(ix, v, 1, ix->L, nullptr, 0, sc, so, locked);
   if (rc) return rc;
@@ -625,33 +626,47 @@ int insert_single(Index* ix, uint32_t id, const float* v, SearchScratch& sc, Sea
   std::memcpy(ix->A(id), edgesA.data(), sizeof(uint32_t) * dA);
   ix->deg[id] = uint16_t(dA);
   if (locked) ix->locks[id].unlock();
+  return 0;
+}
+
+// insertSinglePoint, second half (insert.go:37-66): the back-edge b -> id, pruning b when full.
+void insert_back_edge(Index* ix, uint32_t b, uint32_t id, std::vector<Elem>& cand, std::vector<uint32_t>& eb) {
+  int dB = ix->deg[b];
+  if (dB + 1 > ix->R) {
+    PointDist fn(ix, b);
+    cand.clear();
+    // candidateSet.Add(nodeB.neighbours...), Add(vecA) with a VisitedMap dedupe (insert.go:48-57)
+    uint32_t* nb = ix->A(b);
+    for (int j = 0; j <= dB; ++j) {
+      uint32_t p = j < dB ? nb[j] : id;
+      bool dup = false;
+      for (const Elem& e : cand) if (e.id == p) { dup = true; break; }
+      if (dup) continue;
+      cand.push_back(Elem{p, fn(p), false, false});
+    }
+    for (size_t i = 0; i < cand.size(); ++i)  // candidateSet.Sort()
+      for (size_t j = i; j > 0 && cand[j].dist < cand[j - 1].dist; --j) std::swap(cand[j], cand[j - 1]);
+    int nd = robust_prune(ix, b, cand, eb.data(), nullptr);
+    std::memcpy(nb, eb.data(), sizeof(uint32_t) * nd);
+    ix->deg[b] = uint16_t(nd);
+  } else {
+    ix->A(b)[dB] = id;  // nodeB.AddNeighbour(vecA)
+    ix->deg[b] = uint16_t(dB + 1);
+  }
+}
+
+// insertSinglePoint (shard/index/vamana/insert.go:16-68)
+int insert_single(Index* ix, uint32_t id, const float* v, SearchScratch& sc, SearchOut& so, bool locked) {
+  int rc = insert_link(ix, id, v, sc, so, locked);
+  if (rc) return rc;
+  if (locked) ix->locks[id].lock();
+  std::vector<uint32_t> edgesA(ix->A(id), ix->A(id) + ix->deg[id]);
+  if (locked) ix->locks[id].unlock();
   std::vector<Elem> cand;
   std::vector<uint32_t> eb(ix->R);
-  for (int t = 0; t < dA; ++t) {
-    uint32_t b = edgesA[t];
+  for (uint32_t b : edgesA) {
     if (locked) ix->locks[b].lock();
-    int dB = ix->deg[b];
-    if (dB + 1 > ix->R) {
-      PointDist fn(ix, b);
-      cand.clear();
-      // candidateSet.Add(nodeB.neighbours...), Add(vecA) with a VisitedMap dedupe (insert.go:48-57)
-      uint32_t* nb = ix->A(b);
-      for (int j = 0; j <= dB; ++j) {
-        uint32_t p = j < dB ? nb[j] : id;
-        bool dup = false;
-        for (const Elem& e : cand) if (e.id == p) { dup = true; break; }
-        if (dup) continue;
-        cand.push_back(Elem{p, fn(p), false, false});
-      }
-      for (size_t i = 0; i < cand.size(); ++i)  // candidateSet.Sort()
-        for (size_t j = i; j > 0 && cand[j].dist < cand[j - 1].dist; --j) std::swap(cand[j], cand[j - 1]);
-      int nd = robust_prune(ix, b, cand, eb.data(), nullptr);
-      std::memcpy(nb, eb.data(), sizeof(uint32_t) * nd);
-      ix->deg[b] = uint16_t(nd);
-    } else {
-      ix->A(b)[dB] = id;  // nodeB.AddNeighbour(vecA)
-      ix->deg[b] = uint16_t(dB + 1);
-    }
+    insert_back_edge(ix, b, id, cand, eb);
     if (locked) ix->locks[b].unlock();
   }
   return 0;
@@ -772,6 +787,75 @@ void parallel_for(size_t n, int threads, F f) {
       }
     });
   for (auto& x : th) x.join();
+}
+
+// Reusable barrier of a fixed set of threads (generation counter).
+struct Barrier {
+  explicit Barrier(int n) : n(n) {}
+  void wait() {
+    int gen = generation.load(std::memory_order_acquire);
+    if (arrived.fetch_add(1, std::memory_order_acq_rel) + 1 == n) {
+      arrived.store(0, std::memory_order_relaxed);
+      generation.fetch_add(1, std::memory_order_acq_rel);
+    } else {
+      while (generation.load(std::memory_order_acquire) == gen) std::this_thread::yield();
+    }
+  }
+  const int n;
+  std::atomic<int> arrived{0};
+  std::atomic<int> generation{0};
+};
+
+// Parallel insert whose graph depends on the input alone, not on the thread count or timing.
+// The points go in rounds of a fixed length (1 while the call has inserted fewer than 16
+// points, growing as 1/16 of them, at most max_round). In a round every point searches the
+// graph as it stood at the start of the round and takes its own edges (insert_link, no other
+// writes happen then); then the back-edges are applied, one target per task, in input order.
+// A target's row depends only on its own row and the points added to it, so this is the
+// sequential schedule's result for that round. max_round 1 is the 1-worker schedule.
+int insert_rounds(Index* ix, const uint32_t* ids, const float* vecs, size_t n, int T, size_t max_round) {
+  std::vector<SearchScratch> sc(T);
+  std::vector<SearchOut> so(T);
+  std::vector<std::vector<Elem>> cand(T);
+  std::vector<std::vector<uint32_t>> eb(T, std::vector<uint32_t>(ix->R));
+  std::vector<std::pair<uint32_t, uint32_t>> pairs;  // (target, input index of the new point)
+  std::vector<size_t> group;                         // start of each target's run in pairs
+  std::atomic<size_t> next_link(0), next_target(0);
+  std::atomic<int> err(0);
+  Barrier bar(T);
+  auto worker = [&](int t) {
+    for (size_t s = 0; s < n;) {
+      size_t m = std::min(n - s, std::min(std::max<size_t>(max_round, 1), std::max<size_t>(1, s / 16)));
+      for (size_t i; (i = next_link.fetch_add(1)) < m;) {
+        int rc = insert_link(ix, ids[s + i], vecs + (s + i) * ix->dim, sc[t], so[t], false);
+        if (rc) err.store(rc);
+      }
+      bar.wait();
+      if (t == 0) {
+        pairs.clear();
+        for (size_t i = s; i < s + m; ++i)
+          for (int j = 0; j < ix->deg[ids[i]]; ++j) pairs.emplace_back(ix->A(ids[i])[j], uint32_t(i));
+        std::stable_sort(pairs.begin(), pairs.end(), [](const auto& a, const auto& b) { return a.first < b.first; });
+        group.clear();
+        for (size_t k = 0; k < pairs.size(); ++k)
+          if (k == 0 || pairs[k].first != pairs[k - 1].first) group.push_back(k);
+        group.push_back(pairs.size());
+        next_link.store(0);
+        next_target.store(0);
+      }
+      bar.wait();
+      for (size_t g; (g = next_target.fetch_add(1)) + 1 < group.size();)
+        for (size_t k = group[g]; k < group[g + 1]; ++k)
+          insert_back_edge(ix, pairs[k].first, ids[pairs[k].second], cand[t], eb[t]);
+      bar.wait();
+      s += m;
+    }
+  };
+  std::vector<std::thread> th;
+  for (int t = 1; t < T; ++t) th.emplace_back(worker, t);
+  worker(0);
+  for (auto& x : th) x.join();
+  return err.load();
 }
 
 }  // namespace
@@ -916,6 +1000,24 @@ int orc_index_insert(void* h, const uint32_t* ids, const float* vecs, size_t n, 
     if (rc) err.store(rc);
   });
   return err.load();
+}
+
+// The same insert on the deterministic round schedule (insert_rounds): the graph is a function
+// of the input and max_round only, whatever the thread count.
+int orc_index_insert_rounds(void* h, const uint32_t* ids, const float* vecs, size_t n, int threads, size_t max_round) {
+  auto* ix = static_cast<Index*>(h);
+  uint32_t mx = 0;
+  for (size_t i = 0; i < n; ++i) {
+    if (ids[i] == 0 || ids[i] == 1) return 10;
+    mx = std::max(mx, ids[i]);
+  }
+  ix->reserve(size_t(mx) + 1);
+  if (mx > ix->maxNodeId) ix->maxNodeId = mx;
+  for (size_t i = 0; i < n; ++i) {
+    ix->set(ids[i], vecs + i * ix->dim);
+    ix->deg[ids[i]] = 0;
+  }
+  return insert_rounds(ix, ids, vecs, n, std::max(1, threads), max_round);
 }
 
 // insertUpdateDelete (vamana.go:136-263) without the trailing Fit/flush: classify each

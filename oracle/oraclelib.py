@@ -73,6 +73,8 @@ def lib():
     L.orc_index_set_vectors.argtypes = [C.c_void_p, u32p, f32p, C.c_size_t]
     L.orc_index_insert.restype = C.c_int
     L.orc_index_insert.argtypes = [C.c_void_p, u32p, f32p, C.c_size_t, C.c_int]
+    L.orc_index_insert_rounds.restype = C.c_int
+    L.orc_index_insert_rounds.argtypes = [C.c_void_p, u32p, f32p, C.c_size_t, C.c_int, C.c_size_t]
     L.orc_index_fit.restype = C.c_int
     L.orc_index_fit.argtypes = [C.c_void_p, C.c_size_t, C.c_int, C.c_int]
     L.orc_index_update_delete.argtypes = [C.c_void_p, u32p, f32p, u8p, C.c_size_t, C.c_int]
@@ -240,10 +242,15 @@ class OracleIndex:
         ids, vecs = _u32(ids), _f32(vecs)
         lib().orc_index_set_vectors(self._h, _p(ids, u32p), _p(vecs, f32p), len(ids))
 
-    def insert(self, ids, vecs, threads=1):
+    def insert(self, ids, vecs, threads=1, max_round=0):
+        """max_round 0: the reference's schedule (sequential, or concurrent workers when threads > 1);
+        max_round > 0: rounds of at most that many points, a graph independent of threads and timing."""
         ids, vecs = _u32(ids), _f32(vecs)
         assert vecs.shape == (len(ids), self.dim)
-        rc = lib().orc_index_insert(self._h, _p(ids, u32p), _p(vecs, f32p), len(ids), threads)
+        if max_round:
+            rc = lib().orc_index_insert_rounds(self._h, _p(ids, u32p), _p(vecs, f32p), len(ids), threads, max_round)
+        else:
+            rc = lib().orc_index_insert(self._h, _p(ids, u32p), _p(vecs, f32p), len(ids), threads)
         if rc:
             raise RuntimeError(f"oracle insert failed rc={rc}")
 

@@ -1,5 +1,6 @@
 import sys, time
-sys.path.insert(0, '/root/repo')
+from pathlib import Path
+sys.path.insert(0, str(Path(__file__).resolve().parent.parent))
 import numpy as np
 from semadb_b200 import synth
 from semadb_b200.vamana import IndexVamana, IndexVectorVamanaParameters

@@ -33,3 +33,27 @@ def test_reference_arm_prints_one_json_line_with_the_contract_keys():
 
 def test_reference_arm_is_silent_on_other_ranks():
     assert _run({"RANK": "1", "WORLD_SIZE": "2", "LOCAL_RANK": "1"}).strip() == ""
+
+
+def test_dump_outputs_keeps_the_same_seeded_rows_under_the_limit(tmp_path, monkeypatch):
+    """--dump-outputs: above the size limit every array keeps the same fixed sample of rows, listed
+    in rows.npy, and two runs write the same files."""
+    import numpy as np
+    sys.path.insert(0, str(ROOT))
+    import bench
+    monkeypatch.setattr(bench, "DUMP_BYTES", 4000)
+    ids = np.arange(1000 * 10, dtype=np.float64).reshape(1000, 10)
+    dists = (ids * 0.5).astype(np.float32)
+    for run in ("a", "b"):
+        bench.dump_outputs(tmp_path / run, {"ids": ids, "dists": dists})
+    got = [{p.name: np.load(p) for p in (tmp_path / run).glob("*.npy")} for run in ("a", "b")]
+    assert sorted(got[0]) == ["dists.npy", "ids.npy", "rows.npy"]
+    assert sum(a.nbytes for a in got[0].values()) <= 4000
+    rows = got[0]["rows.npy"].astype(np.int64)
+    assert len(rows) > 0 and (np.diff(rows) > 0).all()
+    assert (got[0]["ids.npy"] == ids[rows]).all() and (got[0]["dists.npy"] == dists[rows]).all()
+    assert all(got[0][k].tobytes() == got[1][k].tobytes() for k in got[0])
+    small = {"counts": np.full(7, 10, np.float32)}
+    bench.dump_outputs(tmp_path / "c", small)
+    assert sorted(p.name for p in (tmp_path / "c").glob("*.npy")) == ["counts.npy"]
+    assert (np.load(tmp_path / "c" / "counts.npy") == small["counts"]).all()

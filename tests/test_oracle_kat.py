@@ -501,3 +501,19 @@ def test_hybrid_merge_semantics():
     # a single sub-search is returned as is (search.go:246-249)
     oi, oh, od, oc = O.hybrid_merge(ids[:1], h[:1], d[:1], c[:1], disjunction=False)
     assert oc[0] == 4 and oi[0].tolist() == [42, 43, 44, 45]
+
+
+def test_round_insert_depends_on_the_input_only():
+    """OracleIndex.insert(max_round=...): the same graph for any thread count, and rounds of one
+    point are the reference's 1-worker schedule, edge for edge."""
+    from semadb_b200 import synth
+    X = synth.sift_shaped(3000, 32, 11)
+
+    def graph(threads, max_round):
+        ix = O.OracleIndex(32, "euclidean", 75, 64, 1.2)
+        ix.set_start(synth.start_vector(32, 5))
+        ix.insert(np.arange(2, len(X) + 2, dtype=np.uint32), X, threads=threads, max_round=max_round)
+        return ix.get_graph()
+
+    for want, got in ((graph(1, 64), graph(7, 64)), (graph(1, 0), graph(4, 1))):
+        assert (want[1] == got[1]).all() and (want[0] == got[0]).all()
