@@ -154,16 +154,30 @@ __device__ __forceinline__ float float_dist_thread(const float* __restrict__ x, 
   return metric_epilogue<METRIC>(s);
 }
 
-// distance.go:33-43 (float64 math like the reference).
-__device__ __forceinline__ float haversine_thread(const float* x, const float* y) {
-  const double degToRad = 3.14159265358979323846 / 180.0, earthRadius = 6371000.0;
-  double latx = double(x[0]) * degToRad, lonx = double(x[1]) * degToRad;
-  double laty = double(y[0]) * degToRad, lony = double(y[1]) * degToRad;
-  double dlat = latx - laty, dlon = lonx - lony;
+// distance.go:33-43 (float64 math like the reference), split so that a caller with one fixed x
+// (the beam search's query) computes x's terms once: haversine_terms(x) then haversine_from(x, y).
+struct HaversineX {
+  double lat, lon, coslat;  // radians; cos(lat)
+};
+constexpr double HAV_DEG_TO_RAD = 3.14159265358979323846 / 180.0;
+__device__ __forceinline__ HaversineX haversine_terms(float x0, float x1) {
+  HaversineX h;
+  h.lat = double(x0) * HAV_DEG_TO_RAD;
+  h.lon = double(x1) * HAV_DEG_TO_RAD;
+  h.coslat = cos(h.lat);
+  return h;
+}
+__device__ __forceinline__ float haversine_from(const HaversineX& x, float y0, float y1) {
+  const double earthRadius = 6371000.0;
+  double laty = double(y0) * HAV_DEG_TO_RAD, lony = double(y1) * HAV_DEG_TO_RAD;
+  double dlat = x.lat - laty, dlon = x.lon - lony;
   double sdlat = sin(dlat / 2), sdlon = sin(dlon / 2);
-  double a = sdlat * sdlat + cos(latx) * cos(laty) * sdlon * sdlon;
+  double a = sdlat * sdlat + x.coslat * cos(laty) * sdlon * sdlon;
   double c = 2 * asin(sqrt(a));
   return float(earthRadius * c);
+}
+__device__ __forceinline__ float haversine_thread(const float* x, const float* y) {
+  return haversine_from(haversine_terms(x[0], x[1]), y[0], y[1]);
 }
 
 // distance.go:45-67 on u64 words.

@@ -237,6 +237,7 @@ int sdb_index_create(const sdb_params* params, sdb_index** out) {
   ix->words = (p.dim + 63) / 64;
   ix->bits_pitch = (ix->words + 1) / 2 * 2;
   ix->store_metric = p.metric;
+  if (const char* g = getenv("SDB_GEO_CTAS")) ix->geo_ctas_per_sm = atoi(g);  // A/B runs of the geo search (search_geo.cu)
   if (p.quantizer == SDB_QUANT_BINARY) {
     ix->bq_metric = p.bq_metric;
     if ((e = cudaMalloc(reinterpret_cast<void**>(&ix->d_bq_thr), p.dim * sizeof(float))) != cudaSuccess) {

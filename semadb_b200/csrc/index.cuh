@@ -152,6 +152,7 @@ struct sdb_index {
   sdb::DevBuf<uint64_t> d_sample_ids;
   uint32_t last_B = 0;
   int vt_level = 0;                  // visited-table size step (search.cu)
+  int geo_ctas_per_sm = 0;           // geo beam search: CTAs/SM cap for A/B runs, SDB_GEO_CTAS read at create (0 = kernel's bound)
   bool retry_check_pending = false;  // d_work holds the retry count of the last search
   cudaStream_t last_search_stream = nullptr;
   uint64_t launches = 0;

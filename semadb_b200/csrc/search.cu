@@ -13,8 +13,27 @@ extern template int launch_float<METRIC_COSINE>(sdb_index*, const SearchArgs&, b
 // search_bits.cu / search_pq.cu: the bit-row and PQ-code evaluators
 int launch_bits(sdb_index* ix, const SearchArgs& a, bool filtered, cudaStream_t stream);
 int launch_pq(sdb_index* ix, const SearchArgs& a, bool filtered, cudaStream_t stream);
+// search_geo.cu: dim-2 haversine rows
+int launch_geo(sdb_index* ix, const SearchArgs& a, bool filtered, cudaStream_t stream);
 }  // namespace launch
 using namespace launch;
+
+// Visited-table slots of the geo kernel (profiles/r03_geo.json, B200 at 1000 W): a geo query evaluates
+// ~590 rows on average at L = 75 (p99 920, max 1240 at 1 M points; p99 1130, max 3500 at 10 M). 1024
+// slots (limit 896) send the tail to the RETRY launch: 3.8 M QPS at 1 M points against 6.0 M with 2048
+// and 4.1 M with 4096 (why 4096 costs that much is not measured). A level is usable when the quotient
+// span (VisitedCompactN::init) leaves a displacement of at least 2 buckets: at 10 M points 2048 slots
+// have span 32768 and no displacement, every bucket collision spills (0.44 M QPS), 4096 slots 2.4 M.
+// So: 2048 slots up to 2^23 rows, 4096 up to 2^24, ...; the retry step-up (vt_level) moves on from there.
+static uint32_t geo_vt_slots(const sdb_index* ix) {
+  static const uint32_t kGeoSlots[4] = {2048, 4096, 8192, 16384};
+  uint32_t b = ix->rows <= 2 ? 1 : 32 - uint32_t(__builtin_clz(ix->rows - 1));
+  if (b < 16) b = 16;
+  int lvl = 0;
+  auto span = [&](int l) { return ((uint64_t(1) << b) + kGeoSlots[l] / 4 - 1) / (kGeoSlots[l] / 4); };
+  while (lvl < 3 && (65535u - std::min<uint64_t>(span(lvl), 65535u)) / span(lvl) < 2) ++lvl;
+  return kGeoSlots[std::min(3, lvl + ix->vt_level)];
+}
 
 static int dispatch_search(sdb_index* ix, const SearchArgs& a, bool filtered, cudaStream_t stream);
 
@@ -41,6 +60,7 @@ int launch_search(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k,
   SDB_CUDA(cudaMemsetAsync(ix->d_work.p, 0, 4 * sizeof(uint32_t), stream));
   SearchArgs a{};
   a.vt_slots = kSlots[ix->vt_level];
+  if (ix->store_metric == SDB_METRIC_HAVERSINE && !ix->quant_active()) a.vt_slots = geo_vt_slots(ix);
   if (const char* e = getenv("SDB_VT_SLOTS")) a.vt_slots = uint32_t(atoi(e)) / 8 * 8;
   a.vec = ix->d_vec;
   a.vec_pitch = ix->vec_pitch;
@@ -130,6 +150,7 @@ static int dispatch_search(sdb_index* ix, const SearchArgs& a, bool filtered, cu
     case SDB_METRIC_EUCLIDEAN: return launch_float<METRIC_EUCLIDEAN>(ix, a, filtered, stream);
     case SDB_METRIC_DOT: return launch_float<METRIC_DOT>(ix, a, filtered, stream);
     case SDB_METRIC_COSINE: return launch_float<METRIC_COSINE>(ix, a, filtered, stream);
+    case SDB_METRIC_HAVERSINE: return launch_geo(ix, a, filtered, stream);
     default: return fail(SDB_ERR_INVALID, "metric not supported by the Vamana search kernel");
   }
 }

@@ -15,7 +15,8 @@
 // Algorithmic bytes per query = n_dist*row_bytes + n_hops*R*4 (SURVEY.md §8d); the
 // kernel reports n_hops and n_dist per query.
 // Evaluators: f32 rows (fixed dims pipelined, any dim generic), bit rows (hamming / jaccard),
-// PQ codes against the query's ADC table in global or in shared memory (bulk async copy).
+// PQ codes against the query's ADC table in global or in shared memory (bulk async copy),
+// dim-2 haversine rows (one lane per candidate, float64 math).
 // Epilogue: the top-k goes to the caller's buffers (device, or mapped host memory) and, for a
 // sharded search, straight into every peer GPU's gather buffer (PeerGather).
 #pragma once
@@ -1197,7 +1198,29 @@ struct AdcEvalFly {
   }
 };
 
-enum EvalKind : int { EVAL_FLOAT_FIXED = 0, EVAL_FLOAT_GENERIC = 1, EVAL_BITS = 2, EVAL_ADC = 3, EVAL_ADC_SMEM = 4, EVAL_ADC_FLY = 5 };
+// dim-2 haversine rows (latitude, longitude in degrees; distance.go:33-43). A row is 8 bytes of a
+// 16-byte pitch, so the 8-lane-per-line layout of the f32 evaluators would leave 7 of 8 lanes idle:
+// here one lane owns a candidate (adjacency slot c in lane c % 32, a second one for c >= 32), both
+// rows are loaded before either distance is computed, and the query's terms (radians, cos(lat)) are
+// computed once per query into registers. haversine_from is haversine_thread's body with the query
+// as x, so every distance is the float sdb_index_query_dists and the flat scan produce.
+struct GeoEval {
+  HaversineX q;
+  __device__ __forceinline__ void load_query(const float* qg) { q = haversine_terms(__ldg(qg), __ldg(qg + 1)); }
+  template <class Hook>
+  __device__ __forceinline__ void eval(const SearchArgs& a, const uint32_t* cid, float* cdist, int n, int lane, Hook&& hook) {
+    const bool h0 = lane < n, h1 = lane + 32 < n;
+    float2 r0 = make_float2(0.f, 0.f), r1 = make_float2(0.f, 0.f);
+    if (h0) r0 = __ldg(reinterpret_cast<const float2*>(a.vec + size_t(cid[lane]) * a.vec_pitch));
+    if (h1) r1 = __ldg(reinterpret_cast<const float2*>(a.vec + size_t(cid[lane + 32]) * a.vec_pitch));
+    hook();
+    if (h0) cdist[lane] = haversine_from(q, r0.x, r0.y);
+    if (h1) cdist[lane + 32] = haversine_from(q, r1.x, r1.y);
+    __syncwarp();
+  }
+};
+
+enum EvalKind : int { EVAL_FLOAT_FIXED = 0, EVAL_FLOAT_GENERIC = 1, EVAL_BITS = 2, EVAL_ADC = 3, EVAL_ADC_SMEM = 4, EVAL_ADC_FLY = 5, EVAL_GEO = 6 };
 
 // ---- shared-memory layout per query-warp ------------------------------------------------
 template <class VT, bool FILTER>
@@ -1267,7 +1290,7 @@ __global__ void __launch_bounds__(32, MINB) beam_search_kernel(SearchArgs a, uin
 
     // ---- per-query setup
     vt.clear(lane);
-    if (KIND != EVAL_ADC && KIND != EVAL_ADC_SMEM && KIND != EVAL_BITS) {
+    if (KIND != EVAL_ADC && KIND != EVAL_ADC_SMEM && KIND != EVAL_BITS && KIND != EVAL_GEO) {
       const float* qg = a.queries + size_t(qi) * a.dim;
       for (uint32_t i = lane; i < qfloats; i += 32) qs[i] = i < a.dim ? __ldg(qg + i) : 0.0f;
     }
@@ -1283,6 +1306,8 @@ __global__ void __launch_bounds__(32, MINB) beam_search_kernel(SearchArgs a, uin
     constexpr bool FLY = (KIND == EVAL_ADC_FLY);
     AdcEvalFly<(FLY && METRIC == METRIC_EUCLIDEAN ? METRIC_EUCLIDEAN : METRIC_DOT), (FLY ? TRIPS : 4)> ev_fly;
     if (FLY) ev_fly.qs = qs;
+    GeoEval ev_geo;
+    if (KIND == EVAL_GEO) ev_geo.load_query(a.queries + size_t(qi) * a.dim);
     if (KIND == EVAL_ADC_SMEM)
       ev_adcs.load_table(tab, a.adc + size_t(qi) * a.pqM * a.pqK, a.pqM * a.pqK, tbar, tphase, lane);
     if (KIND == EVAL_FLOAT_FIXED) ev_fixed.load_query(qs, a.queries + size_t(qi) * a.dim, lane);
@@ -1297,6 +1322,7 @@ __global__ void __launch_bounds__(32, MINB) beam_search_kernel(SearchArgs a, uin
       if (KIND == EVAL_ADC) ev_adc.eval(a, cid, cdist, n, lane, hook);
       if (KIND == EVAL_ADC_SMEM) ev_adcs.eval(a, cid, cdist, n, lane, hook);
       if (KIND == EVAL_ADC_FLY) ev_fly.eval(a, cid, cdist, n, lane, hook);
+      if (KIND == EVAL_GEO) ev_geo.eval(a, cid, cdist, n, lane, hook);
     };
     auto evaluate = [&](int n) { evaluate_h(n, no_hook); };
 
@@ -1481,7 +1507,8 @@ __global__ void __launch_bounds__(32, MINB) beam_search_kernel(SearchArgs a, uin
         if (nnew > 0) {
           if (x0 == 0) evaluate_h(nnew, pf_rows);
           else evaluate(nnew);
-          constexpr bool TIEFIX = (KIND == EVAL_BITS || KIND == EVAL_ADC || KIND == EVAL_ADC_SMEM || KIND == EVAL_ADC_FLY);  // integer-valued / coarse distances
+          // integer-valued / coarse distances; geo: points at one address (exact duplicates) tie exactly
+          constexpr bool TIEFIX = (KIND == EVAL_BITS || KIND == EVAL_ADC || KIND == EVAL_ADC_SMEM || KIND == EVAL_ADC_FLY || KIND == EVAL_GEO);
           if (MERGE_MIN == 0 || !list.template merge<TIEFIX>(cid, cdist, nnew, lane, lt, MERGE_MIN)) add_with_limit(list, nnew);
         }
         if (!XTRA || e != START_ID || x0 >= a.n_start_extra) break;

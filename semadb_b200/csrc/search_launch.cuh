@@ -1,6 +1,7 @@
 // search_launch.cuh — launch plumbing of the beam-search kernel variants (search.cuh), shared by
 // the translation units that instantiate them: search.cu (dispatcher, bit and PQ stores) and
-// search_l2.cu / search_dot.cu / search_cos.cu (one f32 metric each, so the four compile in parallel).
+// search_l2.cu / search_dot.cu / search_cos.cu (one f32 metric each, so the four compile in parallel),
+// search_geo.cu (dim-2 haversine rows).
 #pragma once
 #include "search.cuh"
 
@@ -19,20 +20,23 @@ int launch_variant_x(sdb_index* ix, const SearchArgs& a, cudaStream_t stream) {
   auto kern = beam_search_kernel<KIND, METRIC, TRIPS, SETS, LEGACY, MERGE_MIN, VT, FILTER, RETRY, MINB, XTRA, PF>;
   // FloatEvalGrouped keeps short queries (<= 4 float4 per lane) in registers: no shared copy
   constexpr bool QREG = (KIND == EVAL_FLOAT_FIXED) && !LEGACY && TRIPS <= 4;
-  const uint32_t qfloats = (KIND == EVAL_ADC || KIND == EVAL_ADC_SMEM || KIND == EVAL_BITS || QREG) ? 0 : (a.dim + 3) / 4 * 4;
+  const uint32_t qfloats = (KIND == EVAL_ADC || KIND == EVAL_ADC_SMEM || KIND == EVAL_BITS || KIND == EVAL_GEO || QREG) ? 0 : (a.dim + 3) / 4 * 4;
   const uint32_t qwords = (KIND == EVAL_BITS) ? a.bits_pitch : 0;
   const uint32_t table_floats = (KIND == EVAL_ADC_SMEM) ? a.pqM * a.pqK : 0;
   const size_t smem = warp_smem_bytes<VT, FILTER>(qfloats, qwords, a.vt_slots, table_floats);
   static thread_local int cached_dev = -1;
   static thread_local size_t cached_smem = 0;
   static thread_local int ctas_per_sm = 0;
-  if (cached_dev != ix->device || cached_smem != smem) {
+  // geo kernel: CTAs/SM below the launch bound for A/B runs (sdb_index::geo_ctas_per_sm, 0 = MINB)
+  const int cap = (KIND == EVAL_GEO && MINB > 1 && ix->geo_ctas_per_sm > 0) ? std::min(ix->geo_ctas_per_sm, MINB) : MINB;
+  static thread_local int cached_cap = 0;
+  if (cached_dev != ix->device || cached_smem != smem || cached_cap != cap) {
     if (smem > ix->smem_optin) return fail(SDB_ERR_INTERNAL, "beam search kernel does not fit in shared memory");
     SDB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
     int nb = 0;
     SDB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kern, 32, smem));
     if (nb <= 0) return fail(SDB_ERR_INTERNAL, "beam search kernel cannot be resident");
-    if (MINB > 1 && nb > MINB) nb = MINB;
+    if (MINB > 1 && nb > cap) nb = cap;
     ctas_per_sm = nb;
     // The unified L1/shared array is also where in-flight global loads land: ask for no more
     // shared memory than the resident CTAs need so the rest stays L1 (more rows in flight).
@@ -46,6 +50,7 @@ int launch_variant_x(sdb_index* ix, const SearchArgs& a, cudaStream_t stream) {
               need_smem >> 10);
     cached_smem = smem;
     cached_dev = ix->device;
+    cached_cap = cap;
   }
   uint32_t resident = uint32_t(ix->sm_count) * ctas_per_sm;
   uint32_t need = RETRY ? std::min<uint32_t>(uint32_t(ix->sm_count), ix->retry_slots) : a.n_work;

@@ -146,3 +146,66 @@ def clustered_latent(n: int, dim: int, seed: int, w_seed: int | None = None, lat
     if normalize:
         x /= np.maximum(np.linalg.norm(x, axis=1, keepdims=True), 1e-30)
     return x.astype(np.float32)
+
+
+# ---- geo (haversine, dim 2): rows are (latitude, longitude) in degrees, x[0] = latitude like the
+# reference's KAT [-34.83333, -58.5166646] (Buenos Aires).
+
+def _geo_centres(centres: int, seed: int) -> tuple[np.ndarray, np.ndarray]:
+    """City centres uniform on the sphere (lat = asin(U[-1,1])); centre 0 sits on the north pole,
+    centre 1 on the south pole and centre 2 on the antimeridian, so those cases always occur."""
+    rng = np.random.Generator(np.random.PCG64(seed))
+    clat = np.degrees(np.arcsin(rng.uniform(-1.0, 1.0, centres)))
+    clon = rng.uniform(-180.0, 180.0, centres)
+    if centres > 0:
+        clat[0] = 90.0
+    if centres > 1:
+        clat[1] = -90.0
+    if centres > 2:
+        clon[2] = 180.0
+    return clat, clon
+
+
+def _geo_draw(n: int, rng, clat, clon, spread_deg: float, background: float) -> np.ndarray:
+    lat = np.empty(n, dtype=np.float64)
+    lon = np.empty(n, dtype=np.float64)
+    bg = rng.random(n) < background if len(clat) else np.ones(n, dtype=bool)
+    nb = int(bg.sum())
+    lat[bg] = np.degrees(np.arcsin(rng.uniform(-1.0, 1.0, nb)))
+    lon[bg] = rng.uniform(-180.0, 180.0, nb)
+    nc = n - nb
+    if nc:
+        k = rng.integers(0, len(clat), nc)
+        lat[~bg] = clat[k] + rng.normal(0.0, spread_deg, nc)
+        lon[~bg] = clon[k] + rng.normal(0.0, spread_deg, nc)
+    np.clip(lat, -90.0, 90.0, out=lat)
+    lon = (lon + 180.0) % 360.0 - 180.0  # wrap into [-180, 180)
+    return _geo_f32(lat, lon)
+
+
+def _geo_f32(lat, lon) -> np.ndarray:
+    out = np.stack([lat, lon], 1).astype(np.float32)
+    out[out[:, 1] >= 180.0, 1] = -180.0  # a longitude just below 180 can round up to it in float32
+    return out
+
+
+def geo_points(n: int, seed: int, centres: int = 200, spread_deg: float = 0.5, background: float = 0.1) -> np.ndarray:
+    """float32 [n, 2] (lat, lon) in degrees: a `background` fraction uniform on the sphere, the rest
+    clustered around `centres` "cities" (normal, `spread_deg` per coordinate). Longitudes wrap into
+    [-180, 180), so the antimeridian city straddles it; latitudes are clipped at +-90, so the polar
+    cities pile up on the poles."""
+    clat, clon = _geo_centres(centres, seed)
+    return _geo_draw(n, np.random.Generator(np.random.PCG64(seed + 7919)), clat, clon, spread_deg, background)
+
+
+def geo_queries(n: int, seed: int, centres: int = 200, spread_deg: float = 0.5, background: float = 0.1,
+                jitter_deg: float = 0.01, query_seed: int = 1) -> np.ndarray:
+    """Queries for geo_points(..., seed, centres, spread_deg, background): fresh draws from the same
+    cities and background (own stream, query_seed), each jittered by N(0, jitter_deg)."""
+    clat, clon = _geo_centres(centres, seed)
+    rng = np.random.Generator(np.random.PCG64(seed + 15485863 * query_seed))
+    q = _geo_draw(n, rng, clat, clon, spread_deg, background).astype(np.float64)
+    q += rng.normal(0.0, jitter_deg, q.shape)
+    np.clip(q[:, 0], -90.0, 90.0, out=q[:, 0])
+    q[:, 1] = (q[:, 1] + 180.0) % 360.0 - 180.0
+    return _geo_f32(q[:, 0], q[:, 1])
