@@ -8,7 +8,8 @@
 // a second kernel merges the chunks in chunk order with the same rule.
 // Distances use the reference's exact f32 summation order (common.cuh), one thread per
 // (query, point) pair; the query tile sits transposed in shared memory (conflict-free),
-// the point rows are read through a broadcast shared tile.
+// the point rows are read through a broadcast shared tile of up to FP rows (fewer when FP rows
+// of a wide store do not fit next to the query tile).
 #include "common.cuh"
 #include "index.cuh"
 
@@ -17,7 +18,7 @@ namespace sdb {
 namespace {
 
 constexpr int FQ = 128;      // queries per CTA (one per thread)
-constexpr int FP = 16;       // points per shared tile
+constexpr int FP = 16;       // points per shared tile (at most; FlatArgs::tile_pts)
 constexpr int FMAXK = 75;    // models/search.go:329
 
 struct FlatArgs {
@@ -31,7 +32,8 @@ struct FlatArgs {
   const float* queries;
   uint32_t dim, B, k;
   uint32_t first_id, end_id;  // scan [first_id, end_id)
-  uint32_t chunk;             // points per chunk
+  uint32_t chunk;             // points per chunk (a multiple of tile_pts)
+  uint32_t tile_pts;          // f32 rows per shared point tile, 1..FP
   uint32_t n_chunks;
   uint32_t* part_ids;         // [B][n_chunks][k]
   float* part_d;
@@ -88,8 +90,8 @@ __global__ void __launch_bounds__(FQ) flat_scan_kernel(FlatArgs a) {
     __syncthreads();
     constexpr bool L2 = (METRIC == METRIC_EUCLIDEAN);
     const int blocks = a.dim >> 5;
-    for (uint32_t p0 = lo; p0 < hi; p0 += FP) {
-      uint32_t np = min(uint32_t(FP), hi - p0);
+    for (uint32_t p0 = lo; p0 < hi; p0 += a.tile_pts) {
+      uint32_t np = min(a.tile_pts, hi - p0);
       for (uint32_t i = tid; i < np * a.dim; i += FQ) {
         uint32_t pp = i / a.dim, dd = i % a.dim;
         pt[pp * a.dim + dd] = a.vec[size_t(p0 + pp) * a.vec_pitch + dd];
@@ -236,7 +238,13 @@ int launch_flat_exact(sdb_index* ix, uint32_t B, const float* d_queries, uint32_
   a.n_chunks = std::min<uint32_t>(std::min<uint32_t>(want, max_chunks), 1024);
   a.chunk = (npts + a.n_chunks - 1) / a.n_chunks;
   if (a.chunk == 0) a.chunk = 1;
-  a.chunk = (a.chunk + FP - 1) / FP * FP;
+  // f32 rows: the query tile in shared memory when it fits next to FP point rows; otherwise the
+  // queries are read through L1 and the point tile takes as many rows as fit (14 at dim 4096)
+  const size_t row_bytes = size_t(a.dim) * sizeof(float);
+  const bool qsmem = (size_t(FQ) + FP) * row_bytes <= ix->smem_optin;
+  a.tile_pts = uint32_t(std::min<size_t>(FP, ix->smem_optin / row_bytes));
+  if (a.tile_pts == 0) return fail(SDB_ERR_INVALID, "flat scan: one vector does not fit in shared memory");
+  a.chunk = (a.chunk + a.tile_pts - 1) / a.tile_pts * a.tile_pts;
   a.n_chunks = npts == 0 ? 1 : (npts + a.chunk - 1) / a.chunk;
   int rc;
   size_t parts = size_t(B) * a.n_chunks * k;
@@ -255,9 +263,7 @@ int launch_flat_exact(sdb_index* ix, uint32_t B, const float* d_queries, uint32_
     a.adc = ix->d_adc.p;
     if ((rc = launch_scan<2, 0>(ix, a, 0, stream))) return rc;
   } else {
-    size_t smem = (size_t(a.dim) * FQ + size_t(FP) * a.dim) * sizeof(float);
-    const bool qsmem = smem <= ix->smem_optin;
-    if (!qsmem) smem = size_t(FP) * a.dim * sizeof(float);
+    const size_t smem = ((qsmem ? size_t(FQ) : 0) + a.tile_pts) * row_bytes;
     switch (ix->store_metric) {
       case SDB_METRIC_EUCLIDEAN:
         rc = qsmem ? launch_scan<0, METRIC_EUCLIDEAN, true>(ix, a, smem, stream) : launch_scan<0, METRIC_EUCLIDEAN, false>(ix, a, smem, stream);

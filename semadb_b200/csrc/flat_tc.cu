@@ -1514,6 +1514,15 @@ int launch_flat_tc(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k
   bool& attr_set = attr_set_dev[ix->device & 63];
   if (!attr_set) {
     SDB_CUDA(cudaFuncSetAttribute(tc_filter_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(TC_SMEM)));
+    // the re-score kernels keep queries in dynamic shared memory: RW_WARPS rows pass the 48 KB
+    // default from dim 3 073, one row next to rescore_kernel's static lists from dim ~4 084
+    const int wmax = int(RW_WARPS * MAX_DIM * sizeof(float)), cmax = int(MAX_DIM * sizeof(float));
+    for (auto kern : {rescore_warp_kernel<METRIC_EUCLIDEAN, 1>, rescore_warp_kernel<METRIC_EUCLIDEAN, 3>,
+                      rescore_warp_kernel<METRIC_DOT, 1>, rescore_warp_kernel<METRIC_DOT, 3>,
+                      rescore_warp_kernel<METRIC_COSINE, 1>, rescore_warp_kernel<METRIC_COSINE, 3>})
+      SDB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, wmax));
+    for (auto kern : {rescore_kernel<METRIC_EUCLIDEAN>, rescore_kernel<METRIC_DOT>, rescore_kernel<METRIC_COSINE>})
+      SDB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, cmax));
     attr_set = true;
   }
   // ---- level 0: exact scan of the first LEVEL0 points bounds every query's k-th distance

@@ -122,7 +122,7 @@ int set_rows_device(sdb_index* ix, uint32_t n, const uint32_t* d_ids, const floa
 }
 
 static int validate(const sdb_params& p) {
-  if (p.dim < 1 || p.dim > 4096) return fail(SDB_ERR_INVALID, "vector size must be between 1 and 4096");  // models/index.go:285
+  if (p.dim < 1 || p.dim > MAX_DIM) return fail(SDB_ERR_INVALID, "vector size must be between 1 and 4096");  // models/index.go:285
   if (p.metric < SDB_METRIC_EUCLIDEAN || p.metric > SDB_METRIC_HAVERSINE) return fail(SDB_ERR_INVALID, "unknown distance metric");
   if (p.metric == SDB_METRIC_HAVERSINE && p.dim != 2) return fail(SDB_ERR_INVALID, "haversine distance metric requires vector size 2");
   if (p.search_size > 75 || p.degree_bound > 64) return fail(SDB_ERR_INVALID, "searchSize must be <= 75 and degreeBound <= 64");

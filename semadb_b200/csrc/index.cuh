@@ -12,6 +12,8 @@
 
 namespace sdb {
 
+constexpr uint32_t MAX_DIM = 4096;  // largest vector size an index accepts (models/index.go:285)
+
 void set_error(const std::string& msg);
 int fail(int code, const std::string& msg);
 int cuda_fail(cudaError_t e, const char* what);

@@ -9,6 +9,8 @@ from oracle import oraclelib as O
 from semadb_b200 import synth
 from semadb_b200.vamana import (BinaryQuantizerParameters, IndexVamana, IndexVectorVamanaParameters,
                                 ProductQuantizerParameters, Quantizer)
+from tests.helpers import check_graph_equal as _check_graph_equal
+from tests.helpers import check_search as _check_search
 
 pytestmark = pytest.mark.gpu
 
@@ -23,24 +25,6 @@ def _mirror(oix, X, ids, start, params, relaxed=True):
     adj, deg = oix.get_graph()
     g.set_graph_dense(adj[1:], deg[1:], first_id=1)
     return g
-
-
-def _check_search(oix, g, Q, k=10, L=75):
-    ref = oix.search(Q, k=k, search_size=L, threads=8, diagnostics=True)
-    ids, d, cnt = g.search_batch(Q, k, L)
-    hops, nd = g.last_search_stats(len(Q))
-    assert (cnt == ref["counts"]).all()
-    assert (ids == ref["ids"].astype(np.uint64)).all()
-    assert _same(d, ref["dists"])
-    assert (hops == ref["hops"]).all() and (nd == ref["ndist"]).all()
-
-
-def _check_graph_equal(oix, g, n):
-    adj, odeg = oix.get_graph()
-    deg, e = g.get_edges(np.arange(1, n + 2, dtype=np.uint64))
-    assert (deg == odeg[1:n + 2]).all()
-    for r in range(n + 1):
-        assert e[r, :deg[r]].tolist() == adj[r + 1, :odeg[r + 1]].tolist(), f"node {r + 1}"
 
 
 @pytest.mark.parametrize("metric", ["hamming", "jaccard"])

@@ -4,20 +4,9 @@ import numpy as np
 import pytest
 
 from semadb_b200 import synth
+from tests.helpers import check_search as _check_search
 
 pytestmark = pytest.mark.gpu
-
-
-def _check_search(oix, g, Q, k=10, L=75):
-    ref = oix.search(Q, k=k, search_size=L, threads=8, diagnostics=True)
-    ids, d, cnt = g.search_batch(Q, k, L)
-    hops, nd = g.last_search_stats(len(Q))
-    assert (cnt == ref["counts"]).all()
-    assert (ids == ref["ids"].astype(np.uint64)).all()
-    assert d.tobytes() == ref["dists"].tobytes()
-    assert (hops == ref["hops"]).all()
-    assert (nd == ref["ndist"]).all()
-    return ref
 
 
 @pytest.mark.parametrize("metric", ["euclidean", "dot", "cosine"])
