@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """bench_geo.py — haversine (geo) Vamana indexes on one GPU: build, search, recall, and the
-CTAs/SM x visited-table sweep of the geo beam-search kernel (GeoEval, csrc/search_geo.cu).
+visited-table sizes of the geo beam-search kernel (GeoEval, csrc/search_geo.cu).
 
     python scripts/bench_geo.py [--sizes 1000000,10000000] [--out profiles/r03_geo.json]
 
@@ -17,10 +17,9 @@ synth.geo_queries, 10 k per batch, k 10, L 75, R 64, alpha 1.2. Per size:
            and the algorithmic bytes n_dist*16 + n_hops*R*4 per query;
   recall   recall@10 of 1 000 queries against the exact GPU flat scan (sdb_flat_search_batch), and the
            oracle's search on the GPU-built graph (OracleIndex.set_graph) against the same lists;
-  slots    the insert-built handle searched with SDB_VT_SLOTS = 1024 .. 8192 (where the span is valid);
-  sweep    CTAs/SM in {12, 16, 24, 32} (SDB_GEO_CTAS, read when a handle is created: one handle per
-           value holding the same vectors and graph) x starting visited-table slots (SDB_VT_SLOTS);
-           a slot count whose 16-bit quotient span does not fit the store is listed as invalid.
+  slots    the insert-built handle searched with SDB_VT_SLOTS = 1024 .. 8192 (where the span is valid).
+The CTAs/SM x slots sweep in profiles/r03_geo.json ("sweep") chose the geo kernel's launch bound;
+the residency cap it varied has been removed since, so this script no longer repeats it.
 Timing uses CUDA events and host clocks around synchronised work only. The card's name, power limit
 and maximum SM clock are read with nvidia-smi (read-only query) in the same run.
 """
@@ -150,7 +149,6 @@ def recall(a, b):
 
 
 def run_size(n, first, out_sizes):
-    import torch
     from oracle import oraclelib as O
     from semadb_b200 import synth
     from semadb_b200.vamana import IndexVamana, IndexVectorVamanaParameters
@@ -205,30 +203,6 @@ def run_size(n, first, out_sizes):
                            "rows_identical_to_oracle": int(((gi == ref["ids"].astype(np.uint64)).all(1)).sum()),
                            "ground_truth": "sdb_flat_search_batch (exact haversine scan)", "flat_path": g.flat_last_stats()[0]}
     print(f"[geo {n}] recall {res['recall_at_10']}", flush=True)
-    # sweep: one handle per CTAs/SM value (SDB_GEO_CTAS is read at create), same vectors and graph
-    sweep = []
-    for ctas in (12, 16, 24, 32):
-        os.environ["SDB_GEO_CTAS"] = str(ctas)
-        h = IndexVamana("geo-sweep", IndexVectorVamanaParameters(2, "haversine", L, R, ALPHA), start_vector=start)
-        os.environ.pop("SDB_GEO_CTAS")
-        h.set_vectors(ids, X)
-        for s0 in range(1, n + 2, 1 << 20):
-            s1 = min(n + 2, s0 + (1 << 20))
-            h.set_graph_dense(adj[s0:s1], deg[s0:s1], first_id=s0)
-        for slots in (1024, 2048, 4096):
-            row = {"ctas_per_sm": ctas, "slots": slots}
-            if not slots_valid(h.max_node_id + 1, slots) or not slots_valid(n + 2, slots):
-                row["result"] = "invalid: quotient span beyond 16 bits for this store"
-            else:
-                os.environ["SDB_VT_SLOTS"] = str(slots)
-                r = search_device(h, Q)
-                os.environ.pop("SDB_VT_SLOTS")
-                row.update(qps=r["qps"], batch_ms=r["batch_ms"], kernel_ms_median=sorted(r["kernel_ms"])[len(r["kernel_ms"]) // 2])
-            sweep.append(row)
-            print(f"[geo {n}] sweep {row}", flush=True)
-        h.close()
-        torch.cuda.synchronize()
-    res["sweep"] = sweep
     g.close()
     out_sizes.append(res)
 

@@ -4,7 +4,6 @@
     and out either way, copies inside the timed region);
   * one call's kernel timeline (torch.profiler / CUPTI: name, start offset, duration) so that the
     share of every launch of the call is on record (profiles/r02_flat_timeline.json).
-Environment switches of flat_tc.cu (SDB_FLAT_RATIO, SDB_FLAT_LEVEL0, ...) apply as usual.
 usage: python scripts/flat_timeline.py [--n 1000000] [--B 10000] [--reps 5] [--timeline]"""
 import argparse
 import ctypes as C

@@ -7,7 +7,8 @@
 //      form"): the GEMM runs in minimum mode over a sample of the point tiles spread over the id
 //      range; the k smallest of a query's per-group minima belong to k different points, so the
 //      k-th of them plus the error bound is such a tau_q (kth_thresh_kernel) — no exact work, one
-//      candidate pass over all points, one re-score. Level scheme (mma.sync pass, SDB_FLAT_LEVELS=1):
+//      candidate pass over all points, one re-score. Level scheme (mma.sync pass; SDB_FLAT_LEVELS=1
+//      selects it on the tcgen05 path too, for tests):
 //      exact top-k over the first 128 points, then steps 2-3 level by level over disjoint point
 //      ranges growing x8 (last level up to x16); a level's candidate list is seeded with the exact
 //      top-k of everything before it, so its re-score is the exact top-k of the whole prefix;
@@ -23,11 +24,10 @@
 // A query whose candidate list overflows at any level falls back to the exact scan. The result is
 // therefore bit-identical to flat.cu's, and tests compare the two.
 //
-// Three forms of the GEMM + filter, same candidates:
+// Two forms of the GEMM + filter, same candidates:
 //   * tc5_filter_kernel (default, dim <= 384): tcgen05.mma M128xN256xK16 from TMA-fed (SWIZZLE_128B)
 //     shared memory into TMEM, warp-specialised, bias and threshold folded into the GEMM as a K
 //     extension so the epilogue is a sign test — see the comment above the kernel;
-//   * tc5x2_filter_kernel (SDB_FLAT_2CTA=1): the cta_group::2 form, two SMs per 256 x 256 step;
 //   * tc_filter_kernel (dim > 384, SDB_FLAT_MMA_SYNC=1): mma.sync.m16n8k16 bf16, CTA tile 128 x 128,
 //     8 warps of 64x32, K chunks of 64 double-buffered with cp.async, ldmatrix fragments,
 //     accumulators in registers.
@@ -52,7 +52,7 @@ constexpr int TPAD = 8;                 // bf16 elements of row padding (16 B): 
 constexpr int TROW = TK + TPAD;         // 72 bf16 = 144 B per smem row
 constexpr int TC_THREADS = 256;
 constexpr uint32_t CAND_CAP = 4096;     // candidate ids kept per query
-constexpr uint32_t LEVEL0 = 128;        // points scanned exactly to bound the k-th distance (SDB_FLAT_LEVEL0 overrides: A/B);
+constexpr uint32_t LEVEL0 = 128;        // points scanned exactly to bound the k-th distance
                                         // 1M points: 128 -> 4k -> 131k -> all runs in 5.45 ms, 1024 -> 32k -> all in 5.85 ms
 constexpr uint32_t LEVEL_RATIO = 32;    // each tensor-core level covers 32x more points than the one before
 constexpr size_t TC_SMEM = size_t(2) * (TM + TN) * TROW * 2 + TN * 4;
@@ -758,253 +758,6 @@ tc5_filter_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_consta
   }
 }
 
-
-// ================================================================================================
-// Two-SM form of the same pass (tcgen05 cta_group::2): a cluster of two CTAs on neighbouring SMs
-// works on 256 queries x 256 points per step. Each CTA keeps its own 128-query tile (its half of
-// M = 256) and loads only ITS HALF of every point tile (128 rows) — the pair's MMA reads both
-// halves, so the L2->SM bytes per SM and tile halve (36 KB instead of 72 KB), which is what
-// bounds the one-SM kernel. The leader CTA (cluster rank 0) issues the M256 x N256 x K16 MMAs;
-// both CTAs' TMA loads report to the leader's full barriers (cta_group::2 loads, peer bit of the
-// barrier address cleared); tcgen05.commit multicasts to both CTAs' empty / accumulator-full
-// barriers; both CTAs' epilogue warps arrive on the leader's accumulator-empty barrier.
-constexpr uint32_t T2_XBLK_BYTES = 128 * 128;  // this CTA's half of a point tile, one 64-wide K block
-constexpr uint32_t T2_XEXT_BYTES = 128 * 32;
-constexpr uint32_t T2_PEER_MASK = 0xFEFFFFFFu;  // clears the peer bit of a shared::cluster address: the even CTA's copy
-constexpr uint32_t T2_IDESC = (1u << 4) | (1u << 7) | (1u << 10) | (uint32_t(256 >> 3) << 17) | (uint32_t(256 >> 4) << 24);
-
-__host__ __device__ inline T5Smem t2_layout(uint32_t nkb, int stages) {
-  T5Smem L;
-  L.stages = stages;
-  L.q = 0;
-  L.qe = nkb * T5_QBLK_BYTES;
-  L.x = L.qe + ((T5_QEXT_BYTES + 1023u) & ~1023u);
-  L.xe = L.x + uint32_t(stages) * T2_XBLK_BYTES;
-  L.hits = L.xe + T5_ESTAGES * T2_XEXT_BYTES;
-  L.bars = L.hits + T5_EPI_THREADS * 2 * T5_HITS * 4;
-  L.tmem_slot = L.bars + (2 * uint32_t(stages) + 2 * T5_ESTAGES + 5) * 8;
-  L.total = L.tmem_slot + 16;
-  return L;
-}
-
-__device__ __forceinline__ uint32_t t2_cta_rank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void t2_cluster_sync() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// TMA load into this CTA's shared memory, completion bytes reported to the LEADER CTA's barrier
-__device__ __forceinline__ void t2_tma_load_2d(uint32_t dst, const CUtensorMap* map, int32_t c0, int32_t c1, uint32_t bar) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];" ::"r"(dst),
-      "l"(reinterpret_cast<uint64_t>(map)), "r"(c0), "r"(c1), "r"(bar & T2_PEER_MASK)
-      : "memory");
-}
-__device__ __forceinline__ void t2_mma(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t accumulate) {
-  const uint32_t z = 0;
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "setp.ne.b32 p, %4, 0;\n"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, {%5, %5, %5, %5, %5, %5, %5, %5}, p;\n"
-      "}\n" ::"r"(tmem_d),
-      "l"(adesc), "l"(bdesc), "r"(T2_IDESC), "r"(accumulate), "r"(z)
-      : "memory");
-}
-// arrive once on the barrier at this offset in BOTH CTAs when the MMAs issued so far have completed
-__device__ __forceinline__ void t2_commit_both(uint32_t bar) {
-  const uint16_t mask = 3;
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-               "h"(mask)
-               : "memory");
-}
-__device__ __forceinline__ void t2_arrive_leader(uint32_t bar) {
-  // unqualified form (as CUTLASS's ClusterBarrier::arrive): the .release.cluster variant sat in the MIO
-  // queue for 42 % of all samples; what is ordered here are TMEM reads, fenced by tcgen05.fence before it
-  asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(bar & T2_PEER_MASK) : "memory");
-}
-
-__global__ void __launch_bounds__(T5_THREADS, 1)
-tc5x2_filter_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_x,
-                    const __grid_constant__ CUtensorMap map_qe, const __grid_constant__ CUtensorMap map_xe, TcArgs a, int stages) {
-  extern __shared__ unsigned char t5_raw[];
-  const uint32_t raw = smem_u32(t5_raw);
-  const uint32_t base = (raw + 1023u) & ~1023u;
-  unsigned char* gbase = t5_raw + (base - raw);
-  const uint32_t nkb = a.kp / T5_KB;
-  const T5Smem L = t2_layout(nkb, stages);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rank = t2_cta_rank();
-  const bool leader = rank == 0;
-  auto bar_full = [&](int s) { return base + L.bars + uint32_t(s) * 8; };
-  auto bar_empty = [&](int s) { return base + L.bars + uint32_t(stages + s) * 8; };
-  const uint32_t bar_q = base + L.bars + uint32_t(2 * stages) * 8;
-  auto bar_tfull = [&](int i) { return base + L.bars + uint32_t(2 * stages + 1 + i) * 8; };
-  auto bar_tempty = [&](int i) { return base + L.bars + uint32_t(2 * stages + 3 + i) * 8; };
-  auto bar_efull = [&](int i) { return base + L.bars + uint32_t(2 * stages + 5 + i) * 8; };
-  auto bar_eempty = [&](int i) { return base + L.bars + uint32_t(2 * stages + 5 + T5_ESTAGES + i) * 8; };
-  volatile uint32_t* tmem_slot = reinterpret_cast<volatile uint32_t*>(gbase + L.tmem_slot);
-
-  const uint32_t q0 = blockIdx.x * T5_M;  // this CTA's query tile; blockIdx.x = 2c, 2c+1 form a cluster
-  const uint32_t tile_begin = blockIdx.y * a.tiles_per_cta;
-  const uint32_t ntiles_total = (a.end_id - a.first_id + 255) / 256;
-  const uint32_t tile_end = min(tile_begin + a.tiles_per_cta, ntiles_total);
-
-  if (warp == 0 && lane == 0) {
-    for (int s = 0; s < stages; ++s) {
-      t5_mbar_init(bar_full(s), 1);
-      t5_mbar_init(bar_empty(s), 1);
-    }
-    t5_mbar_init(bar_q, 1);
-    for (int i = 0; i < 2; ++i) {
-      t5_mbar_init(bar_tfull(i), 1);
-      t5_mbar_init(bar_tempty(i), 2 * (T5_EPI_THREADS / 32));  // both CTAs' epilogue warps
-    }
-    for (int i = 0; i < T5_ESTAGES; ++i) {
-      t5_mbar_init(bar_efull(i), 1);
-      t5_mbar_init(bar_eempty(i), 1);
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 1) {  // both CTAs: the pair's TMEM (512 columns in each SM)
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(base + L.tmem_slot), "r"(512u) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-  }
-  t5_fence_before();
-  __syncthreads();
-  t2_cluster_sync();  // the peer's barriers are initialised before anything signals them
-  t5_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (warp == 0) {
-    // ===== TMA producer (both CTAs): own query tile, own half of every point tile =====
-    if (lane == 0) {
-      if (leader) t5_mbar_expect_tx(bar_q, 2 * (nkb * T5_QBLK_BYTES + T5_QEXT_BYTES));
-      for (uint32_t kb = 0; kb < nkb; ++kb)
-        t2_tma_load_2d(base + L.q + kb * T5_QBLK_BYTES, &map_q, int32_t(kb * T5_KB), int32_t(q0), bar_q);
-      t2_tma_load_2d(base + L.qe, &map_qe, int32_t(a.kp), int32_t(q0), bar_q);
-      int s = 0, es = 0;
-      uint32_t ph = 0, eph = 0;
-      for (uint32_t t = tile_begin; t < tile_end; ++t) {
-        const int32_t p0 = int32_t(a.first_id + t * 256 + rank * 128);
-        for (uint32_t kb = 0; kb < nkb; ++kb) {
-          t5_mbar_wait(bar_empty(s), ph ^ 1u);
-          if (leader) t5_mbar_expect_tx(bar_full(s), 2 * T2_XBLK_BYTES);
-          t2_tma_load_2d(base + L.x + uint32_t(s) * T2_XBLK_BYTES, &map_x, int32_t(kb * T5_KB), p0, bar_full(s));
-          if (++s == stages) { s = 0; ph ^= 1u; }
-        }
-        t5_mbar_wait(bar_eempty(es), eph ^ 1u);
-        if (leader) t5_mbar_expect_tx(bar_efull(es), 2 * T2_XEXT_BYTES);
-        t2_tma_load_2d(base + L.xe + uint32_t(es) * T2_XEXT_BYTES, &map_xe, int32_t(a.kp), p0, bar_efull(es));
-        if (++es == T5_ESTAGES) { es = 0; eph ^= 1u; }
-      }
-    }
-  } else if (warp == 1) {
-    // ===== MMA issuer: the leader CTA's elected lane drives both SMs' tensor cores =====
-    if (leader && lane == 0) {
-      t5_mbar_wait(bar_q, 0);
-      t5_fence_after();
-      int s = 0, es = 0;
-      uint32_t ph = 0, eph = 0;
-      uint32_t it = 0;
-      for (uint32_t t = tile_begin; t < tile_end; ++t, ++it) {
-        const uint32_t acc = it & 1u, aph = (it >> 1) & 1u;
-        t5_mbar_wait(bar_tempty(acc), aph ^ 1u);  // both epilogues have drained this accumulator
-        t5_fence_after();
-        const uint32_t d_tmem = tmem_base + acc * 256;
-        for (uint32_t kb = 0; kb < nkb; ++kb) {
-          t5_mbar_wait(bar_full(s), ph);
-          t5_fence_after();
-          const uint64_t adesc = t5_smem_desc(base + L.q + kb * T5_QBLK_BYTES);
-          const uint64_t bdesc = t5_smem_desc(base + L.x + uint32_t(s) * T2_XBLK_BYTES);
-#pragma unroll
-          for (uint32_t k = 0; k < T5_KB / 16; ++k) t2_mma(d_tmem, adesc + 2 * k, bdesc + 2 * k, (kb | k) != 0 ? 1u : 0u);
-          t2_commit_both(bar_empty(s));
-          if (++s == stages) { s = 0; ph ^= 1u; }
-        }
-        t5_mbar_wait(bar_efull(es), eph);
-        t5_fence_after();
-        t2_mma(d_tmem, t5_smem_desc_sw32(base + L.qe), t5_smem_desc_sw32(base + L.xe + uint32_t(es) * T2_XEXT_BYTES), 1u);
-        t2_commit_both(bar_eempty(es));
-        if (++es == T5_ESTAGES) { es = 0; eph ^= 1u; }
-        t2_commit_both(bar_tfull(acc));
-      }
-    }
-  } else {
-    // ===== epilogue (both CTAs): sign filter over this CTA's 128 queries x the tile's 256 points =====
-    const int e = warp - 2;
-    const int quad = warp & 3;
-    const int col0 = (e >> 2) * 128;
-    const int etid = threadIdx.x - 64;
-    const uint32_t q = q0 + uint32_t(quad) * 32 + lane;
-    const bool q_ok = q < a.B;
-    // Two half-buffers per thread. A full half reserves its slots with an atomicAdd whose return
-    // value is NOT consumed yet: the thread goes on filtering into the other half, and copies the
-    // reserved half out at the next flush, when the round trip (~1 us) has long completed. (Waiting
-    // for every atomicAdd was 40 % of the samples of a candidate-dense level.)
-    uint32_t* hit_buf = reinterpret_cast<uint32_t*>(gbase + L.hits) + etid * (2 * T5_HITS);
-    uint32_t* my_hits = hit_buf;
-    int nh = 0, cur_half = 0, pend_n = 0;
-    uint32_t pend_slot = 0;
-    auto drain_pending = [&]() {  // copy out the half reserved by the previous flush
-      const uint32_t* src = hit_buf + (cur_half ^ 1) * T5_HITS;
-      uint32_t slot = pend_slot;
-      for (int i = 0; i < pend_n; ++i, ++slot)
-        if (slot < CAND_CAP) a.cand[size_t(q) * CAND_CAP + slot] = src[i];
-      pend_n = 0;
-    };
-    auto flush_hits = [&]() {
-      drain_pending();
-      if (nh && q_ok) {
-        pend_slot = atomicAdd(&a.cand_cnt[q], uint32_t(nh));
-        pend_n = nh;
-      }
-      cur_half ^= 1;
-      my_hits = hit_buf + cur_half * T5_HITS;
-      nh = 0;
-    };
-    uint32_t it = 0;
-    for (uint32_t t = tile_begin; t < tile_end; ++t, ++it) {
-      const uint32_t acc = it & 1u, aph = (it >> 1) & 1u;
-      const uint32_t p0 = a.first_id + t * 256;
-      t5_mbar_wait(bar_tfull(acc), aph);
-      t5_fence_after();
-      const uint32_t taddr = tmem_base + (uint32_t(quad * 32) << 16) + acc * 256 + uint32_t(col0);
-      uint32_t v[2][32];
-      t5_ld32(taddr, v[0]);
-#pragma unroll
-      for (int c = 0; c < 4; ++c) {
-        t5_wait_ld();
-        if (c + 1 < 4) t5_ld32(taddr + uint32_t(c + 1) * 32, v[(c + 1) & 1]);
-        uint32_t mask = 0;
-#pragma unroll
-        for (int j = 0; j < 32; ++j) mask = __funnelshift_l(v[c & 1][j], mask, 1);
-        while (mask) {
-          const int j = __clz(mask);
-          mask &= ~(0x80000000u >> j);
-          my_hits[nh++] = p0 + uint32_t(col0) + uint32_t(c) * 32 + uint32_t(j);
-          if (nh == T5_HITS) flush_hits();
-        }
-      }
-      t5_fence_before();
-      __syncwarp();
-      if (lane == 0) t2_arrive_leader(bar_tempty(acc));
-    }
-    flush_hits();
-    drain_pending();
-  }
-  t5_fence_before();
-  __syncthreads();
-  t2_cluster_sync();  // nobody leaves while the peer may still read this CTA's shared memory or signal its barriers
-  if (warp == 1) {
-    t5_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
-  }
-}
-
 PFN_cuTensorMapEncodeTiled_v12000 t5_encode_fn() {
   static PFN_cuTensorMapEncodeTiled_v12000 fn = nullptr;
   if (!fn) {
@@ -1073,36 +826,6 @@ int launch_tc5_filter(sdb_index* ix, TcArgs ta, uint32_t B_pad, cudaStream_t str
   ta.tiles_per_cta = (ntiles + ysplit - 1) / ysplit;
   if (ta.gmin) ta.tiles_per_cta = (ta.tiles_per_cta + ta.fold - 1) / ta.fold * ta.fold;  // a group never spans two CTAs
   ysplit = (ntiles + ta.tiles_per_cta - 1) / ta.tiles_per_cta;
-  if (!ta.gmin && getenv("SDB_FLAT_2CTA") && qtiles % 2 == 0) {
-    // two-SM variant: X maps with 128-row boxes (each CTA loads its half of a point tile)
-    const uint32_t fixed2 = t2_layout(nkb, 0).total + 1024;
-    int st2 = int((227u * 1024u - fixed2) / T2_XBLK_BYTES);
-    if (st2 > 8) st2 = 8;
-    const size_t smem2 = size_t(t2_layout(nkb, st2).total) + 1024;
-    CUtensorMap mx2, mxe2;
-    if ((rc = t5_make_map(&mx2, ta.x16, ta.rows_alloc, ta.pitch, 128, T5_KB)) || (rc = t5_make_map(&mxe2, ta.x16, ta.rows_alloc, ta.pitch, 128, 16)))
-      return rc;
-    static size_t attr2_dev[64] = {};
-    if (attr2_dev[ix->device & 63] < smem2) {
-      SDB_CUDA(cudaFuncSetAttribute(tc5x2_filter_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem2)));
-      attr2_dev[ix->device & 63] = smem2;
-    }
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3(qtiles, ysplit);
-    cfg.blockDim = dim3(T5_THREADS);
-    cfg.dynamicSmemBytes = smem2;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 2;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    SDB_CUDA(cudaLaunchKernelEx(&cfg, tc5x2_filter_kernel, mq, mx2, mqe, mxe2, ta, st2));
-    SDB_CUDA(cudaGetLastError());
-    return SDB_OK;
-  }
   tc5_filter_kernel<<<dim3(qtiles, ysplit), T5_THREADS, smem, stream>>>(mq, mx, mqe, mxe, ta, stages);
   SDB_CUDA(cudaGetLastError());
   return SDB_OK;
@@ -1269,139 +992,6 @@ __global__ void __launch_bounds__(32 * RW_WARPS) rescore_warp_kernel(
   if (lane == 0) out_cnt[q] = len;
 }
 
-// Exact re-score of one query's candidates + top-k by (distance asc, id asc). One CTA per query.
-template <int METRIC>
-__global__ void __launch_bounds__(128) rescore_kernel(const float* vec, uint32_t vec_pitch, uint32_t dim, const float* queries,
-                                                      const uint32_t* cand, const uint32_t* cand_cnt, uint32_t k,
-                                                      uint64_t* out_ids, float* out_d, uint32_t* out_cnt,
-                                                      uint32_t* overflow_list, uint32_t* overflow_cnt, uint32_t* overflow_flag,
-                                                      int last_level) {
-  __shared__ float s_d[CAND_CAP];
-  __shared__ uint32_t s_id[CAND_CAP];
-  __shared__ float s_bd[4];
-  __shared__ uint32_t s_bi[4], s_bp[4];
-  extern __shared__ __align__(16) float s_q[];  // [dim rounded up to 4]
-  const uint32_t q = blockIdx.x;
-  const int tid = threadIdx.x, lane = tid & 31, g = lane & 7, grp = tid >> 3;  // 16 groups
-  const uint32_t n = cand_cnt[q];
-  if (n > CAND_CAP) {
-    // Levels cover disjoint point ranges, so a list that overflowed at any level has lost
-    // candidates for good: the query goes to the exact scan after the last level (once: the
-    // per-query flag). Its outputs of this level stay as they were (the previous bound).
-    if (tid == 0) {
-      if (atomicExch(&overflow_flag[q], 1u) == 0u) overflow_list[atomicAdd(overflow_cnt, 1u)] = q;
-      if (last_level) out_cnt[q] = 0;
-    }
-    return;
-  }
-  for (uint32_t i = tid; i < ((dim + 3) & ~3u); i += blockDim.x) s_q[i] = i < dim ? queries[size_t(q) * dim + i] : 0.0f;
-  __syncthreads();
-  constexpr bool L2 = (METRIC == METRIC_EUCLIDEAN);
-  const int trips = dim >> 5;
-  uint32_t c0 = 0;
-  if (trips <= 4) {
-    // rows of up to 4 trips: four candidates per 8-lane group per step, all 16 row loads of a
-    // lane in flight before the first is consumed (the gather is latency-bound otherwise)
-    for (; c0 < n; c0 += 64) {
-      float4 y[4][4];
-      uint32_t pid[4];
-#pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        const uint32_t c = c0 + u * 16 + grp;
-        pid[u] = cand[size_t(q) * CAND_CAP + (c < n ? c : 0)];
-        const float* row = vec + size_t(pid[u]) * vec_pitch + 4 * g;
-#pragma unroll
-        for (int t = 0; t < 4; ++t) y[u][t] = t < trips ? ldg_f4_stream(row + 32 * t) : make_float4(0.f, 0.f, 0.f, 0.f);
-      }
-#pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        const uint32_t c = c0 + u * 16 + grp;
-        const float* row = vec + size_t(pid[u]) * vec_pitch;
-        float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll
-        for (int t = 0; t < 4; ++t)
-          if (t < trips) trip_accum<L2>(*reinterpret_cast<const float4*>(s_q + 32 * t + 4 * g), y[u][t], acc);
-        float tail = 0.0f;
-        if (g == 0)
-          for (uint32_t i = trips << 5; i < dim; ++i) tail = tail_accum<L2>(s_q[i], __ldg(row + i), tail);
-        const float r = group_reduce(acc, tail);
-        if (g == 0 && c < n) {
-          s_d[c] = metric_epilogue<METRIC>(r);
-          s_id[c] = pid[u];
-        }
-      }
-    }
-  }
-  for (; c0 < n; c0 += 16) {
-    const uint32_t c = c0 + grp;
-    const bool act = c < n;
-    const uint32_t pid = cand[size_t(q) * CAND_CAP + (act ? c : 0)];
-    const float* row = vec + size_t(pid) * vec_pitch;
-    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-    for (int t = 0; t < trips; ++t) {
-      const float4 x = *reinterpret_cast<const float4*>(s_q + 32 * t + 4 * g);
-      const float4 y = ldg_f4(row + 32 * t + 4 * g);
-      trip_accum<L2>(x, y, acc);
-    }
-    float tail = 0.0f;
-    if (g == 0)
-      for (uint32_t i = trips << 5; i < dim; ++i) tail = tail_accum<L2>(s_q[i], __ldg(row + i), tail);
-    const float r = group_reduce(acc, tail);
-    if (g == 0 && act) {
-      s_d[c] = metric_epilogue<METRIC>(r);
-      s_id[c] = pid;
-    }
-  }
-  __syncthreads();
-  // k rounds of block-wide arg-min over (distance, id)
-  const uint32_t kk = min(k, n);
-  for (uint32_t r = 0; r < kk; ++r) {
-    float bd = INFINITY;
-    uint32_t bi = 0xFFFFFFFFu, bp = 0xFFFFFFFFu;
-    for (uint32_t i = tid; i < n; i += blockDim.x) {
-      const float d = s_d[i];
-      const uint32_t id = s_id[i];
-      if (id != 0xFFFFFFFFu && (d < bd || (d == bd && id < bi) || bp == 0xFFFFFFFFu)) { bd = d; bi = id; bp = i; }
-    }
-    for (int o = 16; o >= 1; o >>= 1) {
-      const float od = __shfl_xor_sync(SDB_FULL, bd, o);
-      const uint32_t oi = __shfl_xor_sync(SDB_FULL, bi, o), op = __shfl_xor_sync(SDB_FULL, bp, o);
-      if (op != 0xFFFFFFFFu && (bp == 0xFFFFFFFFu || od < bd || (od == bd && oi < bi))) { bd = od; bi = oi; bp = op; }
-    }
-    if (lane == 0) { s_bd[tid >> 5] = bd; s_bi[tid >> 5] = bi; s_bp[tid >> 5] = bp; }
-    __syncthreads();
-    if (tid == 0) {
-      for (int w = 1; w < 4; ++w)
-        if (s_bp[w] != 0xFFFFFFFFu && (bp == 0xFFFFFFFFu || s_bd[w] < bd || (s_bd[w] == bd && s_bi[w] < bi))) {
-          bd = s_bd[w]; bi = s_bi[w]; bp = s_bp[w];
-        }
-      out_ids[size_t(q) * k + r] = bi;
-      out_d[size_t(q) * k + r] = bd;
-      s_id[bp] = 0xFFFFFFFFu;  // taken
-    }
-    __syncthreads();
-  }
-  for (uint32_t r = kk + tid; r < k; r += blockDim.x) {
-    out_ids[size_t(q) * k + r] = 0;
-    out_d[size_t(q) * k + r] = __int_as_float(0x7f800000);
-  }
-  if (tid == 0) out_cnt[q] = kk;
-}
-
-__global__ void sum_counts_kernel(const uint32_t* cnt, uint32_t n, unsigned long long* out) {
-  __shared__ unsigned long long part[8];
-  unsigned long long v = 0;
-  for (uint32_t i = threadIdx.x; i < n; i += blockDim.x) v += cnt[i];
-  for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xFFFFFFFFu, v, o);
-  if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = v;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    unsigned long long t = 0;
-    for (uint32_t w = 0; w < blockDim.x / 32; ++w) t += part[w];
-    *out = t;
-  }
-}
-
 __global__ void gather_queries_kernel(const uint32_t* list, uint32_t n, const float* src, uint32_t dim, float* dst) {
   const uint32_t i = blockIdx.x;
   if (i >= n) return;
@@ -1421,28 +1011,12 @@ __global__ void scatter_results_kernel(const uint32_t* list, uint32_t n, uint32_
 
 }  // namespace
 
-static uint32_t level0_points() {
-  if (const char* e = getenv("SDB_FLAT_LEVEL0")) {
-    const int v = atoi(e);
-    if (v >= 32 && v <= 65536) return uint32_t(v);
-  }
-  return LEVEL0;
-}
-
-// growth of the levels: intermediate levels multiply the covered prefix by ratio_mid, the last level
-// may cover up to ratio_last times the prefix before it (a level's re-score handles ~k * ratio
+// growth of the levels: intermediate levels multiply the covered prefix by LEVEL_MID, the last level
+// may cover up to LEVEL_LAST times the prefix before it (a level's re-score handles ~k * ratio
 // candidates per query; the intermediate re-scores only serve the next threshold, so they are kept
-// small). A/B: SDB_FLAT_RATIO="mid,last".
-static void level_ratios(uint32_t* mid, uint32_t* last) {
-  // measured on 10k x 1M x 128 (host buffers in and out): 32,32 4.64 ms; 16,32 4.83; 8,32 4.19; 8,64 4.25;
-  // 4,32 4.40; 8,16 4.13 ms
-  *mid = 8;
-  *last = 16;
-  if (const char* e = getenv("SDB_FLAT_RATIO")) {
-    int a = 0, b = 0;
-    if (sscanf(e, "%d,%d", &a, &b) == 2 && a >= 2 && a <= 256 && b >= 2 && b <= 256) { *mid = uint32_t(a); *last = uint32_t(b); }
-  }
-}
+// small). Measured on 10k x 1M x 128 (host buffers in and out), mid,last: 32,32 4.64 ms; 16,32 4.83;
+// 8,32 4.19; 8,64 4.25; 4,32 4.40; 8,16 4.13 ms
+static constexpr uint32_t LEVEL_MID = 8, LEVEL_LAST = 16;
 
 bool flat_tc_eligible(const sdb_index* ix, uint32_t k, bool filtered) {
   if (getenv("SDB_FLAT_EXACT")) return false;
@@ -1450,7 +1024,7 @@ bool flat_tc_eligible(const sdb_index* ix, uint32_t k, bool filtered) {
   if (ix->store_metric != SDB_METRIC_EUCLIDEAN && ix->store_metric != SDB_METRIC_DOT && ix->store_metric != SDB_METRIC_COSINE)
     return false;
   const uint32_t end_id = std::max<uint32_t>(2, ix->max_node_id + 1);
-  return end_id - 2 >= LEVEL0 * LEVEL_RATIO && k <= 75;  // (with the default LEVEL0)
+  return end_id - 2 >= LEVEL0 * LEVEL_RATIO && k <= 75;
 }
 
 int launch_flat_tc(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, uint64_t* d_out_ids, float* d_out_dists,
@@ -1465,11 +1039,10 @@ int launch_flat_tc(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k
   const uint32_t pitch = kp + T5_KB;  // one more 64-wide K block: the extension (bias / threshold pieces)
   const bool l2 = ix->store_metric == SDB_METRIC_EUCLIDEAN;
   // squared-L2: the shadow holds x - mu (mu = mean of a sample of the rows), see to_bf16_kernel
-  const int center = (l2 && !getenv("SDB_FLAT_NO_CENTER")) ? 1 : 0;
-  if (ix->tc_epoch != ix->vec_epoch || ix->d_x16.n < size_t(rows_pad) * pitch || ix->tc_centered != center) {
+  if (ix->tc_epoch != ix->vec_epoch || ix->d_x16.n < size_t(rows_pad) * pitch) {
     if ((rc = ix->d_x16.ensure(size_t(rows_pad) * pitch)) || (rc = ix->d_xn.ensure(rows_pad)) || (rc = ix->d_bias.ensure(rows_pad)))
       return rc;
-    if (center) {
+    if (l2) {
       if ((rc = ix->d_mu.ensure(size_t(MU_PARTS + 1) * dim + MU_PARTS))) return rc;
       float* partial = ix->d_mu.p + dim;
       uint32_t* cnt = reinterpret_cast<uint32_t*>(ix->d_mu.p + size_t(MU_PARTS + 1) * dim);
@@ -1481,13 +1054,12 @@ int launch_flat_tc(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k
       mean_final_kernel<<<(dim + 127) / 128, 128, 0, stream>>>(partial, cnt, dim, ix->d_mu.p);
       ix->launches += 2;
     }
-    ix->tc_centered = center;
     to_bf16_kernel<<<(rows_pad + 7) / 8, 256, 0, stream>>>(ix->d_vec, ix->vec_pitch, dim, ix->rows, rows_pad,
                                                           reinterpret_cast<__nv_bfloat16*>(ix->d_x16.p), kp, pitch, 1.0f, ix->d_xn.p,
-                                                          center ? ix->d_mu.p : nullptr);
+                                                          l2 ? ix->d_mu.p : nullptr);
     bias_kernel<<<(rows_pad + 255) / 256, 256, 0, stream>>>(ix->d_xn.p, ix->d_exists, ix->rows, rows_pad, l2 ? 1 : 0, ix->d_bias.p,
                                                             reinterpret_cast<__nv_bfloat16*>(ix->d_x16.p), kp, pitch);
-    // largest squared norm of a stored row (of the centred rows if centred): part of the candidate bound
+    // largest squared norm of a stored row (of the centred rows for squared-L2): part of the candidate bound
     if ((rc = ix->d_xmax.ensure(1))) return rc;
     SDB_CUDA(cudaMemsetAsync(ix->d_xmax.p, 0, sizeof(uint32_t), stream));
     xmax_kernel<<<(end_id - first_id + 255) / 256, 256, 0, stream>>>(ix->d_xn.p, ix->d_exists, first_id, end_id, ix->d_xmax.p);
@@ -1507,26 +1079,23 @@ int launch_flat_tc(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k
   uint32_t* d_ovf_flag = d_misc + 8;                   // [B] query already on the overflow list
   SDB_CUDA(cudaMemsetAsync(d_misc, 0, (8 + size_t(B)) * sizeof(uint32_t), stream));
   to_bf16_kernel<<<(B_pad + 7) / 8, 256, 0, stream>>>(d_queries, dim, dim, B, B_pad, reinterpret_cast<__nv_bfloat16*>(ix->d_q16.p),
-                                                     kp, pitch, l2 ? -2.0f : -1.0f, ix->d_qn.p, center ? ix->d_mu.p : nullptr);
+                                                     kp, pitch, l2 ? -2.0f : -1.0f, ix->d_qn.p, l2 ? ix->d_mu.p : nullptr);
   ix->launches += 1;
   SDB_CUDA(cudaGetLastError());
   static bool attr_set_dev[64] = {};  // cudaFuncSetAttribute is per device
   bool& attr_set = attr_set_dev[ix->device & 63];
   if (!attr_set) {
     SDB_CUDA(cudaFuncSetAttribute(tc_filter_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(TC_SMEM)));
-    // the re-score kernels keep queries in dynamic shared memory: RW_WARPS rows pass the 48 KB
-    // default from dim 3 073, one row next to rescore_kernel's static lists from dim ~4 084
-    const int wmax = int(RW_WARPS * MAX_DIM * sizeof(float)), cmax = int(MAX_DIM * sizeof(float));
+    // the re-score kernel keeps queries in dynamic shared memory: RW_WARPS rows pass the 48 KB
+    // default from dim 3 073
+    const int wmax = int(RW_WARPS * MAX_DIM * sizeof(float));
     for (auto kern : {rescore_warp_kernel<METRIC_EUCLIDEAN, 1>, rescore_warp_kernel<METRIC_EUCLIDEAN, 3>,
                       rescore_warp_kernel<METRIC_DOT, 1>, rescore_warp_kernel<METRIC_DOT, 3>,
                       rescore_warp_kernel<METRIC_COSINE, 1>, rescore_warp_kernel<METRIC_COSINE, 3>})
       SDB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, wmax));
-    for (auto kern : {rescore_kernel<METRIC_EUCLIDEAN>, rescore_kernel<METRIC_DOT>, rescore_kernel<METRIC_COSINE>})
-      SDB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, cmax));
     attr_set = true;
   }
-  // ---- level 0: exact scan of the first LEVEL0 points bounds every query's k-th distance
-  const bool warp_rescore = getenv("SDB_FLAT_RESCORE_CTA") == nullptr;
+  // ---- exact re-score + top-k, one warp per query (rescore_warp_kernel)
   const size_t wsmem = size_t(RW_WARPS) * ((dim + 3) & ~3u) * sizeof(float);
   unsigned long long* d_cand_total = reinterpret_cast<unsigned long long*>(d_misc + 2);  // summed by the last re-score
   auto rescore_warp = [&](uint64_t* o_ids, float* o_d, uint32_t* o_c, int last, uint32_t impl_first, uint32_t impl_n) {
@@ -1558,7 +1127,7 @@ int launch_flat_tc(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k
   // the mma.sync pass and as SDB_FLAT_LEVELS=1.
   uint32_t tiles_a = 0, fold = 1;
   const uint32_t whole_tiles = npts / T5_N;
-  if (t5_eligible(kp) && warp_rescore && !getenv("SDB_FLAT_LEVELS")) {
+  if (t5_eligible(kp) && !getenv("SDB_FLAT_LEVELS")) {
     uint32_t div = 8;  // sample = 1/8 of the points: ~8 k candidates per query before the error margin
     if (const char* e = getenv("SDB_FLAT_SAMPLE_DIV")) { const int v = atoi(e); if (v >= 1 && v <= 4096) div = uint32_t(v); }
     const uint32_t whole = whole_tiles;  // whole tiles only
@@ -1602,23 +1171,16 @@ int launch_flat_tc(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k
               tiles_a * T5_N, G, double(tot) / B, mx, CAND_CAP);
     }
   } else {
-  if (warp_rescore) {
-    rescore_warp(ix->d_sample_ids.p, ix->d_sample_d.p, ix->d_sample_cnt.p, 0, first_id,
-                 std::min<uint32_t>(level0_points(), end_id - first_id));
-    ix->launches++;
-    SDB_CUDA(cudaGetLastError());
-  } else if ((rc = launch_flat_exact(ix, B, d_queries, k, nullptr, ix->d_sample_ids.p, ix->d_sample_d.p, ix->d_sample_cnt.p, stream,
-                                     first_id, first_id + level0_points())))
-    return rc;
+  // ---- level 0: exact scan of the first LEVEL0 points bounds every query's k-th distance
+  rescore_warp(ix->d_sample_ids.p, ix->d_sample_d.p, ix->d_sample_cnt.p, 0, first_id, std::min<uint32_t>(LEVEL0, end_id - first_id));
+  ix->launches++;
+  SDB_CUDA(cudaGetLastError());
   // ---- levels 1..: tensor-core pass over a 32x larger prefix, thresholds from the level before
   const uint32_t qtiles = B_pad / TM;
-  const size_t qsmem = size_t((dim + 3) & ~3u) * sizeof(float);
-  uint64_t covered = level0_points();
+  uint64_t covered = LEVEL0;
   uint32_t lvl_begin = first_id + uint32_t(covered);  // levels cover disjoint ranges [lvl_begin, lvl_end)
-  uint32_t ratio_mid, ratio_last;
-  level_ratios(&ratio_mid, &ratio_last);
   while (covered < npts) {
-    covered = covered * ratio_last >= npts ? npts : std::min<uint64_t>(npts, covered * ratio_mid);
+    covered = covered * LEVEL_LAST >= npts ? npts : std::min<uint64_t>(npts, covered * LEVEL_MID);
     // whole 256-point tiles: what a level scans past its nominal end is not scanned again
     uint64_t span = (first_id + covered - lvl_begin + 255) / 256 * 256;
     const bool last = lvl_begin + span >= end_id;
@@ -1654,21 +1216,7 @@ int launch_flat_tc(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k
     uint64_t* o_ids = last ? d_out_ids : ix->d_sample_ids.p;
     float* o_d = last ? d_out_dists : ix->d_sample_d.p;
     uint32_t* o_c = last ? d_out_counts : ix->d_sample_cnt.p;
-    if (warp_rescore) rescore_warp(o_ids, o_d, o_c, last ? 1 : 0, 0, 0);
-    else switch (ix->store_metric) {
-      case SDB_METRIC_EUCLIDEAN:
-        rescore_kernel<METRIC_EUCLIDEAN><<<B, 128, qsmem, stream>>>(ix->d_vec, ix->vec_pitch, dim, d_queries, ix->d_cand.p, d_cnt, k,
-                                                                    o_ids, o_d, o_c, d_ovf_list, d_misc + 1, d_ovf_flag, last ? 1 : 0);
-        break;
-      case SDB_METRIC_DOT:
-        rescore_kernel<METRIC_DOT><<<B, 128, qsmem, stream>>>(ix->d_vec, ix->vec_pitch, dim, d_queries, ix->d_cand.p, d_cnt, k, o_ids,
-                                                              o_d, o_c, d_ovf_list, d_misc + 1, d_ovf_flag, last ? 1 : 0);
-        break;
-      default:
-        rescore_kernel<METRIC_COSINE><<<B, 128, qsmem, stream>>>(ix->d_vec, ix->vec_pitch, dim, d_queries, ix->d_cand.p, d_cnt, k,
-                                                                 o_ids, o_d, o_c, d_ovf_list, d_misc + 1, d_ovf_flag, last ? 1 : 0);
-        break;
-    }
+    rescore_warp(o_ids, o_d, o_c, last ? 1 : 0, 0, 0);
     ix->launches += 3;
     SDB_CUDA(cudaGetLastError());
     if (debug) {
@@ -1686,11 +1234,7 @@ int launch_flat_tc(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k
   }  // level scheme
   // ---- queries whose candidate list overflowed at some level: exact scan
   // [1] overflow count, [2..3] diagnostic (sdb_flat_last_stats): candidates the last level kept, summed
-  // over the batch on the device (a 16-byte read-back instead of the B counts)
-  if (!warp_rescore) {  // (the warp re-score of the last level has summed them already)
-    sum_counts_kernel<<<1, 256, 0, stream>>>(d_cnt, B, reinterpret_cast<unsigned long long*>(d_misc + 2));
-    ix->launches++;
-  }
+  // over the batch by the last re-score (a 16-byte read-back instead of the B counts)
   // host-buffer call (sdb_flat_search_batch): the result copies go in front of the one synchronisation
   auto copy_out = [&]() -> int {
     const auto& ho = ix->flat_host_out;

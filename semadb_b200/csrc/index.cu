@@ -237,7 +237,6 @@ int sdb_index_create(const sdb_params* params, sdb_index** out) {
   ix->words = (p.dim + 63) / 64;
   ix->bits_pitch = (ix->words + 1) / 2 * 2;
   ix->store_metric = p.metric;
-  if (const char* g = getenv("SDB_GEO_CTAS")) ix->geo_ctas_per_sm = atoi(g);  // A/B runs of the geo search (search_geo.cu)
   if (p.quantizer == SDB_QUANT_BINARY) {
     ix->bq_metric = p.bq_metric;
     if ((e = cudaMalloc(reinterpret_cast<void**>(&ix->d_bq_thr), p.dim * sizeof(float))) != cudaSuccess) {
@@ -587,9 +586,7 @@ static int search_batch_locked(sdb_index* ix, uint32_t B, const float* queries, 
   // once straight from host memory (512 B per query, when a warp picks the query up) and stores
   // the top-k straight back, so the copies disappear from the critical path instead of preceding
   // and following the kernel. Pageable buffers go through the staging copies.
-  const bool zero_copy = getenv("SDB_NO_ZEROCOPY") == nullptr;
   auto mapped = [&](const void* p) -> void* {
-    if (!zero_copy) return nullptr;
     cudaPointerAttributes at;
     if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { cudaGetLastError(); return nullptr; }
     return at.type == cudaMemoryTypeHost ? at.devicePointer : nullptr;

@@ -148,13 +148,11 @@ struct sdb_index {
   sdb::DevBuf<float> d_bias;  // tcgen05 flat pass: per-point score bias (|x|^2 or 0; +inf = no such point)
   sdb::DevBuf<float> d_mu;    // squared-L2: translation applied to the bf16 shadow and the queries (+ partial sums)
   sdb::DevBuf<float> d_gmin;  // tcgen05 flat pass, minimum mode: [groups][B_pad] smallest approximate scores
-  int tc_centered = -1;       // whether the current shadow is centred
   sdb::DevBuf<uint32_t> d_xmax;  // bits of the largest squared norm of a (centred) stored row
   sdb::DevBuf<uint32_t> d_cand, d_candcnt, d_sample_cnt;
   sdb::DevBuf<uint64_t> d_sample_ids;
   uint32_t last_B = 0;
   int vt_level = 0;                  // visited-table size step (search.cu)
-  int geo_ctas_per_sm = 0;           // geo beam search: CTAs/SM cap for A/B runs, SDB_GEO_CTAS read at create (0 = kernel's bound)
   bool retry_check_pending = false;  // d_work holds the retry count of the last search
   cudaStream_t last_search_stream = nullptr;
   uint64_t launches = 0;

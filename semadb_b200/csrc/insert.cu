@@ -46,7 +46,6 @@ struct InsertArgs {
   uint32_t* pair_val;        // [m*R] pair index (batch order)
   int staged_max;            // rows that fit in shared memory
   uint32_t* error_flag;
-  int matrix_max;            // robustPrune: all-pairs bit matrix up to this many candidates
   const uint32_t* ndist;     // [m] distance evaluations of each point's search
   unsigned long long* stats; // running totals for sdb_insert_stats
 };
@@ -71,7 +70,10 @@ __global__ void __launch_bounds__(PRUNE_THREADS) prune_new_kernel(InsertArgs a) 
   stable_sort_by_dist(sh);
   int staged = min(int(n), a.staged_max);
   stage_rows(a.s, sh, dyn, staged);
-  robust_prune_cta(a.s, sh, dyn, staged, A, int(a.R), a.alpha, a.matrix_max);
+  // the sequential robustPrune: a new point's ~80-100 candidates end the walk of search.go:106-138
+  // at R accepted edges with removed candidates skipped, about a third of the pairs — 0.127 s against
+  // 0.218 s for the all-pairs matrix per 1M-point build (a back-edge target's R+1: the matrix wins)
+  robust_prune_cta_seq(a.s, sh, dyn, staged, A, int(a.R), a.alpha);
   const int cnt = *sh.cnt;
   for (uint32_t t = threadIdx.x; t < a.R; t += blockDim.x) {
     uint32_t e = t < uint32_t(cnt) ? sh.edges[t] : INVALID_ID;
@@ -117,7 +119,6 @@ struct BackArgs {
   const uint32_t* seg_count;
   uint32_t* prune_list;        // segments whose target overflows (written by backedge_append_kernel)
   uint32_t* prune_count;
-  int matrix_max;
   int staged_max;
   unsigned long long* stats;
 };
@@ -219,7 +220,7 @@ __global__ void __launch_bounds__(PRUNE_THREADS) backedge_kernel(BackArgs a) {
       stable_sort_by_dist(sh);  // candidateSet.Sort() (insert.go:58)
       int staged = min(n, a.staged_max);
       stage_rows(a.s, sh, dyn, staged);
-      robust_prune_cta(a.s, sh, dyn, staged, B, int(a.R), a.alpha, a.matrix_max);
+      robust_prune_cta(a.s, sh, dyn, staged, B, int(a.R), a.alpha);
       cur_n = *sh.cnt;
       for (int t = threadIdx.x; t < cur_n; t += blockDim.x) cur[t] = sh.edges[t];
       p += uint32_t(c);
@@ -377,12 +378,6 @@ int insert_batch_locked(sdb_index* ix, uint64_t n, const uint64_t* ids, const fl
   INS_CUDA(cudaFuncGetAttributes(&fa, backedge_kernel));
   static_smem = std::max(static_smem, fa.sharedSizeBytes);
 
-  // A/B knobs: candidate-count limit of the all-pairs robustPrune for new points / back-edge targets
-  // (a new point's ~80-100 candidates: the walk of search.go:106-138 stops at R accepted edges and
-  // skips removed candidates, so it evaluates about a third of the pairs — the sequential form wins
-  // there, 0.127 s vs 0.218 s per 1M-point build; a back-edge target's R+1: the matrix wins)
-  const int mm_new = getenv("SDB_PRUNE_MM_NEW") ? atoi(getenv("SDB_PRUNE_MM_NEW")) : 0;
-  const int mm_back = getenv("SDB_PRUNE_MM_BACK") ? atoi(getenv("SDB_PRUNE_MM_BACK")) : PruneShared::MATRIX_MAX;
   const bool debug = getenv("SDB_DEBUG_INSERT") != nullptr;
   uint64_t inserted_before = ix->count > 0 ? ix->count - 1 : 0;  // user points already in the graph
   for (uint64_t c0 = 0; c0 < n; c0 += chunk_pts) {
@@ -409,7 +404,6 @@ int insert_batch_locked(sdb_index* ix, uint64_t n, const uint64_t* ids, const fl
     // ... and the R+1 candidates of a back-edge prune all of them when that costs one more row (dim 128:
     // 65 x 512 B): the all-pairs pass then runs on shared memory only
     if (staged_max == int(R) && size_t(R + 1) * view.row_bytes <= dyn_budget) staged_max = int(R) + 1;
-    if (const char* e = getenv("SDB_STAGED_MAX")) staged_max = std::max(1, std::min(staged_max, atoi(e)));  // A/B knob
     size_t dyn_smem = PruneShared::bytes(MAX_CAND + 1) + size_t(staged_max) * view.row_bytes;
     INS_CUDA(cudaFuncSetAttribute(prune_new_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(dyn_smem)));
     INS_CUDA(cudaFuncSetAttribute(backedge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(dyn_smem)));
@@ -438,7 +432,7 @@ int insert_batch_locked(sdb_index* ix, uint64_t n, const uint64_t* ids, const fl
       ia.new_ids = b_ids; ia.vis_ids = ix->d_vis_ids.p; ia.vis_dists = ix->d_vis_d.p; ia.vis_len = ix->d_vis_len.p;
       ia.vis_cap = vis_cap; ia.m = m; ia.pair_key = d_pair_key.p; ia.pair_val = d_pair_val.p;
       ia.staged_max = staged_max; ia.error_flag = d_err;
-      ia.ndist = ix->d_ndist.p; ia.stats = ix->d_ins_stats; ia.matrix_max = mm_new;
+      ia.ndist = ix->d_ndist.p; ia.stats = ix->d_ins_stats;
       prune_new_kernel<<<m, PRUNE_THREADS, dyn_smem, st>>>(ia);
       ix->launches++;
       INS_CUDA(cudaGetLastError());
@@ -466,7 +460,7 @@ int insert_batch_locked(sdb_index* ix, uint64_t n, const uint64_t* ids, const fl
       ba.s = view; ba.adj = ix->d_adj; ba.deg = ix->d_deg; ba.dirty = ix->d_dirty; ba.R = R; ba.alpha = ix->p.alpha;
       ba.new_ids = b_ids; ba.keys = skeys; ba.vals = svals; ba.n_pairs = np; ba.seg_start = d_seg.p;
       ba.seg_count = d_segcount; ba.staged_max = staged_max; ba.stats = ix->d_ins_stats;
-      ba.prune_list = d_plist.p; ba.prune_count = d_misc.p + 2; ba.matrix_max = mm_back;
+      ba.prune_list = d_plist.p; ba.prune_count = d_misc.p + 2;
       if (m == 1) {
         // a single new point: every target is its own segment, in edge order — no sort needed
         iota_segments_kernel<<<1, 64, 0, st>>>(skeys, np, d_seg.p, d_segcount);

@@ -185,13 +185,13 @@ __device__ inline void stage_rows(const StoreView& s, PruneShared& sh, unsigned 
 // The reference walks the candidates in ascending order; an accepted candidate p* removes every
 // later candidate c with alpha * d(p*, c) < d(node, c) (search.go:132, strict). Whether p* removes
 // c does not depend on the walk, only on the pair — so for lists of up to MATRIX_MAX candidates
-// (back-edge prunes have R+1 = 65, a new point's visited list ~80-100) all pairs (i < j) are
-// evaluated first, in parallel by the CTA's 8-lane groups with no barrier in the loop, into a
-// bit matrix kill[i] = {j : alpha * d(i, j) < sdist[j]}; one warp then replays the walk with bit
-// operations: skip removed / self, accept, stop at R, removed |= kill[i]. Same distances, same
-// comparisons, same edges as the sequential form (kept below for longer lists), which spent its
-// time in one block-wide barrier per accepted candidate (profiles/r01_ab_insert.txt: 30 % barrier
-// stalls in backedge_kernel).
+// (back-edge prunes have R+1 = 65) all pairs (i < j) are evaluated first, in parallel by the CTA's
+// 8-lane groups with no barrier in the loop, into a bit matrix kill[i] = {j : alpha * d(i, j) <
+// sdist[j]}; one warp then replays the walk with bit operations: skip removed / self, accept, stop
+// at R, removed |= kill[i]. Same distances, same comparisons, same edges as the sequential form
+// (kept below for longer lists, and for a new point's ~80-100 candidates, insert.cu), which spent
+// its time in one block-wide barrier per accepted candidate (profiles/r01_ab_insert.txt: 30 %
+// barrier stalls in backedge_kernel).
 __device__ inline void robust_prune_cta_seq(const StoreView& s, PruneShared& sh, const unsigned char* rows, int staged,
                                             uint32_t node, int R, float alpha) {
   const int n = sh.n;
@@ -263,14 +263,13 @@ __device__ __forceinline__ void prune_fill_kill(const StoreView& s, PruneShared&
 }
 
 __device__ inline void robust_prune_cta(const StoreView& s, PruneShared& sh, const unsigned char* rows, int staged,
-                                        uint32_t node, int R, float alpha, int matrix_max = PruneShared::MATRIX_MAX) {
+                                        uint32_t node, int R, float alpha) {
   const int n = sh.n;
-  if (n > matrix_max || n > PruneShared::MATRIX_MAX || sh.kill == nullptr) {
+  if (n > PruneShared::MATRIX_MAX || sh.kill == nullptr) {
     robust_prune_cta_seq(s, sh, rows, staged, node, R, alpha);
     return;
   }
   constexpr int KW = PruneShared::MATRIX_MAX / 32;
-  const int lane = threadIdx.x & 31;
   for (int t = threadIdx.x; t < n * KW; t += blockDim.x) sh.kill[t] = 0;
   __syncthreads();
   // the store's DistanceFromPoint, resolved once per prune rather than per pair. Fast path: f32 rows

@@ -102,10 +102,6 @@ int launch_search(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k,
     a.bitmap_words = words;
     ix->retry_slots = slots;
   }
-  {
-    const char* e = getenv("SDB_K1_FLAGS");
-    a.flags = e ? uint32_t(atoi(e)) : 0u;
-  }
   if (ix->gather) a.pg = *ix->gather;
   a.work_counter = ix->d_work.p;
   a.retry_count = ix->d_work.p + 1;

@@ -22,8 +22,6 @@
 #pragma once
 #include "common.cuh"
 
-#include <type_traits>
-
 namespace sdb {
 
 constexpr int LIST_SLOTS = 80;   // > max searchSize (75); lanes cover positions lane + 32j, j < 3
@@ -102,165 +100,9 @@ struct SearchArgs {
   // work distribution: work_counter hands out batch slots; a query whose visited table
   // overflows is appended to retry_list and re-run by the RETRY launch (bigger table).
   uint32_t vt_slots;  // VisitedCompactN slot count for this launch
-  uint32_t flags;  // tuning (A/B): bit 0 = probe the two ids of a lane one after the other
   uint32_t* work_counter;
   uint32_t* retry_list;
   uint32_t* retry_count;
-};
-
-// ---- exact visited set: open-addressed u32 hash in shared memory ------------------
-template <int HBITS>
-struct VisitedTable {
-  static constexpr uint32_t SLOTS = 1u << HBITS;
-  static constexpr uint32_t LIMIT = SLOTS - SLOTS / 8;  // refuse beyond 87.5 % load
-  static constexpr size_t BYTES = size_t(SLOTS) * 4;
-  static __host__ __device__ constexpr size_t bytes(uint32_t) { return BYTES; }
-  uint32_t* t;
-  bool failed;
-  __device__ __forceinline__ uint32_t limit() const { return LIMIT; }
-  __device__ __forceinline__ void init(unsigned char* base, uint32_t, uint32_t, uint32_t*, uint32_t) { t = reinterpret_cast<uint32_t*>(base); }
-  __device__ __forceinline__ void clear(int lane) {
-    uint4 e = make_uint4(INVALID_ID, INVALID_ID, INVALID_ID, INVALID_ID);
-    uint4* p = reinterpret_cast<uint4*>(t);
-    for (uint32_t i = lane; i < SLOTS / 4; i += 32) p[i] = e;
-    failed = false;
-  }
-  // true if id was NOT present (and is now) — CheckAndVisit negated (distset.go:105-111).
-  // Warp-convergent: every lane calls it (active = this lane has an id to test) and the
-  // probe loop is driven by a vote, so the compiler keeps the warp converged afterwards.
-  __device__ __forceinline__ bool test_and_set(uint32_t id, bool active, int) {
-    uint32_t slot = (id * 0x9E3779B1u) >> (32 - HBITS);
-    bool pending = active, isnew = false;
-    while (__any_sync(SDB_FULL, pending)) {
-      if (pending) {
-        uint32_t old = atomicCAS(&t[slot], INVALID_ID, id);
-        if (old == INVALID_ID) { isnew = true; pending = false; }
-        else if (old == id) pending = false;
-        else slot = (slot + 1) & (SLOTS - 1);
-      }
-    }
-    return isnew;
-  }
-  __device__ __forceinline__ void test_and_set2(uint32_t i0, bool a0, uint32_t i1, bool a1, bool& n0, bool& n1, int lane) {
-    n0 = test_and_set(i0, a0, lane);
-    n1 = test_and_set(i1, a1, lane);
-  }
-  __device__ __forceinline__ bool maybe_new(uint32_t) const { return true; }
-};
-
-// ---- exact visited set, compact form: 8192 x 16-bit entries + a 32-entry u32 stash ------
-// Ids are < rows <= 2^b. pi(id) = id*A mod 2^b (A odd) is a bijection on b bits; the top 13
-// bits of pi(id) pick the home slot and the low rb = b-13 bits are the remainder. An entry
-// stores 1 + rem + (disp << rb), disp = linear-probe displacement, so (slot, entry)
-// identifies the id exactly (quotienting) and 0 means empty. A probe that would need
-// disp > dmax = 2^(16-rb) - 2 cannot be encoded: the query is then re-run by the RETRY
-// launch (u32 table). dmax is 254 at 2M rows and 30 at 16M rows, so this is rare. Half the
-// footprint of the u32 table => twice the resident queries per SM.
-struct VisitedCompact {
-  static constexpr int HB = 13;
-  static constexpr uint32_t SLOTS = 1u << HB;
-  static constexpr uint32_t LIMIT = SLOTS - SLOTS / 8;
-  static constexpr size_t BYTES = SLOTS * 2;
-  static __host__ __device__ constexpr size_t bytes(uint32_t) { return BYTES; }
-  unsigned short* t;
-  uint32_t mask, rb, rmask, dmax;
-  bool failed;
-  __device__ __forceinline__ uint32_t limit() const { return LIMIT; }
-  __device__ __forceinline__ void init(unsigned char* base, uint32_t rows, uint32_t, uint32_t*, uint32_t) {
-    t = reinterpret_cast<unsigned short*>(base);
-    uint32_t b = rows <= SLOTS ? HB : 32 - __clz(rows - 1);
-    if (b < HB) b = HB;
-    rb = b - HB;
-    mask = b >= 32 ? 0xFFFFFFFFu : ((1u << b) - 1);
-    rmask = (1u << rb) - 1;
-    dmax = rb >= 15 ? 0 : ((1u << (16 - rb)) - 2);
-    if (dmax > 4096) dmax = 4096;
-  }
-  __device__ __forceinline__ void clear(int lane) {
-    uint4 z = make_uint4(0, 0, 0, 0);
-    uint4* p = reinterpret_cast<uint4*>(t);
-    for (uint32_t i = lane; i < SLOTS * 2 / 16; i += 32) p[i] = z;
-    failed = false;
-  }
-  __device__ __forceinline__ bool test_and_set(uint32_t id, bool active, int lane) {
-    const uint32_t v = (id * 0x9E3779B1u) & mask;
-    uint32_t slot = v >> rb;
-    const uint32_t code0 = 1 + (v & rmask);
-    uint32_t disp = 0;
-    bool pending = active, isnew = false, spill = false;
-    // 16-bit compare-and-swap done as a 32-bit CAS on the containing word, inside the same
-    // vote-driven loop (the library's 16-bit atomicCAS hides a divergent retry loop, which
-    // makes the compiler fall back to WARPSYNC.COLLECTIVE shuffles for the rest of the kernel)
-    volatile uint32_t* tw = reinterpret_cast<volatile uint32_t*>(t);
-    while (__any_sync(SDB_FULL, pending)) {
-      if (pending) {
-        const uint32_t code = code0 + (disp << rb);
-        const uint32_t sh = (slot & 1) * 16;
-        const uint32_t w = tw[slot >> 1];
-        const uint32_t half = (w >> sh) & 0xFFFFu;
-        if (half == 0) {
-          const uint32_t old = atomicCAS(const_cast<uint32_t*>(tw) + (slot >> 1), w, w | (code << sh));
-          if (old == w) { isnew = true; pending = false; }
-          // else: the word changed under us; re-read the same slot next round
-        } else if (half == code) {
-          pending = false;
-        } else {
-          slot = (slot + 1) & (SLOTS - 1);
-          if (++disp > dmax) { pending = false; spill = true; }
-        }
-      }
-    }
-    // a probe chain longer than dmax cannot be encoded: hand the query to the RETRY launch
-    if (__any_sync(SDB_FULL, spill)) failed = true;
-    return isnew;
-  }
-  // Two ids per lane (adjacency slots lane and lane+32) probed in one vote-driven loop: the
-  // two probe chains overlap instead of running back to back. Slot-0 ids are tried first
-  // inside an iteration, so a lane's own pair keeps adjacency order.
-  __device__ __forceinline__ void test_and_set2(uint32_t i0, bool a0, uint32_t i1, bool a1, bool& n0, bool& n1, int) {
-    const uint32_t v0 = (i0 * 0x9E3779B1u) & mask, v1 = (i1 * 0x9E3779B1u) & mask;
-    uint32_t slot0 = v0 >> rb, slot1 = v1 >> rb;
-    const uint32_t c0 = 1 + (v0 & rmask), c1 = 1 + (v1 & rmask);
-    uint32_t disp0 = 0, disp1 = 0;
-    bool p0 = a0, p1 = a1, spill = false;
-    n0 = false;
-    n1 = false;
-    volatile uint32_t* tw = reinterpret_cast<volatile uint32_t*>(t);
-    while (__any_sync(SDB_FULL, p0 || p1)) {
-      if (p0) {
-        const uint32_t code = c0 + (disp0 << rb);
-        const uint32_t sh = (slot0 & 1) * 16;
-        const uint32_t w = tw[slot0 >> 1];
-        const uint32_t half = (w >> sh) & 0xFFFFu;
-        if (half == 0) {
-          const uint32_t old = atomicCAS(const_cast<uint32_t*>(tw) + (slot0 >> 1), w, w | (code << sh));
-          if (old == w) { n0 = true; p0 = false; }
-        } else if (half == code) {
-          p0 = false;
-        } else {
-          slot0 = (slot0 + 1) & (SLOTS - 1);
-          if (++disp0 > dmax) { p0 = false; spill = true; }
-        }
-      }
-      if (p1) {
-        const uint32_t code = c1 + (disp1 << rb);
-        const uint32_t sh = (slot1 & 1) * 16;
-        const uint32_t w = tw[slot1 >> 1];
-        const uint32_t half = (w >> sh) & 0xFFFFu;
-        if (half == 0) {
-          const uint32_t old = atomicCAS(const_cast<uint32_t*>(tw) + (slot1 >> 1), w, w | (code << sh));
-          if (old == w) { n1 = true; p1 = false; }
-        } else if (half == code) {
-          p1 = false;
-        } else {
-          slot1 = (slot1 + 1) & (SLOTS - 1);
-          if (++disp1 > dmax) { p1 = false; spill = true; }
-        }
-      }
-    }
-    if (__any_sync(SDB_FULL, spill)) failed = true;
-  }
-  __device__ __forceinline__ bool maybe_new(uint32_t) const { return true; }
 };
 
 // ---- exact visited set, compact form with a launch-time slot count ------------------------
@@ -351,11 +193,6 @@ struct VisitedCompactN {
       if (p1) p1 = !step(b1, c1, d1, n1, spill);
     }
     if (__any_sync(SDB_FULL, spill)) failed = true;
-  }
-  __device__ __forceinline__ bool test_and_set(uint32_t id, bool active, int lane) {
-    bool n0, n1;
-    test_and_set2(id, active, 0, false, n0, n1, lane);
-    return n0;
   }
   // Read-only hint for the speculative row prefetch: false only if id is certainly in the set
   // (home bucket and the next one, no loop, no vote); "true" may be wrong, which costs one wasted
@@ -602,54 +439,6 @@ struct CandList {
 
 // ---- distance evaluators -----------------------------------------------------------
 // Each evaluates cdist[c] = dist(query, row cid[c]) for c in [0, n), warp-cooperatively.
-
-// (A/B baseline) f32 rows, dim = 32*TRIPS: batches of 4*UNROLL rows, no pipelining across batches.
-template <int METRIC, int TRIPS, int UNROLL>
-struct FloatEvalBatch {
-  static constexpr bool L2 = (METRIC == METRIC_EUCLIDEAN);
-  static constexpr bool QREG = (TRIPS <= 4);
-  float4 q[QREG ? TRIPS : 1];
-  const float* qs;
-  __device__ __forceinline__ void load_query(const float* qsmem, const float*, int lane) {
-    qs = qsmem;
-    if (QREG) {
-#pragma unroll
-      for (int t = 0; t < TRIPS; ++t) q[t] = *reinterpret_cast<const float4*>(qsmem + 32 * t + 4 * (lane & 7));
-    }
-  }
-  __device__ __forceinline__ void eval(const SearchArgs& a, const uint32_t* cid, float* cdist, int n, int lane) {
-    const int g = lane & 7, grp = lane >> 3;
-    for (int base = 0; base < n; base += 4 * UNROLL) {
-      float4 v[UNROLL][TRIPS];
-#pragma unroll
-      for (int u = 0; u < UNROLL; ++u) {
-        int ci = base + 4 * u + grp;
-        if (ci < n) {
-          const float* row = a.vec + size_t(cid[ci]) * a.vec_pitch + 4 * g;
-#pragma unroll
-          for (int t = 0; t < TRIPS; ++t) v[u][t] = ldg_f4_stream(row + 32 * t);
-        } else {
-#pragma unroll
-          for (int t = 0; t < TRIPS; ++t) v[u][t] = make_float4(0.f, 0.f, 0.f, 0.f);
-        }
-      }
-#pragma unroll
-      for (int u = 0; u < UNROLL; ++u) {
-        if (base + 4 * u >= n) break;  // warp-uniform
-        float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll
-        for (int t = 0; t < TRIPS; ++t) {
-          float4 x = QREG ? q[t] : *reinterpret_cast<const float4*>(qs + 32 * t + 4 * g);
-          trip_accum<L2>(x, v[u][t], acc);
-        }
-        float r = group_reduce(acc, 0.0f);
-        int ci = base + 4 * u + grp;
-        if (g == 0 && ci < n) cdist[ci] = metric_epilogue<METRIC>(r);
-      }
-    }
-    __syncwarp();
-  }
-};
 
 // f32 rows, dim = 32*TRIPS exactly. An 8-lane group owns a row: lane g loads the float4 at
 // element 32t + 4g of every trip (one full 128-byte line per group per load instruction) and
@@ -1234,11 +1023,10 @@ __host__ __device__ constexpr size_t warp_smem_bytes(uint32_t qfloats, uint32_t 
 // ---- the kernel ---------------------------------------------------------------------
 // One warp per CTA, one query per warp at a time; MINB = CTAs per SM the register budget
 // must allow (launch bounds).
-// SETS: FloatEvalFixed pipeline depth (LEGACY: the unpipelined FloatEvalBatch, kept as the
-// A/B baseline); MERGE_MIN > 0: use the batch form of AddWithLimit (CandList::merge) when at
-// least that many candidates survive.
+// SETS: FloatEvalFixed pipeline depth; MERGE_MIN > 0: use the batch form of AddWithLimit
+// (CandList::merge) when at least that many candidates survive.
 // XTRA: the start node has edges beyond R (a.start_extra) — compiled in only when it does.
-template <int KIND, int METRIC, int TRIPS, int SETS, bool LEGACY, int MERGE_MIN, class VT, bool FILTER, bool RETRY, int MINB,
+template <int KIND, int METRIC, int TRIPS, int SETS, int MERGE_MIN, class VT, bool FILTER, bool RETRY, int MINB,
           bool XTRA, bool PF>
 __global__ void __launch_bounds__(32, MINB) beam_search_kernel(SearchArgs a, uint32_t qfloats, uint32_t qwords) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -1296,8 +1084,7 @@ __global__ void __launch_bounds__(32, MINB) beam_search_kernel(SearchArgs a, uin
     }
     __syncwarp();
     constexpr bool FIXED = (KIND == EVAL_FLOAT_FIXED);
-    typename std::conditional<LEGACY, FloatEvalBatch<METRIC, (FIXED ? TRIPS : 1), (FIXED ? SETS : 1)>,
-                              FloatEvalFixed<METRIC, (FIXED ? TRIPS : 1), (FIXED ? SETS : 1)>>::type ev_fixed;
+    FloatEvalFixed<METRIC, (FIXED ? TRIPS : 1), (FIXED ? SETS : 1)> ev_fixed;
     FloatEvalGeneric<METRIC> ev_gen;
     constexpr bool BITS = (KIND == EVAL_BITS);
     BitEval<(BITS ? METRIC : METRIC_HAMMING), (BITS ? TRIPS : 1), (BITS ? SETS : 1)> ev_bits;
@@ -1361,12 +1148,7 @@ __global__ void __launch_bounds__(32, MINB) beam_search_kernel(SearchArgs a, uin
     // test-and-set into cid[]; returns how many
     auto visit_and_stage = [&](uint32_t i0, bool a0, uint32_t i1, bool a1) -> int {
       bool new0, new1;
-      if (a.flags & 1u) {
-        new0 = vt.test_and_set(i0, a0, lane);
-        new1 = vt.test_and_set(i1, a1, lane);
-      } else {
-        vt.test_and_set2(i0, a0, i1, a1, new0, new1, lane);
-      }
+      vt.test_and_set2(i0, a0, i1, a1, new0, new1, lane);
       uint32_t b0 = __ballot_sync(SDB_FULL, new0), b1 = __ballot_sync(SDB_FULL, new1);
       const int t0 = __popc(b0);
       if (new0) cid[__popc(b0 & lt)] = i0;

@@ -9,26 +9,22 @@ int launch_bits(sdb_index* ix, const SearchArgs& a, bool filtered, cudaStream_t 
     const bool jac = ix->bq_metric == SDB_METRIC_JACCARD;
     const uint32_t nch = (ix->bits_pitch + 15) / 16;
     if (filtered) {
-      return jac ? launch_with_retry<EVAL_BITS, METRIC_JACCARD, 4, 2, false, 0, true, 1>(ix, a, stream)
-                 : launch_with_retry<EVAL_BITS, METRIC_HAMMING, 4, 2, false, 0, true, 1>(ix, a, stream);
+      return jac ? launch_with_retry<EVAL_BITS, METRIC_JACCARD, 4, 2, 0, true, 1>(ix, a, stream)
+                 : launch_with_retry<EVAL_BITS, METRIC_HAMMING, 4, 2, 0, true, 1>(ix, a, stream);
     }
     if (jac) {
-      if (nch <= 1) return launch_with_retry<EVAL_BITS, METRIC_JACCARD, 1, 8, false, 2, false, 12>(ix, a, stream);
-      return launch_with_retry<EVAL_BITS, METRIC_JACCARD, 4, 2, false, 2, false, 12>(ix, a, stream);
+      if (nch <= 1) return launch_with_retry<EVAL_BITS, METRIC_JACCARD, 1, 8, 2, false, 12>(ix, a, stream);
+      return launch_with_retry<EVAL_BITS, METRIC_JACCARD, 4, 2, 2, false, 12>(ix, a, stream);
     }
-    if (nch <= 1 && ix->bits_pitch % 4 == 0 && !getenv("SDB_K2_LANES8")) {
+    if (nch <= 1 && ix->bits_pitch % 4 == 0) {
       // rows of whole 32-byte pieces (1024 bits: the C5b shape): four lanes per row, 256-bit loads
-      return launch_with_retry<EVAL_BITS, METRIC_HAMMING, 0, 4, false, 2, false, 16>(ix, a, stream);
+      return launch_with_retry<EVAL_BITS, METRIC_HAMMING, 0, 4, 2, false, 16>(ix, a, stream);
     }
-    if (nch <= 1) {
-      // 128-byte rows: the search is latency-bound on each warp's dependent chain, not on HBM or on
-      // L1 capacity like the f32 kernel, so more resident query-warps pay (SDB_K2_MINB=12: A/B)
-      static const bool m12 = getenv("SDB_K2_MINB") != nullptr && atoi(getenv("SDB_K2_MINB")) == 12;
-      if (m12) return launch_with_retry<EVAL_BITS, METRIC_HAMMING, 1, 8, false, 2, false, 12>(ix, a, stream);
-      return launch_with_retry<EVAL_BITS, METRIC_HAMMING, 1, 8, false, 2, false, 16>(ix, a, stream);
-    }
-    if (nch <= 2) return launch_with_retry<EVAL_BITS, METRIC_HAMMING, 2, 4, false, 2, false, 12>(ix, a, stream);
-    return launch_with_retry<EVAL_BITS, METRIC_HAMMING, 4, 2, false, 2, false, 12>(ix, a, stream);
+    // 128-byte rows: the search is latency-bound on each warp's dependent chain, not on HBM or on
+    // L1 capacity like the f32 kernel, so more resident query-warps pay (16 per SM)
+    if (nch <= 1) return launch_with_retry<EVAL_BITS, METRIC_HAMMING, 1, 8, 2, false, 16>(ix, a, stream);
+    if (nch <= 2) return launch_with_retry<EVAL_BITS, METRIC_HAMMING, 2, 4, 2, false, 12>(ix, a, stream);
+    return launch_with_retry<EVAL_BITS, METRIC_HAMMING, 4, 2, 2, false, 12>(ix, a, stream);
 }
 
 }  // namespace launch

@@ -14,12 +14,12 @@
 namespace sdb {
 namespace launch {
 
-template <int KIND, int METRIC, int TRIPS, int SETS, bool LEGACY, int MERGE_MIN, class VT, bool FILTER, bool RETRY, int MINB,
-          bool XTRA, bool PF = false>
+template <int KIND, int METRIC, int TRIPS, int SETS, int MERGE_MIN, class VT, bool FILTER, bool RETRY, int MINB, bool XTRA,
+          bool PF = false>
 int launch_variant_x(sdb_index* ix, const SearchArgs& a, cudaStream_t stream) {
-  auto kern = beam_search_kernel<KIND, METRIC, TRIPS, SETS, LEGACY, MERGE_MIN, VT, FILTER, RETRY, MINB, XTRA, PF>;
-  // FloatEvalGrouped keeps short queries (<= 4 float4 per lane) in registers: no shared copy
-  constexpr bool QREG = (KIND == EVAL_FLOAT_FIXED) && !LEGACY && TRIPS <= 4;
+  auto kern = beam_search_kernel<KIND, METRIC, TRIPS, SETS, MERGE_MIN, VT, FILTER, RETRY, MINB, XTRA, PF>;
+  // FloatEvalFixed keeps short queries (<= 4 float4 per lane) in registers: no shared copy
+  constexpr bool QREG = (KIND == EVAL_FLOAT_FIXED) && TRIPS <= 4;
   const uint32_t qfloats = (KIND == EVAL_ADC || KIND == EVAL_ADC_SMEM || KIND == EVAL_BITS || KIND == EVAL_GEO || QREG) ? 0 : (a.dim + 3) / 4 * 4;
   const uint32_t qwords = (KIND == EVAL_BITS) ? a.bits_pitch : 0;
   const uint32_t table_floats = (KIND == EVAL_ADC_SMEM) ? a.pqM * a.pqK : 0;
@@ -27,22 +27,18 @@ int launch_variant_x(sdb_index* ix, const SearchArgs& a, cudaStream_t stream) {
   static thread_local int cached_dev = -1;
   static thread_local size_t cached_smem = 0;
   static thread_local int ctas_per_sm = 0;
-  // geo kernel: CTAs/SM below the launch bound for A/B runs (sdb_index::geo_ctas_per_sm, 0 = MINB)
-  const int cap = (KIND == EVAL_GEO && MINB > 1 && ix->geo_ctas_per_sm > 0) ? std::min(ix->geo_ctas_per_sm, MINB) : MINB;
-  static thread_local int cached_cap = 0;
-  if (cached_dev != ix->device || cached_smem != smem || cached_cap != cap) {
+  if (cached_dev != ix->device || cached_smem != smem) {
     if (smem > ix->smem_optin) return fail(SDB_ERR_INTERNAL, "beam search kernel does not fit in shared memory");
     SDB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
     int nb = 0;
     SDB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kern, 32, smem));
     if (nb <= 0) return fail(SDB_ERR_INTERNAL, "beam search kernel cannot be resident");
-    if (MINB > 1 && nb > cap) nb = cap;
+    if (MINB > 1 && nb > MINB) nb = MINB;
     ctas_per_sm = nb;
     // The unified L1/shared array is also where in-flight global loads land: ask for no more
     // shared memory than the resident CTAs need so the rest stays L1 (more rows in flight).
     const size_t need_smem = size_t(nb) * (smem + 1024);
     int pct = int((need_smem * 100 + ix->smem_per_sm - 1) / ix->smem_per_sm);
-    if (const char* e = getenv("SDB_K1_CARVEOUT")) pct = atoi(e);
     if (pct > 100) pct = 100;
     SDB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, pct));
     if (getenv("SDB_DEBUG_OCC"))
@@ -50,17 +46,11 @@ int launch_variant_x(sdb_index* ix, const SearchArgs& a, cudaStream_t stream) {
               need_smem >> 10);
     cached_smem = smem;
     cached_dev = ix->device;
-    cached_cap = cap;
   }
   uint32_t resident = uint32_t(ix->sm_count) * ctas_per_sm;
   uint32_t need = RETRY ? std::min<uint32_t>(uint32_t(ix->sm_count), ix->retry_slots) : a.n_work;
   uint32_t grid = need < resident ? need : resident;
   if (grid == 0) grid = 1;
-  if (!RETRY && (a.flags & 2u) && a.n_work > grid) {
-    // equal number of queries per resident warp: no half-empty last wave
-    const uint32_t waves = (a.n_work + grid - 1) / grid;
-    grid = (a.n_work + waves - 1) / waves;
-  }
   kern<<<grid, 32, smem, stream>>>(a, qfloats, qwords);
   ix->launches++;
   SDB_CUDA(cudaGetLastError());
@@ -69,26 +59,21 @@ int launch_variant_x(sdb_index* ix, const SearchArgs& a, cudaStream_t stream) {
 
 // the start node's overflow edges (after deletes; normally none) get their own instantiation so
 // the common case pays nothing for them (the extra loop cost 5 % on C2)
-template <int KIND, int METRIC, int TRIPS, int SETS, bool LEGACY, int MERGE_MIN, class VT, bool FILTER, bool RETRY, int MINB>
+template <int KIND, int METRIC, int TRIPS, int SETS, int MERGE_MIN, class VT, bool FILTER, bool RETRY, int MINB>
 int launch_variant(sdb_index* ix, const SearchArgs& a, cudaStream_t stream) {
   if (a.n_start_extra != 0)
-    return launch_variant_x<KIND, METRIC, TRIPS, SETS, LEGACY, MERGE_MIN, VT, FILTER, RETRY, MINB, true>(ix, a, stream);
-  // speculative row prefetch (small-row evaluators, unfiltered first pass); SDB_NO_PF=1 = A/B switch
+    return launch_variant_x<KIND, METRIC, TRIPS, SETS, MERGE_MIN, VT, FILTER, RETRY, MINB, true>(ix, a, stream);
+  // speculative row prefetch (small-row evaluators, unfiltered first pass)
   // (PQ kernels: +1.6 %; bit rows: -1.6 %, the probes cost more than the L2 hits save — off there)
-  constexpr bool CAN_PF = !FILTER && !RETRY && (KIND == EVAL_ADC_SMEM || KIND == EVAL_ADC || KIND == EVAL_ADC_FLY);
-  if (CAN_PF) {
-    static const bool no_pf = getenv("SDB_NO_PF") != nullptr;
-    if (!no_pf)
-      return launch_variant_x<KIND, METRIC, TRIPS, SETS, LEGACY, MERGE_MIN, VT, FILTER, RETRY, MINB, false, CAN_PF>(ix, a, stream);
-  }
-  return launch_variant_x<KIND, METRIC, TRIPS, SETS, LEGACY, MERGE_MIN, VT, FILTER, RETRY, MINB, false>(ix, a, stream);
+  constexpr bool PF = !FILTER && !RETRY && (KIND == EVAL_ADC_SMEM || KIND == EVAL_ADC || KIND == EVAL_ADC_FLY);
+  return launch_variant_x<KIND, METRIC, TRIPS, SETS, MERGE_MIN, VT, FILTER, RETRY, MINB, false, PF>(ix, a, stream);
 }
 
-template <int KIND, int METRIC, int TRIPS, int SETS, bool LEGACY, int MERGE_MIN, bool FILTER, int MINB, class VT = VisitedCompactN>
+template <int KIND, int METRIC, int TRIPS, int SETS, int MERGE_MIN, bool FILTER, int MINB>
 int launch_with_retry(sdb_index* ix, SearchArgs a, cudaStream_t stream) {
   const bool prof = ix->prof_on && ix->prof_n < sdb_index::PROF_RING;
   if (prof) SDB_CUDA(cudaEventRecord(ix->prof_ev[2 * ix->prof_n], stream));
-  int rc = launch_variant<KIND, METRIC, TRIPS, SETS, LEGACY, MERGE_MIN, VT, FILTER, false, MINB>(ix, a, stream);
+  int rc = launch_variant<KIND, METRIC, TRIPS, SETS, MERGE_MIN, VisitedCompactN, FILTER, false, MINB>(ix, a, stream);
   if (rc) return rc;
   if (prof) {
     SDB_CUDA(cudaEventRecord(ix->prof_ev[2 * ix->prof_n + 1], stream));
@@ -109,11 +94,12 @@ int launch_with_retry(sdb_index* ix, SearchArgs a, cudaStream_t stream) {
     cudaMemcpy(h, a.work_counter - 2, sizeof(h), cudaMemcpyDeviceToHost);
     fprintf(stderr, "[sdb] beam search: %u of %u queries overflowed the compact visited table -> retry launch\n", h[1], a.B);
   }
-  return launch_variant<RK, METRIC, RT, RS, false, 0, VisitedBitmap, FILTER, true, 1>(ix, a, stream);
+  return launch_variant<RK, METRIC, RT, RS, 0, VisitedBitmap, FILTER, true, 1>(ix, a, stream);
 }
 
 // PQ search without per-query tables: sub-vectors of 4, 8 or 16 floats whose number is a multiple
-// of 4 (C4: 96 x 8). SDB_ADC_TABLE=1 keeps the table kernels (A/B; they also serve other shapes).
+// of 4 (C4: 96 x 8). SDB_ADC_TABLE=1 keeps the table kernels (they also serve other shapes), so the
+// tests can compare the two.
 inline bool adc_on_the_fly(const sdb_index* ix) {
   const bool table = getenv("SDB_ADC_TABLE") != nullptr || getenv("SDB_ADC_GLOBAL") != nullptr;
   return !table && (ix->pqSub == 4 || ix->pqSub == 8 || ix->pqSub == 16) && ix->pqM % 4 == 0 && ix->store_metric != SDB_METRIC_COSINE;
@@ -125,41 +111,26 @@ template <int SUB>
 int launch_pq_fly(sdb_index* ix, const SearchArgs& a, bool filtered, cudaStream_t stream) {
   const bool l2 = ix->store_metric == SDB_METRIC_EUCLIDEAN;
   if (filtered)
-    return l2 ? launch_with_retry<EVAL_ADC_FLY, METRIC_EUCLIDEAN, SUB, 1, false, 0, true, 1>(ix, a, stream)
-              : launch_with_retry<EVAL_ADC_FLY, METRIC_DOT, SUB, 1, false, 0, true, 1>(ix, a, stream);
-  return l2 ? launch_with_retry<EVAL_ADC_FLY, METRIC_EUCLIDEAN, SUB, 1, false, 2, false, 12>(ix, a, stream)
-            : launch_with_retry<EVAL_ADC_FLY, METRIC_DOT, SUB, 1, false, 2, false, 12>(ix, a, stream);
-}
-
-// Tuning knob for A/B runs on the GPU (not part of the ABI): SDB_K1_VARIANT picks the
-// evaluator layout / list-update form of the dim-128 kernel.
-inline int k1_variant() {
-  const char* e = getenv("SDB_K1_VARIANT");
-  return e ? atoi(e) : -1;
+    return l2 ? launch_with_retry<EVAL_ADC_FLY, METRIC_EUCLIDEAN, SUB, 1, 0, true, 1>(ix, a, stream)
+              : launch_with_retry<EVAL_ADC_FLY, METRIC_DOT, SUB, 1, 0, true, 1>(ix, a, stream);
+  return l2 ? launch_with_retry<EVAL_ADC_FLY, METRIC_EUCLIDEAN, SUB, 1, 2, false, 12>(ix, a, stream)
+            : launch_with_retry<EVAL_ADC_FLY, METRIC_DOT, SUB, 1, 2, false, 12>(ix, a, stream);
 }
 
 template <int METRIC>
 int launch_float(sdb_index* ix, const SearchArgs& a, bool filtered, cudaStream_t stream) {
-  if (filtered) return launch_with_retry<EVAL_FLOAT_GENERIC, METRIC, 1, 1, false, 0, true, 1>(ix, a, stream);
+  if (filtered) return launch_with_retry<EVAL_FLOAT_GENERIC, METRIC, 1, 1, 0, true, 1>(ix, a, stream);
   if (a.dim % 32 == 0) {
     switch (a.dim / 32) {
-      case 4:
-        switch (k1_variant()) {
-          // round-1 baseline (unpipelined evaluator, sequential list update, 8192-slot table)
-          case 0: return launch_with_retry<EVAL_FLOAT_FIXED, METRIC, 4, 8, true, 0, false, 12, VisitedCompact>(ix, a, stream);
-          case 1: return launch_with_retry<EVAL_FLOAT_FIXED, METRIC, 4, 6, false, 0, false, 12>(ix, a, stream);
-          case 2: return launch_with_retry<EVAL_FLOAT_FIXED, METRIC, 4, 5, false, 2, false, 12, VisitedCompactN>(ix, a, stream);
-          default: return launch_with_retry<EVAL_FLOAT_FIXED, METRIC, 4, 6, false, 2, false, 12>(ix, a, stream);
-        }
-      case 8: return launch_with_retry<EVAL_FLOAT_FIXED, METRIC, 8, 3, false, 2, false, 12>(ix, a, stream);
-      case 12: return launch_with_retry<EVAL_FLOAT_FIXED, METRIC, 12, 2, false, 2, false, 12>(ix, a, stream);
-      case 24: return launch_with_retry<EVAL_FLOAT_FIXED, METRIC, 24, 1, false, 2, false, 12>(ix, a, stream);
+      case 4: return launch_with_retry<EVAL_FLOAT_FIXED, METRIC, 4, 6, 2, false, 12>(ix, a, stream);
+      case 8: return launch_with_retry<EVAL_FLOAT_FIXED, METRIC, 8, 3, 2, false, 12>(ix, a, stream);
+      case 12: return launch_with_retry<EVAL_FLOAT_FIXED, METRIC, 12, 2, 2, false, 12>(ix, a, stream);
+      case 24: return launch_with_retry<EVAL_FLOAT_FIXED, METRIC, 24, 1, 2, false, 12>(ix, a, stream);
       default: break;
     }
   }
-  return launch_with_retry<EVAL_FLOAT_GENERIC, METRIC, 1, 1, false, 2, false, 12>(ix, a, stream);
+  return launch_with_retry<EVAL_FLOAT_GENERIC, METRIC, 1, 1, 2, false, 12>(ix, a, stream);
 }
-
 
 }  // namespace launch
 }  // namespace sdb

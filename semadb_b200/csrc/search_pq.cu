@@ -28,13 +28,13 @@ int launch_pq(sdb_index* ix, const SearchArgs& a, bool filtered, cudaStream_t st
       SearchArgs t = a;
       if (t.vt_slots > room) t.vt_slots = uint32_t(room) / 8 * 8;
       const uint32_t nch = (ix->pqM + 15) / 16;
-      if (nch <= 2) return launch_with_retry<EVAL_ADC_SMEM, 0, 2, 1, false, 2, false, 12>(ix, t, stream);
-      if (nch <= 4) return launch_with_retry<EVAL_ADC_SMEM, 0, 4, 1, false, 2, false, 12>(ix, t, stream);
-      if (nch <= 6) return launch_with_retry<EVAL_ADC_SMEM, 0, 6, 1, false, 2, false, 12>(ix, t, stream);
-      return launch_with_retry<EVAL_ADC_SMEM, 0, 8, 1, false, 2, false, 12>(ix, t, stream);
+      if (nch <= 2) return launch_with_retry<EVAL_ADC_SMEM, 0, 2, 1, 2, false, 12>(ix, t, stream);
+      if (nch <= 4) return launch_with_retry<EVAL_ADC_SMEM, 0, 4, 1, 2, false, 12>(ix, t, stream);
+      if (nch <= 6) return launch_with_retry<EVAL_ADC_SMEM, 0, 6, 1, 2, false, 12>(ix, t, stream);
+      return launch_with_retry<EVAL_ADC_SMEM, 0, 8, 1, 2, false, 12>(ix, t, stream);
     }
-    return filtered ? launch_with_retry<EVAL_ADC, 0, 1, 1, false, 0, true, 1>(ix, a, stream)
-                    : launch_with_retry<EVAL_ADC, 0, 1, 1, false, 2, false, 12>(ix, a, stream);
+    return filtered ? launch_with_retry<EVAL_ADC, 0, 1, 1, 0, true, 1>(ix, a, stream)
+                    : launch_with_retry<EVAL_ADC, 0, 1, 1, 2, false, 12>(ix, a, stream);
   }
 }
 

@@ -101,31 +101,12 @@ def test_tcgen05_candidate_pass_matches_mma_sync_pass(metric, dim):
     assert (d[0] == b[0]).all() and d[1].tobytes() == b[1].tobytes()
 
 
-def test_two_sm_variant_matches(monkeypatch):
-    """SDB_FLAT_2CTA=1 selects the cta_group::2 form of the pass (clusters of two CTAs, each loading
-    half of every point tile, the leader issuing M256 MMAs for both SMs): same candidates, same
-    results. Kept opt-in: it halves the L2->SM bytes but the pass is MMA-bound, so it is not faster."""
-    n, dim = 70_000, 128
-    X, Q = synth.sift_shaped(n, dim, 3), synth.sift_shaped(600, dim, 4, w_seed=3)
-    g = IndexFlat(IndexVectorFlatParameters(dim, "euclidean"))
-    g.set_vectors(np.arange(2, n + 2, dtype=np.uint64), X)
-    monkeypatch.delenv("SDB_FLAT_2CTA", raising=False)
-    a = g.flat_search_batch(Q, 10)
-    pa, ca, oa = g.flat_last_stats()
-    monkeypatch.setenv("SDB_FLAT_2CTA", "1")
-    b = g.flat_search_batch(Q, 10)
-    pb, cb, ob = g.flat_last_stats()
-    assert pa == 2 and pb == 2 and oa == 0 and ob == 0
-    assert abs(ca - cb) <= 0.01 * ca + 5
-    assert (a[0] == b[0]).all() and a[1].tobytes() == b[1].tobytes()
-
-
-@pytest.mark.parametrize("variant", ["levels", "no_center", "sample_all", "sample_small"])
+@pytest.mark.parametrize("variant", ["levels", "sample_all", "sample_small"])
 def test_flat_tc_variants_equal_exact_scan(variant, monkeypatch):
     """Every form of the candidate generation returns the exact scan's lists: the level scheme
-    (SDB_FLAT_LEVELS=1), the two-pass form without centring, with the whole store as the sample and
-    with a sample so small that the bound is loose."""
-    env = {"levels": ("SDB_FLAT_LEVELS", "1"), "no_center": ("SDB_FLAT_NO_CENTER", "1"), "sample_all": ("SDB_FLAT_SAMPLE_DIV", "1"),
+    (SDB_FLAT_LEVELS=1), the two-pass form with the whole store as the sample and with a sample so
+    small that the bound is loose."""
+    env = {"levels": ("SDB_FLAT_LEVELS", "1"), "sample_all": ("SDB_FLAT_SAMPLE_DIV", "1"),
            "sample_small": ("SDB_FLAT_SAMPLE_DIV", "64")}[variant]
     n, dim = 70_000, 128
     X, Q = synth.sift_shaped(n, dim, 3), synth.sift_shaped(400, dim, 4, w_seed=3)
