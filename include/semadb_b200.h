@@ -165,11 +165,35 @@ int sdb_search_visited(sdb_index* ix, uint32_t B, const float* queries, uint32_t
  * ascending id order (the reference's Go-map order is unspecified; ties: lower id wins). */
 int sdb_flat_search_batch(sdb_index* ix, uint32_t B, const float* queries, uint32_t k, const uint64_t* filter_ids,
                           uint64_t n_filter, uint64_t* out_ids, float* out_dists, uint32_t* out_counts);
+/* Flat search with one filter per request (shard/index/search.go:59-85 -> flat.go:94-96). The
+ * filters follow sdb_search_batch_filters: filter f is filter_ids[filter_offsets[f] ..
+ * filter_offsets[f+1]), strictly ascending; request b uses filter query_filter[b], or none if
+ * query_filter[b] < 0 (query_filter == NULL: every request uses filter 0); an EMPTY list is a
+ * filter and its request returns no result; n_filters == 0 = nobody is filtered. Flat rules:
+ *   - an id that is not stored (deleted or never inserted), is >= the allocated rows, or is < 2
+ *     is simply never matched — not an error (flat search has no GetMany of seeds);
+ *   - unsorted or duplicate ids, or a query_filter index >= n_filters, return SDB_ERR_INVALID;
+ *   - k must be 1..75.
+ * Row b of the output equals, bit for bit, sdb_flat_search_batch run on query b alone with b's
+ * filter (or with none). Each filter takes one of two routes, chosen from its size and its number
+ * of requests: its rows gathered by id and scored for each of its requests, or the range scan
+ * over the store with its bitmap (sdb_flat_last_filter_stats reports the split). Unfiltered
+ * requests of a mixed batch go through the unfiltered pass. sdb_flat_search_batch(filter_ids,
+ * n_filter) is the one-filter case: it sorts and de-duplicates the ids, so any order is accepted. */
+int sdb_flat_search_batch_filters(sdb_index* ix, uint32_t B, const float* queries, uint32_t k, uint32_t n_filters,
+                                  const uint64_t* filter_ids, const uint64_t* filter_offsets, const int32_t* query_filter,
+                                  uint64_t* out_ids, float* out_dists, uint32_t* out_counts);
+/* Diagnostics of the most recent flat search on this handle: filters (with at least one request)
+ * that took the gather route and the range-scan route, and the (request, id) pairs the gather
+ * route scored (ids of deleted points included). All 0 after an unfiltered call. */
+int sdb_flat_last_filter_stats(sdb_index* ix, uint32_t* gathered_filters, uint32_t* scanned_filters,
+                               uint64_t* gathered_pairs);
 
 /* Diagnostics of the most recent sdb_flat_search_batch on this handle: path = 0 exact CUDA-core
  * scan, 1 tensor-core candidate pass (mma.sync), 2 tensor-core candidate pass (tcgen05 + TMA);
  * candidates = (query, point) pairs the last candidate level kept for exact re-scoring, summed
- * over the batch; overflowed = queries that fell back to the exact scan. */
+ * over the batch; overflowed = queries that fell back to the exact scan. With filters, these
+ * describe the pass that served the unfiltered requests (all 0 when there were none). */
 int sdb_flat_last_stats(sdb_index* ix, int32_t* path, uint64_t* candidates, uint32_t* overflowed);
 
 /* ---- insert: replaces IndexVamana.InsertUpdateDelete's insert branch (vamana.go:136-201,

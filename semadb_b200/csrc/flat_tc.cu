@@ -42,6 +42,7 @@
 
 #include "common.cuh"
 #include "index.cuh"
+#include "warp_topk.cuh"
 
 namespace sdb {
 
@@ -845,10 +846,8 @@ __global__ void seed_cand_kernel(const uint64_t* prev_ids, const uint32_t* prev_
 // Exact re-score, one WARP per query (four queries per CTA, no block-wide barrier): the candidates'
 // rows are gathered 16 at a time (an 8-lane group per row, all 16 row loads of a lane in flight),
 // scored with the reference's summation order, and offered to a k-slot list sorted by (distance asc,
-// id asc) that lives in REGISTERS (slot p = lane + 32 j, NS slots per lane: 1 for k <= 32, 3 up to
-// k = 96): an insertion is three ballots' worth of compares and two shuffles per slot row, no
-// shared-memory round trip. A candidate that does not beat the current k-th (kept in a uniform
-// register pair) is dropped by the lane that holds it, so the warp-wide insertion runs
+// id asc) that lives in REGISTERS (WarpTopK, warp_topk.cuh). A candidate that does not beat the
+// current k-th is dropped by the lane that holds it, so the warp-wide insertion runs
 // ~k ln(n/k) times per query. implicit_n > 0: the candidates are the implicit_n points first_id,
 // first_id+1, ... (level 0 of the level scheme: no list in memory). cand_total: optional running
 // sum of the list lengths (the sdb_flat_last_stats diagnostic).
@@ -881,58 +880,7 @@ __global__ void __launch_bounds__(32 * RW_WARPS) rescore_warp_kernel(
   __syncwarp();
   constexpr bool L2 = (METRIC == METRIC_EUCLIDEAN);
   const int trips = dim >> 5;
-  float kd[NS];
-  uint32_t ki[NS];
-#pragma unroll
-  for (int j = 0; j < NS; ++j) { kd[j] = 0.0f; ki[j] = 0u; }
-  uint32_t len = 0;
-  float wd = 0.0f;   // the k-th entry once the list is full (uniform)
-  uint32_t wi = 0u;
-  const int wj = int(k - 1) >> 5, wl = int(k - 1) & 31;
-  // offer (d, id), held by every lane, to the sorted list; warp-synchronous
-  auto insert = [&](float d, uint32_t id) {
-    uint32_t pos = 0;
-#pragma unroll
-    for (int j = 0; j < NS; ++j) {
-      const uint32_t p = lane + 32 * j;
-      const bool before = p < len && (kd[j] < d || (kd[j] == d && ki[j] < id));
-      pos += __popc(__ballot_sync(SDB_FULL, before));
-    }
-    if (pos >= k) return;
-#pragma unroll
-    for (int j = NS - 1; j >= 0; --j) {  // slots >= pos move up by one; the rows below are still unmodified
-      float pd = __shfl_up_sync(SDB_FULL, kd[j], 1);
-      uint32_t pi = __shfl_up_sync(SDB_FULL, ki[j], 1);
-      if (j > 0) {
-        const float cd = __shfl_sync(SDB_FULL, kd[j > 0 ? j - 1 : 0], 31);
-        const uint32_t ci = __shfl_sync(SDB_FULL, ki[j > 0 ? j - 1 : 0], 31);
-        if (lane == 0) { pd = cd; pi = ci; }
-      }
-      const uint32_t p = lane + 32 * j;
-      if (p > pos) { kd[j] = pd; ki[j] = pi; }
-      else if (p == pos) { kd[j] = d; ki[j] = id; }
-    }
-    if (len < k) ++len;
-    if (len == k) {
-      float sd = kd[0];
-      uint32_t si = ki[0];
-#pragma unroll
-      for (int j = 1; j < NS; ++j)
-        if (j == wj) { sd = kd[j]; si = ki[j]; }
-      wd = __shfl_sync(SDB_FULL, sd, wl);
-      wi = __shfl_sync(SDB_FULL, si, wl);
-    }
-  };
-  // the lanes that hold a fresh (d, id) (lane 0 of each group) offer it if it can enter the list
-  auto offer = [&](float d, uint32_t id, bool have) {
-    const bool want = have && (len < k || d < wd || (d == wd && id < wi));
-    uint32_t m = __ballot_sync(SDB_FULL, want);
-    while (m) {
-      const int src = __ffs(m) - 1;
-      m &= m - 1;
-      insert(__shfl_sync(SDB_FULL, d, src), __shfl_sync(SDB_FULL, id, src));
-    }
-  };
+  SDB_WARP_TOPK_STATE(top, NS, k, lane);
   auto cand_id = [&](uint32_t c) -> uint32_t { return implicit_n ? first_id + c : cand[size_t(q) * CAND_CAP + c]; };
   uint32_t c0 = 0;
   if (trips <= 4) {
@@ -960,7 +908,7 @@ __global__ void __launch_bounds__(32 * RW_WARPS) rescore_warp_kernel(
           for (uint32_t i = trips << 5; i < dim; ++i) tail = tail_accum<L2>(s_q[i], __ldg(row + i), tail);
         const float r = metric_epilogue<METRIC>(group_reduce(acc, tail));
         const bool have = g == 0 && c < n && (!implicit_n || exists[pid[u]]);
-        offer(r, pid[u], have);
+        top.offer(r, pid[u], have);
       }
     }
   }
@@ -979,18 +927,20 @@ __global__ void __launch_bounds__(32 * RW_WARPS) rescore_warp_kernel(
     if (g == 0)
       for (uint32_t i = trips << 5; i < dim; ++i) tail = tail_accum<L2>(s_q[i], __ldg(row + i), tail);
     const float r = metric_epilogue<METRIC>(group_reduce(acc, tail));
-    offer(r, pid, g == 0 && act && (!implicit_n || exists[pid]));
+    top.offer(r, pid, g == 0 && act && (!implicit_n || exists[pid]));
   }
 #pragma unroll
   for (int j = 0; j < NS; ++j) {
     const uint32_t r = lane + 32 * j;
     if (r < k) {
-      out_ids[size_t(q) * k + r] = r < len ? uint64_t(ki[j]) : 0;
-      out_d[size_t(q) * k + r] = r < len ? kd[j] : __int_as_float(0x7f800000);
+      out_ids[size_t(q) * k + r] = r < top.len ? uint64_t(top.ki[j]) : 0;
+      out_d[size_t(q) * k + r] = r < top.len ? top.kd[j] : __int_as_float(0x7f800000);
     }
   }
-  if (lane == 0) out_cnt[q] = len;
+  if (lane == 0) out_cnt[q] = top.len;
 }
+
+}  // namespace
 
 __global__ void gather_queries_kernel(const uint32_t* list, uint32_t n, const float* src, uint32_t dim, float* dst) {
   const uint32_t i = blockIdx.x;
@@ -1008,8 +958,6 @@ __global__ void scatter_results_kernel(const uint32_t* list, uint32_t n, uint32_
   }
   if (threadIdx.x == 0) out_cnt[q] = cnt[i];
 }
-
-}  // namespace
 
 // growth of the levels: intermediate levels multiply the covered prefix by LEVEL_MID, the last level
 // may cover up to LEVEL_LAST times the prefix before it (a level's re-score handles ~k * ratio

@@ -509,9 +509,11 @@ static int ensure_out_scratch(sdb_index* ix, uint32_t B, uint32_t k) {
 // filter f = filter_ids[filter_offsets[f] .. filter_offsets[f+1]); query_filter[b] < 0 = request b
 // is not filtered (nullptr: every request uses filter 0). An EMPTY list is still a filter: the
 // reference then seeds nothing and returns no result (search.go:33-51 with an empty bitmap).
+// Ids below min_id are dropped like ids beyond the store (flat search: 2, the scan's first id);
+// h_off, if given, receives the staged offsets.
 static int stage_filters(sdb_index* ix, uint32_t B, uint32_t n_filters, const uint64_t* filter_ids,
                          const uint64_t* filter_offsets, const int32_t* query_filter, uint32_t L, bool want_bits,
-                         SearchFilters* out) {
+                         SearchFilters* out, uint64_t min_id = 0, std::vector<uint32_t>* h_off = nullptr) {
   if (n_filters == 0 || !filter_offsets) return fail(SDB_ERR_INVALID, "filters: need at least one filter and its offsets");
   std::vector<uint32_t> ids, off(size_t(n_filters) + 1, 0), qf_plain, qf_filtered;
   std::vector<int32_t> qfil;
@@ -530,7 +532,7 @@ static int stage_filters(sdb_index* ix, uint32_t B, uint32_t n_filters, const ui
       prev = id;
       if (i - b0 < L && (id == 0 || id >= ix->rows || !ix->h_exists[id]))
         return fail(SDB_ERR_NOTFOUND, "failed to get filter points");  // GetMany of the seeds, search.go:45-48
-      if (id < ix->rows) ids.push_back(uint32_t(id));  // ids beyond the store can never be expanded
+      if (id < ix->rows && id >= min_id) ids.push_back(uint32_t(id));  // ids beyond the store can never be expanded
     }
   }
   off[n_filters] = uint32_t(ids.size());
@@ -575,6 +577,7 @@ static int stage_filters(sdb_index* ix, uint32_t B, uint32_t n_filters, const ui
     out->n_plain = uint32_t(qf_plain.size());
   }
   SDB_CUDA(cudaStreamSynchronize(ix->stream));  // host vectors go out of scope
+  if (h_off) *h_off = std::move(off);
   return SDB_OK;
 }
 
@@ -740,6 +743,41 @@ int sdb_search_visited(sdb_index* ix, uint32_t B, const float* queries, uint32_t
   return SDB_OK;
 }
 
+// Flat search of a batch (sdb_flat_search_batch, sdb_flat_search_batch_filters): n_filters == 0 =
+// nobody is filtered, otherwise the filters of sdb_search_batch_filters, routed by launch_flat_filtered.
+static int flat_batch_locked(sdb_index* ix, uint32_t B, const float* queries, uint32_t k, uint32_t n_filters,
+                             const uint64_t* filter_ids, const uint64_t* filter_offsets, const int32_t* query_filter,
+                             uint64_t* out_ids, float* out_dists, uint32_t* out_counts) {
+  int rc;
+  SearchFilters sf;
+  std::vector<uint32_t> h_off;
+  // flat search has no GetMany of seeds (L = 0): ids that are not stored are simply never matched
+  if (n_filters && (rc = stage_filters(ix, B, n_filters, filter_ids, filter_offsets, query_filter, 0, false, &sf, 2, &h_off)))
+    return rc;
+  if ((rc = ix->d_q.ensure(size_t(B) * ix->p.dim))) return rc;
+  if ((rc = ensure_out_scratch(ix, B, k))) return rc;
+  SDB_CUDA(cudaMemcpyAsync(ix->d_q.p, queries, size_t(B) * ix->p.dim * sizeof(float), cudaMemcpyHostToDevice, ix->stream));
+  if (n_filters) {
+    rc = launch_flat_filtered(ix, B, ix->d_q.p, k, n_filters, h_off.data(), query_filter, sf.ids, ix->d_oid.p, ix->d_od.p,
+                              ix->d_oc.p, ix->stream);
+    if (rc) return rc;
+  } else {
+    ix->flat_last_gathered = ix->flat_last_scanned = 0;
+    ix->flat_last_pairs = 0;
+    ix->flat_host_out.ids = out_ids; ix->flat_host_out.dists = out_dists; ix->flat_host_out.counts = out_counts;
+    ix->flat_host_out.armed = true; ix->flat_host_out.done = false;
+    rc = launch_flat(ix, B, ix->d_q.p, k, nullptr, ix->d_oid.p, ix->d_od.p, ix->d_oc.p, ix->stream);
+    ix->flat_host_out.armed = false;
+    if (rc) return rc;
+    if (ix->flat_host_out.done) return SDB_OK;  // copied and synchronised by the tensor-core path
+  }
+  SDB_CUDA(cudaMemcpyAsync(out_ids, ix->d_oid.p, size_t(B) * k * sizeof(uint64_t), cudaMemcpyDeviceToHost, ix->stream));
+  SDB_CUDA(cudaMemcpyAsync(out_dists, ix->d_od.p, size_t(B) * k * sizeof(float), cudaMemcpyDeviceToHost, ix->stream));
+  SDB_CUDA(cudaMemcpyAsync(out_counts, ix->d_oc.p, size_t(B) * sizeof(uint32_t), cudaMemcpyDeviceToHost, ix->stream));
+  SDB_CUDA(cudaStreamSynchronize(ix->stream));
+  return SDB_OK;
+}
+
 int sdb_flat_search_batch(sdb_index* ix, uint32_t B, const float* queries, uint32_t k, const uint64_t* filter_ids,
                           uint64_t n_filter, uint64_t* out_ids, float* out_dists, uint32_t* out_counts) {
   if (!ix) return fail(SDB_ERR_INVALID, "null index");
@@ -748,28 +786,34 @@ int sdb_flat_search_batch(sdb_index* ix, uint32_t B, const float* queries, uint3
   if (k < 1 || k > 75) return fail(SDB_ERR_INVALID, "invalid limit for vector query, expected 1-75");  // models/search.go:329
   std::lock_guard<std::mutex> g(ix->mu);
   SDB_CUDA(cudaSetDevice(ix->device));
-  int rc;
-  const bool filtered = filter_ids != nullptr;
-  if (filtered) {
-    std::vector<uint32_t> bits((size_t(ix->rows) + 31) / 32, 0);
-    for (uint64_t i = 0; i < n_filter; ++i)
-      if (filter_ids[i] < ix->rows) bits[filter_ids[i] >> 5] |= 1u << (filter_ids[i] & 31);
-    if ((rc = ix->d_filter_bits.ensure(bits.size() + 1))) return rc;
-    SDB_CUDA(cudaMemcpy(ix->d_filter_bits.p, bits.data(), bits.size() * 4, cudaMemcpyHostToDevice));
-  }
-  if ((rc = ix->d_q.ensure(size_t(B) * ix->p.dim))) return rc;
-  if ((rc = ensure_out_scratch(ix, B, k))) return rc;
-  SDB_CUDA(cudaMemcpyAsync(ix->d_q.p, queries, size_t(B) * ix->p.dim * sizeof(float), cudaMemcpyHostToDevice, ix->stream));
-  ix->flat_host_out.ids = out_ids; ix->flat_host_out.dists = out_dists; ix->flat_host_out.counts = out_counts;
-  ix->flat_host_out.armed = true; ix->flat_host_out.done = false;
-  rc = launch_flat(ix, B, ix->d_q.p, k, filtered ? ix->d_filter_bits.p : nullptr, ix->d_oid.p, ix->d_od.p, ix->d_oc.p, ix->stream);
-  ix->flat_host_out.armed = false;
-  if (rc) return rc;
-  if (ix->flat_host_out.done) return SDB_OK;  // copied and synchronised by the tensor-core path
-  SDB_CUDA(cudaMemcpyAsync(out_ids, ix->d_oid.p, size_t(B) * k * sizeof(uint64_t), cudaMemcpyDeviceToHost, ix->stream));
-  SDB_CUDA(cudaMemcpyAsync(out_dists, ix->d_od.p, size_t(B) * k * sizeof(float), cudaMemcpyDeviceToHost, ix->stream));
-  SDB_CUDA(cudaMemcpyAsync(out_counts, ix->d_oc.p, size_t(B) * sizeof(uint32_t), cudaMemcpyDeviceToHost, ix->stream));
-  SDB_CUDA(cudaStreamSynchronize(ix->stream));
+  if (!filter_ids) return flat_batch_locked(ix, B, queries, k, 0, nullptr, nullptr, nullptr, out_ids, out_dists, out_counts);
+  // this entry takes the ids in any order, duplicates included: the one-filter case of the per-request form
+  std::vector<uint64_t> ids(filter_ids, filter_ids + n_filter);
+  std::sort(ids.begin(), ids.end());
+  ids.erase(std::unique(ids.begin(), ids.end()), ids.end());
+  const uint64_t offs[2] = {0, ids.size()};
+  return flat_batch_locked(ix, B, queries, k, 1, ids.data(), offs, nullptr, out_ids, out_dists, out_counts);
+}
+
+int sdb_flat_search_batch_filters(sdb_index* ix, uint32_t B, const float* queries, uint32_t k, uint32_t n_filters,
+                                  const uint64_t* filter_ids, const uint64_t* filter_offsets, const int32_t* query_filter,
+                                  uint64_t* out_ids, float* out_dists, uint32_t* out_counts) {
+  if (!ix) return fail(SDB_ERR_INVALID, "null index");
+  if (B == 0) return SDB_OK;
+  if (!queries || !out_ids || !out_dists || !out_counts) return fail(SDB_ERR_INVALID, "null argument");
+  if (k < 1 || k > 75) return fail(SDB_ERR_INVALID, "invalid limit for vector query, expected 1-75");  // models/search.go:329
+  std::lock_guard<std::mutex> g(ix->mu);
+  SDB_CUDA(cudaSetDevice(ix->device));
+  return flat_batch_locked(ix, B, queries, k, n_filters, filter_ids, filter_offsets, query_filter, out_ids, out_dists,
+                           out_counts);
+}
+
+int sdb_flat_last_filter_stats(sdb_index* ix, uint32_t* gathered_filters, uint32_t* scanned_filters, uint64_t* gathered_pairs) {
+  if (!ix) return fail(SDB_ERR_INVALID, "null index");
+  std::lock_guard<std::mutex> g(ix->mu);
+  if (gathered_filters) *gathered_filters = ix->flat_last_gathered;
+  if (scanned_filters) *scanned_filters = ix->flat_last_scanned;
+  if (gathered_pairs) *gathered_pairs = ix->flat_last_pairs;
   return SDB_OK;
 }
 

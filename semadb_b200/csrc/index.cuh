@@ -142,6 +142,16 @@ struct sdb_index {
   uint64_t flat_last_candidates = 0;  // tensor-core flat scan: candidates kept by the last level, all queries
   uint32_t flat_last_overflow = 0;    // ... and queries that fell back to the exact scan
   int flat_last_path = 0;             // 0 exact scan, 1 mma.sync candidate pass, 2 tcgen05 candidate pass
+  // filtered flat search (flat.cu launch_flat_filtered, flat_filter.cu): routes of the last flat call
+  // (sdb_flat_last_filter_stats), host staging of the gather route's work, device scratch of both routes
+  uint32_t flat_last_gathered = 0, flat_last_scanned = 0;  // filters that took each route
+  uint64_t flat_last_pairs = 0;                             // (request, id) pairs the gather route scored
+  std::vector<uint4> h_fg_items;
+  std::vector<uint32_t> h_fg_req;
+  sdb::DevBuf<uint4> d_fg_items;
+  sdb::DevBuf<uint32_t> d_fg_req, d_fg_part32, d_fsub_list, d_fsub_cnt;
+  sdb::DevBuf<float> d_fg_partf, d_fsub_q, d_fsub_d;
+  sdb::DevBuf<uint64_t> d_fsub_ids;
   uint64_t vec_epoch = 1, tc_epoch = 0;  // vec_epoch: bumped by every change to vec / exists
   sdb::DevBuf<uint16_t> d_x16, d_q16;
   sdb::DevBuf<float> d_xn, d_qn, d_thr, d_sample_d;
@@ -206,6 +216,25 @@ int launch_flat(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, c
 int launch_flat_exact(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, const uint32_t* d_filter_bits,
                       uint64_t* d_out_ids, float* d_out_dists, uint32_t* d_out_counts, cudaStream_t stream,
                       uint32_t first_id, uint32_t end_id);
+// Flat search of a batch whose requests carry filters (staged as by the Vamana search: ascending
+// u32 ids in d_ids, filter f = [h_off[f], h_off[f+1]), ids 0 and 1 and ids >= rows dropped);
+// query_filter[b] < 0 = request b unfiltered, nullptr = every request uses filter 0. Routes each
+// filter to the gather kernel or to the range scan and the unfiltered requests to launch_flat.
+int launch_flat_filtered(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, uint32_t n_filters,
+                         const uint32_t* h_off, const int32_t* query_filter, const uint32_t* d_ids, uint64_t* d_out_ids,
+                         float* d_out_dists, uint32_t* d_out_counts, cudaStream_t stream);
+// flat_filter.cu: score each work item's ids (x = batch row, [y, z) = range of d_ids) and merge a
+// request's items (d_req_items[r] .. d_req_items[r+1]) into output row d_req_rows[r]
+int launch_flat_gather(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, const uint32_t* d_ids,
+                       uint32_t n_items, const uint4* d_items, uint32_t n_req, const uint32_t* d_req_rows,
+                       const uint32_t* d_req_items, uint64_t* d_out_ids, float* d_out_dists, uint32_t* d_out_counts,
+                       cudaStream_t stream);
+// the row bitmap of an id list (d_bits: rows/32 words, cleared first)
+int launch_filter_bits(sdb_index* ix, const uint32_t* d_ids, uint32_t n, uint32_t* d_bits, cudaStream_t stream);
+// flat_tc.cu: compact the rows list[0..n) of a batch, and scatter a compacted batch's results back
+__global__ void gather_queries_kernel(const uint32_t* list, uint32_t n, const float* src, uint32_t dim, float* dst);
+__global__ void scatter_results_kernel(const uint32_t* list, uint32_t n, uint32_t k, const uint64_t* ids, const float* d,
+                                       const uint32_t* cnt, uint64_t* out_ids, float* out_d, uint32_t* out_cnt);
 bool flat_tc_eligible(const sdb_index* ix, uint32_t k, bool filtered);
 int launch_flat_tc(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, uint64_t* d_out_ids, float* d_out_dists,
                    uint32_t* d_out_counts, cudaStream_t stream);

@@ -374,6 +374,37 @@ class _DeviceIndex:
                                               _ptr(cnt, u32p)))
         return ids, d, cnt
 
+    def flat_search_batch_filters(self, queries, filters, query_filter=None, k: int = 10):
+        """Flat search with one filter per request, shaped like search_batch_filters: `filters` is a
+        list of id collections (an empty one filters everything out; ids that are not stored never
+        match), query_filter[b] the filter index of request b or -1 for none (None: every request
+        uses filters[0]). Row b equals flat_search_batch(queries[b:b+1], k, filters[query_filter[b]])."""
+        q = _f32(queries)
+        if q.ndim != 2 or q.shape[1] != self.dim:
+            raise SdbError(_capi.ERR_INVALID, "queries must be [B, dim]")
+        B = q.shape[0]
+        lists = [np.unique(_u64(f)) for f in filters]
+        off = np.zeros(len(lists) + 1, dtype=np.uint64)
+        off[1:] = np.cumsum([len(x) for x in lists])
+        flat = np.concatenate(lists) if lists and off[-1] else np.zeros(0, dtype=np.uint64)
+        qf = None if query_filter is None else np.ascontiguousarray(query_filter, dtype=np.int32)
+        ids = np.zeros((B, k), dtype=np.uint64)
+        d = np.zeros((B, k), dtype=np.float32)
+        cnt = np.zeros(B, dtype=np.uint32)
+        check(self._lib.sdb_flat_search_batch_filters(self._h, B, _ptr(q, f32p), k, len(lists),
+                                                      _ptr(flat, u64p) if len(flat) else None, _ptr(off, u64p),
+                                                      None if qf is None else _ptr(qf, _capi.i32p), _ptr(ids, u64p),
+                                                      _ptr(d, f32p), _ptr(cnt, u32p)))
+        return ids, d, cnt
+
+    def flat_last_filter_stats(self):
+        """(gathered_filters, scanned_filters, gathered_pairs) of the last flat search: filters that
+        took the gather route and the range-scan route, and the (request, id) pairs gathered."""
+        import ctypes as C
+        g, s, p = C.c_uint32(0), C.c_uint32(0), C.c_uint64(0)
+        check(self._lib.sdb_flat_last_filter_stats(self._h, C.byref(g), C.byref(s), C.byref(p)))
+        return g.value, s.value, p.value
+
     def flat_last_stats(self):
         """(path, candidates, overflowed) of the last flat_search_batch: path 0 = exact CUDA-core
         scan, 1 = mma.sync candidate pass, 2 = tcgen05 + TMA candidate pass."""
