@@ -189,11 +189,22 @@ int sdb_flat_search_batch_filters(sdb_index* ix, uint32_t B, const float* querie
 int sdb_flat_last_filter_stats(sdb_index* ix, uint32_t* gathered_filters, uint32_t* scanned_filters,
                                uint64_t* gathered_pairs);
 
-/* Diagnostics of the most recent sdb_flat_search_batch on this handle: path = 0 exact CUDA-core
+/* Unfiltered flat search with device-resident queries and outputs (the flat twin of
+ * sdb_search_batch_device): enqueues everything on `stream` (cudaStream_t) and returns without
+ * synchronising; row b equals sdb_flat_search_batch's row b on the same queries, byte for byte.
+ * Serves every store the flat search serves (f32 on the tensor-core or exact path, haversine, binary,
+ * PQ); a rebuild of the bf16 shadow after a store change runs on `stream` too. d_queries may be
+ * page-locked host memory (mapped). k must be 1..75. The first call of a larger shape allocates
+ * scratch, which synchronises the device. */
+int sdb_flat_search_batch_device(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, uint64_t* d_out_ids,
+                                 float* d_out_dists, uint32_t* d_out_counts, void* stream);
+/* Diagnostics of the most recent flat search on this handle: path = 0 exact CUDA-core
  * scan, 1 tensor-core candidate pass (mma.sync), 2 tensor-core candidate pass (tcgen05 + TMA);
  * candidates = (query, point) pairs the last candidate level kept for exact re-scoring, summed
  * over the batch; overflowed = queries that fell back to the exact scan. With filters, these
- * describe the pass that served the unfiltered requests (all 0 when there were none). */
+ * describe the pass that served the unfiltered requests (all 0 when there were none). After a
+ * device-entry call (sdb_flat_search_batch_device, sdb_flat_search_batch_gather_device) this waits
+ * for that call to complete on its stream before it reads the counters. */
 int sdb_flat_last_stats(sdb_index* ix, int32_t* path, uint64_t* candidates, uint32_t* overflowed);
 
 /* ---- insert: replaces IndexVamana.InsertUpdateDelete's insert branch (vamana.go:136-201,
@@ -320,11 +331,21 @@ typedef struct sdb_peer_gather {
 int sdb_search_batch_gather_device(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, uint32_t search_size,
                                    uint64_t* d_out_ids, float* d_out_dists, uint32_t* d_out_counts,
                                    const sdb_peer_gather* peers, void* stream);
+/* Flat shards: sdb_flat_search_batch_device on this GPU's shard, then one kernel stores every
+ * query's final list (the exact fallback of overflowed queries included) into slot [shard][query]
+ * of EVERY peer's buffer, byte for byte what the beam-search epilogue stores: ids (shard << 40 | id)
+ * and distances of the first count ranks, id 0 and +inf in the other slots, count
+ * min(count, per_shard_limit or k). Same argument checks and SDB_ERR_STATE refusal as
+ * sdb_search_batch_gather_device; k must be 1..75. Unfiltered; no synchronisation. */
+int sdb_flat_search_batch_gather_device(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k,
+                                        uint64_t* d_out_ids, float* d_out_dists, uint32_t* d_out_counts,
+                                        const sdb_peer_gather* peers, void* stream);
 int sdb_peer_barrier_device(int32_t device, uint32_t n_peers, uint32_t me, uint32_t* const* peer_flags, uint32_t epoch,
                             void* stream);
 /* A peer that never arrives is given ~20 s; the barrier kernel then records the timeout in a
  * page-locked status word of its device. From then on sdb_peer_barrier_device,
- * sdb_search_batch_gather_device and sdb_merge_topk_device on that device fail with SDB_ERR_STATE
+ * sdb_search_batch_gather_device, sdb_flat_search_batch_gather_device and sdb_merge_topk_device on
+ * that device fail with SDB_ERR_STATE
  * (the step whose barrier timed out merged stale slots). sdb_peer_barrier_check reads the word
  * (no synchronisation: call it after synchronising the step's stream to validate that step) and
  * returns SDB_OK or SDB_ERR_STATE; clear != 0 resets it once the caller has recovered. */

@@ -86,6 +86,10 @@ _SIGS = {
     "sdb_launch_count": (C.c_uint64, [H]),
     "sdb_search_visited": (C.c_int, [H, C.c_uint32, f32p, C.c_uint32, C.c_uint32, u64p, f32p, u32p]),
     "sdb_flat_search_batch": (C.c_int, [H, C.c_uint32, f32p, C.c_uint32, u64p, C.c_uint64, u64p, f32p, u32p]),
+    "sdb_flat_search_batch_device": (C.c_int, [H, C.c_uint32, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                               C.c_void_p]),
+    "sdb_flat_search_batch_gather_device": (C.c_int, [H, C.c_uint32, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p,
+                                                      C.c_void_p, C.POINTER(SdbPeerGather), C.c_void_p]),
     "sdb_flat_last_stats": (C.c_int, [H, i32p, u64p, u32p]),
     "sdb_flat_search_batch_filters": (C.c_int, [H, C.c_uint32, f32p, C.c_uint32, C.c_uint32, u64p, u64p, i32p, u64p, f32p,
                                                 u32p]),

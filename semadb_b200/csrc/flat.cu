@@ -42,7 +42,33 @@ struct FlatArgs {
   uint32_t* part_ids;         // [B][n_chunks][k]
   float* part_d;
   uint32_t* part_cnt;         // [B][n_chunks]
+  // query list on the device (launch_flat_exact_list): slot s < min(*qcount, B) is batch row
+  // qlist[s]; the split into chunks is derived from the count on the device
+  const uint32_t* qlist;
+  const uint32_t* qcount;
+  uint32_t sm_count;
 };
+
+struct FlatSplit {
+  uint32_t n_chunks, chunk;
+};
+
+// (query block x point chunk) split of a scan of nq queries over npts points: about 4 CTAs per SM,
+// chunks of at least 256 points, whole shared point tiles. The host (launch_flat_exact) and the
+// device (a list whose count only the device knows) derive the same split from the same count.
+__host__ __device__ inline FlatSplit flat_split(uint32_t nq, uint32_t npts, uint32_t tile_pts, uint32_t sm_count) {
+  const uint32_t qblocks = (nq + FQ - 1) / FQ;
+  uint32_t want = (sm_count * 4 + qblocks - 1) / qblocks;
+  if (want < 1) want = 1;
+  uint32_t max_chunks = (npts + 255) / 256;
+  if (max_chunks < 1) max_chunks = 1;
+  uint32_t n = want < max_chunks ? want : max_chunks;
+  if (n > 1024) n = 1024;
+  uint32_t chunk = (npts + n - 1) / n;
+  if (chunk == 0) chunk = 1;
+  chunk = (chunk + tile_pts - 1) / tile_pts * tile_pts;
+  return {npts == 0 ? 1 : (npts + chunk - 1) / chunk, chunk};
+}
 
 struct TopK {
   float d[FMAXK];
@@ -64,30 +90,31 @@ struct TopK {
   }
 };
 
+// One work item: query block qb (slots qb*FQ .. of nq) against point chunk c.
 // mode 0: f32 rows (METRIC template), 1: bits, 2: PQ codes via ADC table
 // QSMEM: the query tile fits transposed in shared memory; otherwise (large dim) each thread
 // streams its query row through L1.
-template <int MODE, int METRIC, bool QSMEM>
-__global__ void __launch_bounds__(FQ) flat_scan_kernel(FlatArgs a) {
-  extern __shared__ __align__(16) unsigned char sm[];
+template <int MODE, int METRIC, bool QSMEM, bool LIST>
+__device__ __forceinline__ void scan_item(const FlatArgs& a, unsigned char* sm, uint32_t qb, uint32_t c, uint32_t nq,
+                                          uint32_t chunk, uint32_t n_chunks) {
   const int tid = threadIdx.x;
-  const uint32_t q = blockIdx.x * FQ + tid;
-  const bool qvalid = q < a.B;
-  const uint32_t c = blockIdx.y;
-  uint32_t lo = a.first_id + c * a.chunk;
-  uint32_t hi = min(a.end_id, lo + a.chunk);
+  const uint32_t slot = qb * FQ + tid;
+  const bool qvalid = slot < nq;
+  const uint32_t q = qvalid ? (LIST ? a.qlist[slot] : slot) : 0;  // batch row
+  uint32_t lo = a.first_id + c * chunk;
+  uint32_t hi = min(a.end_id, lo + chunk);
   TopK top;
 
   if (MODE == 0) {
     // shared: qT[dim][FQ] floats, pt[FP][dim] floats
     float* qT = reinterpret_cast<float*>(sm);
     float* pt = qT + (QSMEM ? size_t(a.dim) * FQ : 0);
-    const float* qrow = a.queries + size_t(qvalid ? q : 0) * a.dim;
+    const float* qrow = a.queries + size_t(q) * a.dim;
     if (QSMEM) {
       for (uint32_t i = tid; i < a.dim * FQ; i += FQ) {
         uint32_t qq = i / a.dim, dd = i % a.dim;  // coalesced read of query rows
-        uint32_t gq = blockIdx.x * FQ + qq;
-        qT[dd * FQ + qq] = gq < a.B ? a.queries[size_t(gq) * a.dim + dd] : 0.0f;
+        uint32_t gs = qb * FQ + qq;
+        qT[dd * FQ + qq] = gs < nq ? a.queries[size_t(LIST ? a.qlist[gs] : gs) * a.dim + dd] : 0.0f;
       }
     }
     auto qat = [&](uint32_t i) -> float { return QSMEM ? qT[i * FQ + tid] : __ldg(qrow + i); };
@@ -161,7 +188,7 @@ __global__ void __launch_bounds__(FQ) flat_scan_kernel(FlatArgs a) {
       top.offer(pid, bits_finish(a.bit_metric, x, u), a.k);
     }
   } else {
-    const float* table = a.adc + size_t(qvalid ? q : 0) * a.pqM * a.pqK;
+    const float* table = a.adc + size_t(q) * a.pqM * a.pqK;
     for (uint32_t pid = lo; pid < hi; ++pid) {
       bool ok = a.exists[pid] && (!a.filter_bits || ((a.filter_bits[pid >> 5] >> (pid & 31)) & 1u));
       if (!ok || !qvalid) continue;
@@ -172,22 +199,44 @@ __global__ void __launch_bounds__(FQ) flat_scan_kernel(FlatArgs a) {
     }
   }
   if (qvalid) {
-    size_t o = (size_t(q) * a.n_chunks + c) * a.k;
+    size_t o = (size_t(slot) * n_chunks + c) * a.k;
     for (int i = 0; i < top.n; ++i) { a.part_ids[o + i] = top.id[i]; a.part_d[o + i] = top.d[i]; }
-    a.part_cnt[size_t(q) * a.n_chunks + c] = top.n;
+    a.part_cnt[size_t(slot) * n_chunks + c] = top.n;
   }
 }
 
-__global__ void flat_merge_kernel(const uint32_t* part_ids, const float* part_d, const uint32_t* part_cnt,
-                                  uint32_t n_chunks, uint32_t B, uint32_t k, uint64_t* out_ids, float* out_d,
-                                  uint32_t* out_cnt) {
-  uint32_t q = blockIdx.x * blockDim.x + threadIdx.x;
-  if (q >= B) return;
+// LIST = false: one work item per CTA, grid (query blocks, chunks) split on the host.
+// LIST = true: a fixed grid loops over the items of the split of min(*qcount, B) listed queries.
+template <int MODE, int METRIC, bool QSMEM, bool LIST>
+__global__ void __launch_bounds__(FQ) flat_scan_kernel(FlatArgs a) {
+  extern __shared__ __align__(16) unsigned char sm[];
+  if (!LIST) {
+    scan_item<MODE, METRIC, QSMEM, false>(a, sm, blockIdx.x, blockIdx.y, a.B, a.chunk, a.n_chunks);
+    return;
+  }
+  const uint32_t nq = min(*a.qcount, a.B);
+  if (nq == 0) return;
+  const FlatSplit s = flat_split(nq, a.end_id - a.first_id, a.tile_pts, a.sm_count);
+  const uint32_t items = (nq + FQ - 1) / FQ * s.n_chunks;
+  for (uint32_t w = blockIdx.x; w < items; w += gridDim.x) {
+    scan_item<MODE, METRIC, QSMEM, true>(a, sm, w / s.n_chunks, w % s.n_chunks, nq, s.chunk, s.n_chunks);
+    __syncthreads();  // the next item refills the shared query tile
+  }
+}
+
+// merges slot q's chunk lists in chunk order (= ascending id order) into output row q, or, with a
+// query list, into row qlist[q]
+__global__ void flat_merge_kernel(FlatArgs a, uint64_t* out_ids, float* out_d, uint32_t* out_cnt) {
+  const uint32_t s = blockIdx.x * blockDim.x + threadIdx.x;
+  const uint32_t nq = a.qlist ? min(*a.qcount, a.B) : a.B;
+  if (s >= nq) return;
+  const uint32_t n_chunks = a.qlist ? flat_split(nq, a.end_id - a.first_id, a.tile_pts, a.sm_count).n_chunks : a.n_chunks;
+  const uint32_t q = a.qlist ? a.qlist[s] : s, k = a.k;
   TopK top;
-  for (uint32_t c = 0; c < n_chunks; ++c) {  // chunk order = ascending id order
-    size_t o = (size_t(q) * n_chunks + c) * k;
-    uint32_t n = part_cnt[size_t(q) * n_chunks + c];
-    for (uint32_t i = 0; i < n; ++i) top.offer(part_ids[o + i], part_d[o + i], k);
+  for (uint32_t c = 0; c < n_chunks; ++c) {
+    size_t o = (size_t(s) * n_chunks + c) * k;
+    uint32_t n = a.part_cnt[size_t(s) * n_chunks + c];
+    for (uint32_t i = 0; i < n; ++i) top.offer(a.part_ids[o + i], a.part_d[o + i], k);
   }
   for (uint32_t i = 0; i < k; ++i) {
     out_ids[size_t(q) * k + i] = i < uint32_t(top.n) ? uint64_t(top.id[i]) : 0;
@@ -196,14 +245,39 @@ __global__ void flat_merge_kernel(const uint32_t* part_ids, const float* part_d,
   out_cnt[q] = top.n;
 }
 
-template <int MODE, int METRIC, bool QSMEM = true>
-int launch_scan(sdb_index* ix, const FlatArgs& a, size_t smem, cudaStream_t stream) {
-  auto kern = flat_scan_kernel<MODE, METRIC, QSMEM>;
+template <int MODE, int METRIC, bool QSMEM = true, bool LIST = false>
+int launch_scan(sdb_index* ix, const FlatArgs& a, size_t smem, uint32_t list_grid, cudaStream_t stream) {
+  auto kern = flat_scan_kernel<MODE, METRIC, QSMEM, LIST>;
   if (smem > 48 * 1024) SDB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem)));
-  dim3 grid((a.B + FQ - 1) / FQ, a.n_chunks);
+  dim3 grid = LIST ? dim3(list_grid) : dim3((a.B + FQ - 1) / FQ, a.n_chunks);
   kern<<<grid, FQ, smem, stream>>>(a);
   ix->launches++;
   SDB_CUDA(cudaGetLastError());
+  return SDB_OK;
+}
+
+// store and query fields of a scan over [first_id, end_id), and the rows of its shared point tile
+int flat_args(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, const uint32_t* d_filter_bits,
+              uint32_t first_id, uint32_t end_id, FlatArgs& a, bool& qsmem) {
+  a = FlatArgs{};
+  a.vec = ix->d_vec; a.vec_pitch = ix->vec_pitch;
+  a.bits = ix->d_bits; a.bits_pitch = ix->bits_pitch; a.words = ix->words;
+  a.codes = ix->d_codes; a.codes_pitch = ix->codes_pitch;
+  a.pqM = ix->pqM; a.pqK = ix->pqK;
+  a.bq_thr = ix->d_bq_thr; a.bit_metric = ix->bq_metric;
+  a.exists = ix->d_exists;
+  a.filter_bits = d_filter_bits;
+  a.queries = d_queries;
+  a.dim = ix->p.dim; a.B = B; a.k = k;
+  a.first_id = first_id;  // from 2: the start node is not a flat-index point
+  a.end_id = std::min(std::max(end_id, first_id), std::max<uint32_t>(2, ix->max_node_id + 1));
+  a.sm_count = uint32_t(ix->sm_count);
+  // f32 rows: the query tile in shared memory when it fits next to FP point rows; otherwise the
+  // queries are read through L1 and the point tile takes as many rows as fit (14 at dim 4096)
+  const size_t row_bytes = size_t(a.dim) * sizeof(float);
+  qsmem = (size_t(FQ) + FP) * row_bytes <= ix->smem_optin;
+  a.tile_pts = uint32_t(std::min<size_t>(FP, ix->smem_optin / row_bytes));
+  if (a.tile_pts == 0) return fail(SDB_ERR_INVALID, "flat scan: one vector does not fit in shared memory");
   return SDB_OK;
 }
 
@@ -216,41 +290,32 @@ int launch_flat(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, c
   if (flat_tc_eligible(ix, k, d_filter_bits != nullptr))
     return launch_flat_tc(ix, B, d_queries, k, d_out_ids, d_out_dists, d_out_counts, stream);
   ix->flat_last_path = 0;
+  ix->flat_stats_pending = false;
   return launch_flat_exact(ix, B, d_queries, k, d_filter_bits, d_out_ids, d_out_dists, d_out_counts, stream, 2,
                            std::max<uint32_t>(2, ix->max_node_id + 1));
+}
+
+// Unfiltered flat search of device-resident queries into device-resident outputs, all enqueued on
+// `stream` with no host synchronisation (once a call of the same shape has run: growing scratch
+// frees and allocates device memory). The host entry and both device entries run through it.
+int flat_device_locked(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, uint64_t* d_out_ids, float* d_out_dists,
+                       uint32_t* d_out_counts, cudaStream_t stream) {
+  ix->flat_last_gathered = ix->flat_last_scanned = 0;
+  ix->flat_last_pairs = 0;
+  return launch_flat(ix, B, d_queries, k, nullptr, d_out_ids, d_out_dists, d_out_counts, stream);
 }
 
 int launch_flat_exact(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, const uint32_t* d_filter_bits,
                       uint64_t* d_out_ids, float* d_out_dists, uint32_t* d_out_counts, cudaStream_t stream,
                       uint32_t first_id, uint32_t end_id) {
-  FlatArgs a{};
-  a.vec = ix->d_vec; a.vec_pitch = ix->vec_pitch;
-  a.bits = ix->d_bits; a.bits_pitch = ix->bits_pitch; a.words = ix->words;
-  a.codes = ix->d_codes; a.codes_pitch = ix->codes_pitch;
-  a.pqM = ix->pqM; a.pqK = ix->pqK;
-  a.bq_thr = ix->d_bq_thr; a.bit_metric = ix->bq_metric;
-  a.exists = ix->d_exists;
-  a.filter_bits = d_filter_bits;
-  a.queries = d_queries;
-  a.dim = ix->p.dim; a.B = B; a.k = k;
-  a.first_id = first_id;  // from 2: the start node is not a flat-index point
-  a.end_id = std::min(std::max(end_id, first_id), std::max<uint32_t>(2, ix->max_node_id + 1));
-  uint32_t npts = a.end_id - a.first_id;
-  uint32_t qblocks = (B + FQ - 1) / FQ;
-  uint32_t want = std::max<uint32_t>(1, (uint32_t(ix->sm_count) * 4 + qblocks - 1) / qblocks);
-  uint32_t max_chunks = std::max<uint32_t>(1, (npts + 255) / 256);
-  a.n_chunks = std::min<uint32_t>(std::min<uint32_t>(want, max_chunks), 1024);
-  a.chunk = (npts + a.n_chunks - 1) / a.n_chunks;
-  if (a.chunk == 0) a.chunk = 1;
-  // f32 rows: the query tile in shared memory when it fits next to FP point rows; otherwise the
-  // queries are read through L1 and the point tile takes as many rows as fit (14 at dim 4096)
-  const size_t row_bytes = size_t(a.dim) * sizeof(float);
-  const bool qsmem = (size_t(FQ) + FP) * row_bytes <= ix->smem_optin;
-  a.tile_pts = uint32_t(std::min<size_t>(FP, ix->smem_optin / row_bytes));
-  if (a.tile_pts == 0) return fail(SDB_ERR_INVALID, "flat scan: one vector does not fit in shared memory");
-  a.chunk = (a.chunk + a.tile_pts - 1) / a.tile_pts * a.tile_pts;
-  a.n_chunks = npts == 0 ? 1 : (npts + a.chunk - 1) / a.chunk;
+  FlatArgs a;
+  bool qsmem;
   int rc;
+  if ((rc = flat_args(ix, B, d_queries, k, d_filter_bits, first_id, end_id, a, qsmem))) return rc;
+  const uint32_t npts = a.end_id - a.first_id;
+  const FlatSplit sp = flat_split(B, npts, a.tile_pts, a.sm_count);
+  a.n_chunks = sp.n_chunks;
+  a.chunk = sp.chunk;
   size_t parts = size_t(B) * a.n_chunks * k;
   if ((rc = ix->d_tmp32.ensure(parts + size_t(B) * a.n_chunks))) return rc;
   if ((rc = ix->d_tmpf.ensure(parts))) return rc;
@@ -258,33 +323,79 @@ int launch_flat_exact(sdb_index* ix, uint32_t B, const float* d_queries, uint32_
   a.part_cnt = ix->d_tmp32.p + parts;
   a.part_d = ix->d_tmpf.p;
 
+  const size_t row_bytes = size_t(a.dim) * sizeof(float);
   if (ix->p.quantizer == SDB_QUANT_BINARY && ix->bq_fitted) {
     size_t smem = size_t(FQ) * (a.words | 1) * 8;
-    if ((rc = launch_scan<1, 0>(ix, a, smem, stream))) return rc;
+    if ((rc = launch_scan<1, 0>(ix, a, smem, 0, stream))) return rc;
   } else if (ix->p.quantizer == SDB_QUANT_PRODUCT && ix->pq_fitted) {
     if ((rc = ix->d_adc.ensure(size_t(B) * ix->pqM * ix->pqK))) return rc;
     if ((rc = launch_adc_tables(ix, B, d_queries, ix->d_adc.p, stream))) return rc;
     a.adc = ix->d_adc.p;
-    if ((rc = launch_scan<2, 0>(ix, a, 0, stream))) return rc;
+    if ((rc = launch_scan<2, 0>(ix, a, 0, 0, stream))) return rc;
   } else {
     const size_t smem = ((qsmem ? size_t(FQ) : 0) + a.tile_pts) * row_bytes;
     switch (ix->store_metric) {
       case SDB_METRIC_EUCLIDEAN:
-        rc = qsmem ? launch_scan<0, METRIC_EUCLIDEAN, true>(ix, a, smem, stream) : launch_scan<0, METRIC_EUCLIDEAN, false>(ix, a, smem, stream);
+        rc = qsmem ? launch_scan<0, METRIC_EUCLIDEAN, true>(ix, a, smem, 0, stream) : launch_scan<0, METRIC_EUCLIDEAN, false>(ix, a, smem, 0, stream);
         break;
       case SDB_METRIC_DOT:
-        rc = qsmem ? launch_scan<0, METRIC_DOT, true>(ix, a, smem, stream) : launch_scan<0, METRIC_DOT, false>(ix, a, smem, stream);
+        rc = qsmem ? launch_scan<0, METRIC_DOT, true>(ix, a, smem, 0, stream) : launch_scan<0, METRIC_DOT, false>(ix, a, smem, 0, stream);
         break;
       case SDB_METRIC_COSINE:
-        rc = qsmem ? launch_scan<0, METRIC_COSINE, true>(ix, a, smem, stream) : launch_scan<0, METRIC_COSINE, false>(ix, a, smem, stream);
+        rc = qsmem ? launch_scan<0, METRIC_COSINE, true>(ix, a, smem, 0, stream) : launch_scan<0, METRIC_COSINE, false>(ix, a, smem, 0, stream);
         break;
-      case SDB_METRIC_HAVERSINE: rc = launch_scan<0, METRIC_HAVERSINE, true>(ix, a, smem, stream); break;
+      case SDB_METRIC_HAVERSINE: rc = launch_scan<0, METRIC_HAVERSINE, true>(ix, a, smem, 0, stream); break;
       default: return fail(SDB_ERR_INVALID, "metric not supported by the flat scan");
     }
     if (rc) return rc;
   }
-  flat_merge_kernel<<<(B + 127) / 128, 128, 0, stream>>>(a.part_ids, a.part_d, a.part_cnt, a.n_chunks, B, k, d_out_ids,
-                                                         d_out_dists, d_out_counts);
+  flat_merge_kernel<<<(B + 127) / 128, 128, 0, stream>>>(a, d_out_ids, d_out_dists, d_out_counts);
+  ix->launches++;
+  SDB_CUDA(cudaGetLastError());
+  return SDB_OK;
+}
+
+int launch_flat_exact_list(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, const uint32_t* d_list,
+                           const uint32_t* d_count, uint64_t* d_out_ids, float* d_out_dists, uint32_t* d_out_counts,
+                           cudaStream_t stream, uint32_t first_id, uint32_t end_id) {
+  if (ix->quant_active() || ix->store_metric == SDB_METRIC_HAVERSINE)
+    return fail(SDB_ERR_INTERNAL, "flat scan of a query list: f32 squared-L2 / dot / cosine stores only");
+  FlatArgs a;
+  bool qsmem;
+  int rc;
+  if ((rc = flat_args(ix, B, d_queries, k, nullptr, first_id, end_id, a, qsmem))) return rc;
+  a.qlist = d_list;
+  a.qcount = d_count;
+  // the count is only known on the device: size the partial lists and the grid for the largest
+  // split any count 1..B can take (one CTA per work item at the worst count)
+  const uint32_t npts = a.end_id - a.first_id;
+  size_t parts = 0;
+  uint32_t grid = 1;
+  for (uint32_t qb = 1; qb <= (B + FQ - 1) / FQ; ++qb) {
+    const uint32_t nq = std::min(B, qb * FQ);
+    const FlatSplit sp = flat_split(nq, npts, a.tile_pts, a.sm_count);
+    parts = std::max(parts, size_t(nq) * sp.n_chunks);
+    grid = std::max(grid, qb * sp.n_chunks);
+  }
+  if ((rc = ix->d_tmp32.ensure(parts * (k + 1)))) return rc;
+  if ((rc = ix->d_tmpf.ensure(parts * k))) return rc;
+  a.part_ids = ix->d_tmp32.p;
+  a.part_cnt = ix->d_tmp32.p + parts * k;
+  a.part_d = ix->d_tmpf.p;
+  const size_t smem = ((qsmem ? size_t(FQ) : 0) + a.tile_pts) * size_t(a.dim) * sizeof(float);
+  switch (ix->store_metric) {
+    case SDB_METRIC_EUCLIDEAN:
+      rc = qsmem ? launch_scan<0, METRIC_EUCLIDEAN, true, true>(ix, a, smem, grid, stream) : launch_scan<0, METRIC_EUCLIDEAN, false, true>(ix, a, smem, grid, stream);
+      break;
+    case SDB_METRIC_DOT:
+      rc = qsmem ? launch_scan<0, METRIC_DOT, true, true>(ix, a, smem, grid, stream) : launch_scan<0, METRIC_DOT, false, true>(ix, a, smem, grid, stream);
+      break;
+    default:
+      rc = qsmem ? launch_scan<0, METRIC_COSINE, true, true>(ix, a, smem, grid, stream) : launch_scan<0, METRIC_COSINE, false, true>(ix, a, smem, grid, stream);
+      break;
+  }
+  if (rc) return rc;
+  flat_merge_kernel<<<(B + 127) / 128, 128, 0, stream>>>(a, d_out_ids, d_out_dists, d_out_counts);
   ix->launches++;
   SDB_CUDA(cudaGetLastError());
   return SDB_OK;
@@ -355,6 +466,7 @@ int launch_flat_filtered(sdb_index* ix, uint32_t B, const float* d_queries, uint
   ix->flat_last_path = 0;
   ix->flat_last_candidates = 0;
   ix->flat_last_overflow = 0;
+  ix->flat_stats_pending = false;
   for (uint32_t f = 0; f < n_filters; ++f) {
     const uint64_t nf = first[f + 1] - first[f], mf = h_off[f + 1] - h_off[f];
     if (nf == 0) continue;

@@ -1180,44 +1180,35 @@ int launch_flat_tc(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k
     lvl_begin = lvl_end;
   }
   }  // level scheme
-  // ---- queries whose candidate list overflowed at some level: exact scan
-  // [1] overflow count, [2..3] diagnostic (sdb_flat_last_stats): candidates the last level kept, summed
-  // over the batch by the last re-score (a 16-byte read-back instead of the B counts)
-  // host-buffer call (sdb_flat_search_batch): the result copies go in front of the one synchronisation
-  auto copy_out = [&]() -> int {
-    const auto& ho = ix->flat_host_out;
-    if (!ho.armed) return SDB_OK;
-    SDB_CUDA(cudaMemcpyAsync(ho.ids, d_out_ids, size_t(B) * k * sizeof(uint64_t), cudaMemcpyDeviceToHost, stream));
-    SDB_CUDA(cudaMemcpyAsync(ho.dists, d_out_dists, size_t(B) * k * sizeof(float), cudaMemcpyDeviceToHost, stream));
-    SDB_CUDA(cudaMemcpyAsync(ho.counts, d_out_counts, size_t(B) * sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
-    return SDB_OK;
-  };
-  if ((rc = copy_out())) return rc;
-  uint32_t h_misc[4] = {0, 0, 0, 0};
-  SDB_CUDA(cudaMemcpyAsync(h_misc, d_misc, sizeof(h_misc), cudaMemcpyDeviceToHost, stream));
-  SDB_CUDA(cudaStreamSynchronize(stream));
-  const uint32_t h_ovf = h_misc[1];
-  ix->flat_last_candidates = uint64_t(h_misc[2]) | (uint64_t(h_misc[3]) << 32);
-  ix->flat_last_overflow = h_ovf;
+  // ---- queries whose candidate list overflowed at some level: the exact scan of the list the
+  // re-score built (d_ovf_list, count d_misc[1]). Enqueued every time and split by the count on the
+  // device, so nothing here waits for the host: two near-empty launches when nothing overflowed.
+  if ((rc = launch_flat_exact_list(ix, B, d_queries, k, d_ovf_list, d_misc + 1, d_out_ids, d_out_dists, d_out_counts, stream,
+                                   first_id, end_id)))
+    return rc;
+  // [1] overflow count, [2..3] candidates the last level kept, summed over the batch by the last
+  // re-score: a 16-byte copy into page-locked memory behind the last kernel, read by
+  // flat_stats_settle once the call has completed
+  if ((rc = ix->h_flat_misc.ensure(4))) return rc;
+  if (!ix->flat_stats_ev) SDB_CUDA(cudaEventCreateWithFlags(&ix->flat_stats_ev, cudaEventDisableTiming));
+  SDB_CUDA(cudaMemcpyAsync(ix->h_flat_misc.p, d_misc, 4 * sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
+  SDB_CUDA(cudaEventRecord(ix->flat_stats_ev, stream));
+  ix->flat_stats_pending = true;
   ix->flat_last_path = t5_eligible(kp) ? 2 : 1;
-  if (debug) fprintf(stderr, "[sdb] flat tc: %u of %u queries overflowed -> exact scan\n", h_ovf, B);
-  if (h_ovf) {
-    DevBuf<float> d_q2, d_d2;
-    DevBuf<uint64_t> d_i2;
-    DevBuf<uint32_t> d_c2;
-    struct Rel { DevBuf<float>&a, &b; DevBuf<uint64_t>& c; DevBuf<uint32_t>& d; ~Rel() { a.release(); b.release(); c.release(); d.release(); } } rel{d_q2, d_d2, d_i2, d_c2};
-    if ((rc = d_q2.ensure(size_t(h_ovf) * dim)) || (rc = d_d2.ensure(size_t(h_ovf) * k)) || (rc = d_i2.ensure(size_t(h_ovf) * k)) ||
-        (rc = d_c2.ensure(h_ovf)))
-      return rc;
-    gather_queries_kernel<<<h_ovf, 128, 0, stream>>>(d_ovf_list, h_ovf, d_queries, dim, d_q2.p);
-    if ((rc = launch_flat_exact(ix, h_ovf, d_q2.p, k, nullptr, d_i2.p, d_d2.p, d_c2.p, stream, first_id, end_id))) return rc;
-    scatter_results_kernel<<<h_ovf, 128, 0, stream>>>(d_ovf_list, h_ovf, k, d_i2.p, d_d2.p, d_c2.p, d_out_ids, d_out_dists, d_out_counts);
-    ix->launches += 2;
-    SDB_CUDA(cudaGetLastError());
-    if ((rc = copy_out())) return rc;  // again, with the exact lists of the overflowed queries
+  if (debug) {
     SDB_CUDA(cudaStreamSynchronize(stream));
+    fprintf(stderr, "[sdb] flat tc: %u of %u queries overflowed -> exact scan\n", ix->h_flat_misc.p[1], B);
   }
-  if (ix->flat_host_out.armed) ix->flat_host_out.done = true;
+  return SDB_OK;
+}
+
+int flat_stats_settle(sdb_index* ix) {
+  if (!ix->flat_stats_pending) return SDB_OK;
+  SDB_CUDA(cudaEventSynchronize(ix->flat_stats_ev));
+  const uint32_t* h = ix->h_flat_misc.p;
+  ix->flat_last_candidates = uint64_t(h[2]) | (uint64_t(h[3]) << 32);
+  ix->flat_last_overflow = h[1];
+  ix->flat_stats_pending = false;
   return SDB_OK;
 }
 
@@ -1226,6 +1217,8 @@ int launch_flat_tc(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k
 extern "C" int sdb_flat_last_stats(sdb_index* ix, int32_t* path, uint64_t* candidates, uint32_t* overflowed) {
   if (!ix) return sdb::fail(SDB_ERR_INVALID, "null index");
   std::lock_guard<std::mutex> g(ix->mu);
+  SDB_CUDA(cudaSetDevice(ix->device));
+  if (int rc = sdb::flat_stats_settle(ix)) return rc;  // waits for a device-entry call still in flight
   if (path) *path = ix->flat_last_path;
   if (candidates) *candidates = ix->flat_last_candidates;
   if (overflowed) *overflowed = ix->flat_last_overflow;

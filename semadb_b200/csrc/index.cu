@@ -287,6 +287,8 @@ void sdb_index_destroy(sdb_index* ix) {
   ix->d_ndist.release(); ix->d_work.release(); ix->d_adc.release(); ix->d_filter_ids.release(); ix->d_filter_off.release();
   ix->d_filter_bits.release(); ix->d_qmap.release(); ix->d_query_filter.release(); ix->d_retry_bitmap.release(); ix->d_vis_ids.release(); ix->d_vis_len.release(); ix->d_vis_d.release();
   ix->d_ids64.release(); ix->d_tmp32.release(); ix->d_tmpf.release(); ix->d_tmp8.release(); ix->h_stage.release();
+  ix->h_flat_misc.release();
+  if (ix->flat_stats_ev) cudaEventDestroy(ix->flat_stats_ev);
   for (auto& e : ix->prof_ev)
     if (e) cudaEventDestroy(e);
   if (ix->stream) cudaStreamDestroy(ix->stream);
@@ -762,20 +764,15 @@ static int flat_batch_locked(sdb_index* ix, uint32_t B, const float* queries, ui
                               ix->d_oc.p, ix->stream);
     if (rc) return rc;
   } else {
-    ix->flat_last_gathered = ix->flat_last_scanned = 0;
-    ix->flat_last_pairs = 0;
-    ix->flat_host_out.ids = out_ids; ix->flat_host_out.dists = out_dists; ix->flat_host_out.counts = out_counts;
-    ix->flat_host_out.armed = true; ix->flat_host_out.done = false;
-    rc = launch_flat(ix, B, ix->d_q.p, k, nullptr, ix->d_oid.p, ix->d_od.p, ix->d_oc.p, ix->stream);
-    ix->flat_host_out.armed = false;
+    rc = flat_device_locked(ix, B, ix->d_q.p, k, ix->d_oid.p, ix->d_od.p, ix->d_oc.p, ix->stream);
     if (rc) return rc;
-    if (ix->flat_host_out.done) return SDB_OK;  // copied and synchronised by the tensor-core path
   }
+  // the result copies go in front of the call's one synchronisation
   SDB_CUDA(cudaMemcpyAsync(out_ids, ix->d_oid.p, size_t(B) * k * sizeof(uint64_t), cudaMemcpyDeviceToHost, ix->stream));
   SDB_CUDA(cudaMemcpyAsync(out_dists, ix->d_od.p, size_t(B) * k * sizeof(float), cudaMemcpyDeviceToHost, ix->stream));
   SDB_CUDA(cudaMemcpyAsync(out_counts, ix->d_oc.p, size_t(B) * sizeof(uint32_t), cudaMemcpyDeviceToHost, ix->stream));
   SDB_CUDA(cudaStreamSynchronize(ix->stream));
-  return SDB_OK;
+  return flat_stats_settle(ix);
 }
 
 int sdb_flat_search_batch(sdb_index* ix, uint32_t B, const float* queries, uint32_t k, const uint64_t* filter_ids,
@@ -806,6 +803,17 @@ int sdb_flat_search_batch_filters(sdb_index* ix, uint32_t B, const float* querie
   SDB_CUDA(cudaSetDevice(ix->device));
   return flat_batch_locked(ix, B, queries, k, n_filters, filter_ids, filter_offsets, query_filter, out_ids, out_dists,
                            out_counts);
+}
+
+int sdb_flat_search_batch_device(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, uint64_t* d_out_ids,
+                                 float* d_out_dists, uint32_t* d_out_counts, void* stream) {
+  if (!ix) return fail(SDB_ERR_INVALID, "null index");
+  if (B == 0) return SDB_OK;
+  if (!d_queries || !d_out_ids || !d_out_dists || !d_out_counts) return fail(SDB_ERR_INVALID, "null argument");
+  if (k < 1 || k > 75) return fail(SDB_ERR_INVALID, "invalid limit for vector query, expected 1-75");  // models/search.go:329
+  std::lock_guard<std::mutex> g(ix->mu);
+  SDB_CUDA(cudaSetDevice(ix->device));
+  return flat_device_locked(ix, B, d_queries, k, d_out_ids, d_out_dists, d_out_counts, static_cast<cudaStream_t>(stream));
 }
 
 int sdb_flat_last_filter_stats(sdb_index* ix, uint32_t* gathered_filters, uint32_t* scanned_filters, uint64_t* gathered_pairs) {

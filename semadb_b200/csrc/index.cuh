@@ -136,12 +136,14 @@ struct sdb_index {
   sdb::DevBuf<uint8_t> d_tmp8;
   sdb::PinBuf<uint8_t> h_stage;
   // tensor-core flat scan (flat_tc.cu): bf16 shadow of the store + per-call scratch
-  // sdb_flat_search_batch arms this with the caller's host buffers: the tensor-core path then queues the
-  // result copies itself, in front of its one synchronisation (flat_tc.cu), and sets done
-  struct FlatHostOut { uint64_t* ids = nullptr; float* dists = nullptr; uint32_t* counts = nullptr; bool armed = false, done = false; } flat_host_out;
   uint64_t flat_last_candidates = 0;  // tensor-core flat scan: candidates kept by the last level, all queries
   uint32_t flat_last_overflow = 0;    // ... and queries that fell back to the exact scan
   int flat_last_path = 0;             // 0 exact scan, 1 mma.sync candidate pass, 2 tcgen05 candidate pass
+  // the two counters above as the last tensor-core call left them on the device: copied to h_flat_misc
+  // behind its last kernel, event recorded after the copy; flat_stats_settle reads them when pending
+  sdb::PinBuf<uint32_t> h_flat_misc;
+  cudaEvent_t flat_stats_ev = nullptr;
+  bool flat_stats_pending = false;
   // filtered flat search (flat.cu launch_flat_filtered, flat_filter.cu): routes of the last flat call
   // (sdb_flat_last_filter_stats), host staging of the gather route's work, device scratch of both routes
   uint32_t flat_last_gathered = 0, flat_last_scanned = 0;  // filters that took each route
@@ -216,6 +218,17 @@ int launch_flat(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, c
 int launch_flat_exact(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, const uint32_t* d_filter_bits,
                       uint64_t* d_out_ids, float* d_out_dists, uint32_t* d_out_counts, cudaStream_t stream,
                       uint32_t first_id, uint32_t end_id);
+// the exact scan of the batch rows d_list[0 .. min(*d_count, B)) (f32 stores without a filter): the
+// count is read on the device, which splits the scan from it as launch_flat_exact does from B; each
+// row's list goes to its row of the outputs, other rows are left as they are
+int launch_flat_exact_list(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, const uint32_t* d_list,
+                           const uint32_t* d_count, uint64_t* d_out_ids, float* d_out_dists, uint32_t* d_out_counts,
+                           cudaStream_t stream, uint32_t first_id, uint32_t end_id);
+// completes flat_last_candidates / flat_last_overflow of the last tensor-core call (waits for it)
+int flat_stats_settle(sdb_index* ix);
+// unfiltered flat search, device queries and outputs, enqueued on `stream` (index.cu)
+int flat_device_locked(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, uint64_t* d_out_ids, float* d_out_dists,
+                       uint32_t* d_out_counts, cudaStream_t stream);
 // Flat search of a batch whose requests carry filters (staged as by the Vamana search: ascending
 // u32 ids in d_ids, filter f = [h_off[f], h_off[f+1]), ids 0 and 1 and ids >= rows dropped);
 // query_filter[b] < 0 = request b unfiltered, nullptr = every request uses filter 0. Routes each

@@ -1,4 +1,5 @@
-// search.cu — dispatch of the beam-search kernel variants (search.cuh).
+// search.cu — dispatch of the beam-search kernel variants (search.cuh), and the entries that search
+// a shard and store its lists into every peer GPU's gather buffer (beam search and flat search).
 #include "search_launch.cuh"
 
 #include <algorithm>
@@ -151,6 +152,46 @@ static int dispatch_search(sdb_index* ix, const SearchArgs& a, bool filtered, cu
   }
 }
 
+// the caller's peer buffers (sdb_peer_gather) as the kernels take them, for a top-k of k slots
+static int peer_gather_args(const sdb_peer_gather* pg, uint32_t k, PeerGather* g) {
+  if (pg->n_peers == 0 || pg->n_peers > SDB_MAX_PEERS || pg->shard >= (1u << 24))
+    return fail(SDB_ERR_INVALID, "peer gather: n_peers must be 1..16");
+  *g = PeerGather{};
+  g->n = pg->n_peers;
+  g->shard = pg->shard;
+  g->limit = pg->per_shard_limit == 0 || pg->per_shard_limit > k ? k : pg->per_shard_limit;
+  g->tag = uint64_t(pg->shard) << 40;
+  for (uint32_t p = 0; p < pg->n_peers; ++p) {
+    if (!pg->ids[p] || !pg->dists[p] || !pg->counts[p]) return fail(SDB_ERR_INVALID, "peer gather: null peer buffer");
+    g->ids[p] = pg->ids[p];
+    g->dists[p] = pg->dists[p];
+    g->counts[p] = pg->counts[p];
+  }
+  return SDB_OK;
+}
+
+// Flat shards: the flat search's last writer is known only once its whole sequence has run (the
+// overflow fallback rewrites rows after the re-score), so a kernel of its own publishes the final
+// lists. Slot [shard][q] of every peer's buffer gets the bytes the beam-search epilogue stores:
+// tagged ids and the distances of the first count ranks, id 0 / +inf in the rest, count
+// min(count, limit). One thread per (query, rank); rank 0's thread also writes the counts.
+__global__ void flat_publish_kernel(PeerGather g, uint32_t B, uint32_t k, const uint64_t* ids, const float* dists,
+                                    const uint32_t* counts) {
+  const uint64_t t = uint64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (t >= uint64_t(B) * k) return;
+  const uint32_t q = uint32_t(t / k), r = uint32_t(t % k);
+  const uint32_t cnt = min(counts[q], k);
+  const bool have = r < cnt;
+  const uint64_t id = have ? (ids[t] | g.tag) : 0;
+  const float d = have ? dists[t] : __int_as_float(0x7f800000);
+  const size_t o = (size_t(g.shard) * B + q) * k + r;
+  for (uint32_t s = 0; s < g.n; ++s) {
+    g.ids[s][o] = id;
+    g.dists[s][o] = d;
+    if (r == 0) g.counts[s][size_t(g.shard) * B + q] = min(cnt, g.limit);
+  }
+}
+
 }  // namespace sdb
 
 using namespace sdb;
@@ -161,20 +202,9 @@ extern "C" int sdb_search_batch_gather_device(sdb_index* ix, uint32_t B, const f
   if (!ix || !pg) return fail(SDB_ERR_INVALID, "null argument");
   if (B == 0) return SDB_OK;
   if (!d_queries || !d_out_ids || !d_out_dists || !d_out_counts) return fail(SDB_ERR_INVALID, "null argument");
-  if (pg->n_peers == 0 || pg->n_peers > SDB_MAX_PEERS || pg->shard >= (1u << 24))
-    return fail(SDB_ERR_INVALID, "peer gather: n_peers must be 1..16");
+  PeerGather g;
+  if (int prc = peer_gather_args(pg, k, &g)) return prc;
   if (k == 0 || search_size < k) return fail(SDB_ERR_INVALID, "searchSize must be greater than or equal to k");
-  PeerGather g{};
-  g.n = pg->n_peers;
-  g.shard = pg->shard;
-  g.limit = pg->per_shard_limit == 0 || pg->per_shard_limit > k ? k : pg->per_shard_limit;
-  g.tag = uint64_t(pg->shard) << 40;
-  for (uint32_t p = 0; p < pg->n_peers; ++p) {
-    if (!pg->ids[p] || !pg->dists[p] || !pg->counts[p]) return fail(SDB_ERR_INVALID, "peer gather: null peer buffer");
-    g.ids[p] = pg->ids[p];
-    g.dists[p] = pg->dists[p];
-    g.counts[p] = pg->counts[p];
-  }
   std::lock_guard<std::mutex> lk(ix->mu);
   SDB_CUDA(cudaSetDevice(ix->device));
   if (int prc = peer_barrier_poisoned(ix->device)) return prc;
@@ -185,3 +215,24 @@ extern "C" int sdb_search_batch_gather_device(sdb_index* ix, uint32_t B, const f
   return rc;
 }
 
+extern "C" int sdb_flat_search_batch_gather_device(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k,
+                                                   uint64_t* d_out_ids, float* d_out_dists, uint32_t* d_out_counts,
+                                                   const sdb_peer_gather* pg, void* stream) {
+  if (!ix || !pg) return fail(SDB_ERR_INVALID, "null argument");
+  if (B == 0) return SDB_OK;
+  if (!d_queries || !d_out_ids || !d_out_dists || !d_out_counts) return fail(SDB_ERR_INVALID, "null argument");
+  PeerGather g;
+  if (int prc = peer_gather_args(pg, k, &g)) return prc;
+  if (k < 1 || k > 75) return fail(SDB_ERR_INVALID, "invalid limit for vector query, expected 1-75");  // models/search.go:329
+  std::lock_guard<std::mutex> lk(ix->mu);
+  SDB_CUDA(cudaSetDevice(ix->device));
+  if (int prc = peer_barrier_poisoned(ix->device)) return prc;
+  const cudaStream_t st = static_cast<cudaStream_t>(stream);
+  int rc = flat_device_locked(ix, B, d_queries, k, d_out_ids, d_out_dists, d_out_counts, st);
+  if (rc) return rc;
+  const uint64_t n = uint64_t(B) * k;
+  flat_publish_kernel<<<uint32_t((n + 255) / 256), 256, 0, st>>>(g, B, k, d_out_ids, d_out_dists, d_out_counts);
+  ix->launches++;
+  SDB_CUDA(cudaGetLastError());
+  return SDB_OK;
+}

@@ -14,6 +14,9 @@ uniform random partition into near-equal shards (SURVEY.md §2a).
 
 One process per GPU (torch.distributed, backend nccl); torch is plumbing only (device
 tensors, the collective). The merge runs through the C ABI.
+
+The shards carry either index kind: an IndexVamana shard runs the beam search, an IndexFlat shard
+the flat search (every point of the shard scanned, so G GPUs each scan N/G points).
 """
 from __future__ import annotations
 
@@ -132,7 +135,9 @@ class ShardedSearcher:
     def __init__(self, index, rank: Optional[int] = None, world: Optional[int] = None, group=None,
                  exchange: str = "auto", pipeline: bool = False):
         import torch.distributed as dist
+        from .vamana import IndexFlat
         self.index = index
+        self._flat = isinstance(index, IndexFlat)  # search_size is unused for a flat index
         self.group = group
         self.exchange = exchange
         self.pipeline = pipeline  # fused exchange only: barrier + merge of step e overlap the search of step e+1
@@ -177,7 +182,27 @@ class ShardedSearcher:
                       torch.zeros((B, k), dtype=torch.float32, device=device),
                       torch.zeros((B,), dtype=torch.int32, device=device))
 
-    def search_batch_pinned(self, h_queries, k: int, search_size: int, h_ids, h_dists, h_counts, device,
+    def _search_shard(self, q, k: int, search_size, l_ids, l_d, l_c, stream, pg=None):
+        """This rank's shard search of the [B, dim] query tensor q (device or page-locked) into l_*
+        and, with pg, into slot [rank] of every peer's gather buffer: the flat entries for an
+        IndexFlat, the beam-search entries otherwise. Enqueued on `stream`, no synchronisation."""
+        B = int(q.shape[0])
+        L = None if self._flat else (self.index.L if search_size is None else int(search_size))
+        if pg is None:
+            if self._flat:
+                self.index.flat_search_batch_device(q, k, l_ids, l_d, l_c, stream)
+            else:
+                self.index.search_batch_device(q, k, L, l_ids, l_d, l_c, stream)
+            return
+        lib = _capi.lib()
+        outs = (l_ids.data_ptr(), l_d.data_ptr(), l_c.data_ptr())
+        if self._flat:
+            rc = lib.sdb_flat_search_batch_gather_device(self.index._h, B, q.data_ptr(), k, *outs, C.byref(pg), stream)
+        else:
+            rc = lib.sdb_search_batch_gather_device(self.index._h, B, q.data_ptr(), k, L, *outs, C.byref(pg), stream)
+        _capi.check(rc)
+
+    def search_batch_pinned(self, h_queries, k: int, search_size: Optional[int], h_ids, h_dists, h_counts, device,
                             max_search_limit: int = 75):
         """Host-facing twin of search_batch_device for page-locked (pinned) torch CPU tensors:
         pinned memory is mapped into the device address space, so K1 reads the broadcast query
@@ -207,8 +232,7 @@ class ShardedSearcher:
         pg.per_shard_limit = shard_limit(k, self.world, max_search_limit)
         lib = _capi.lib()
         di = device.index or 0
-        _capi.check(lib.sdb_search_batch_gather_device(self.index._h, B, h_queries.data_ptr(), k, search_size,
-                                                       l_ids.data_ptr(), l_d.data_ptr(), l_c.data_ptr(), C.byref(pg), stream))
+        self._search_shard(h_queries, k, search_size, l_ids, l_d, l_c, stream, pg)
         _capi.check(lib.sdb_peer_barrier_device(di, self.world, self.rank, pb._flags, pb.epoch, stream))
         g_i, g_dd, g_cc = pb.local(par)
         # The merge is a short kernel: its 300 k small stores would sit exposed on PCIe if they went
@@ -224,9 +248,10 @@ class ShardedSearcher:
         # the step is complete on this GPU: a barrier that gave up on a peer makes it an error
         _capi.check(lib.sdb_peer_barrier_check(di, 0))
 
-    def search_batch_device(self, d_queries, k: int, search_size: int, max_search_limit: int = 75):
+    def search_batch_device(self, d_queries, k: int, search_size: Optional[int], max_search_limit: int = 75):
         """d_queries: [B, dim] f32 CUDA tensor, identical on every rank (broadcast by the
-        caller). Returns merged (global ids [B,k] int64, dists [B,k], counts [B]) on every rank."""
+        caller). Returns merged (global ids [B,k] int64, dists [B,k], counts [B]) on every rank.
+        search_size: the beam width of a Vamana shard (None = the index's); unused for a flat one."""
         import torch
         B = int(d_queries.shape[0])
         dev = d_queries.device
@@ -256,9 +281,7 @@ class ShardedSearcher:
                 par = pb.epoch % pb.NBUF
                 pg = pb._pg[par]
                 pg.per_shard_limit = per_shard
-                _capi.check(lib.sdb_search_batch_gather_device(self.index._h, B, d_queries.data_ptr(), k, search_size,
-                                                               l_ids.data_ptr(), l_d.data_ptr(), l_c.data_ptr(),
-                                                               C.byref(pg), stream))
+                self._search_shard(d_queries, k, search_size, l_ids, l_d, l_c, stream, pg)
                 _capi.check(lib.sdb_peer_barrier_device(di, self.world, self.rank, pb._flags, pb.epoch, stream))
                 g_i, g_dd, g_cc = pb.local(par)
                 _capi.check(lib.sdb_merge_topk_device(di, self.world, B, k, g_i, g_dd, g_cc, m_ids.data_ptr(),
@@ -281,9 +304,7 @@ class ShardedSearcher:
                 main.wait_event(self._bar_done[(e - 2) % pb.NBUF])
             pg = pb._pg[par]
             pg.per_shard_limit = per_shard
-            _capi.check(lib.sdb_search_batch_gather_device(self.index._h, B, d_queries.data_ptr(), k, search_size,
-                                                           l_ids.data_ptr(), l_d.data_ptr(), l_c.data_ptr(),
-                                                           C.byref(pg), main.cuda_stream))
+            self._search_shard(d_queries, k, search_size, l_ids, l_d, l_c, main.cuda_stream, pg)
             self._k1_done.record(main)
             side.wait_event(self._k1_done)
             o_ids, o_d, o_c = self._pipe_out[par]
@@ -294,7 +315,7 @@ class ShardedSearcher:
                                                   o_d.data_ptr(), o_c.data_ptr(), side.cuda_stream))
             self._pending = True
             return o_ids, o_d, o_c
-        self.index.search_batch_device(d_queries, k, search_size, l_ids, l_d, l_c, stream)
+        self._search_shard(d_queries, k, search_size, l_ids, l_d, l_c, stream)
         if per_shard < k:
             l_c.clamp_(max=per_shard)
         if self.world == 1:

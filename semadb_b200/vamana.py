@@ -374,6 +374,14 @@ class _DeviceIndex:
                                               _ptr(cnt, u32p)))
         return ids, d, cnt
 
+    def flat_search_batch_device(self, d_queries, k: int, d_out_ids, d_out_dists, d_out_counts, stream: int = 0):
+        """Flat twin of search_batch_device: torch tensors (contiguous) queries f32 [B,dim] on the
+        device or page-locked, out ids int64/uint64 [B,k], dists f32 [B,k], counts int32/uint32 [B].
+        Enqueues on `stream` (raw cudaStream_t) without synchronising; rows equal flat_search_batch."""
+        B = int(d_queries.shape[0])
+        check(self._lib.sdb_flat_search_batch_device(self._h, B, d_queries.data_ptr(), k, d_out_ids.data_ptr(),
+                                                     d_out_dists.data_ptr(), d_out_counts.data_ptr(), stream))
+
     def flat_search_batch_filters(self, queries, filters, query_filter=None, k: int = 10):
         """Flat search with one filter per request, shaped like search_batch_filters: `filters` is a
         list of id collections (an empty one filters everything out; ids that are not stored never
@@ -406,8 +414,9 @@ class _DeviceIndex:
         return g.value, s.value, p.value
 
     def flat_last_stats(self):
-        """(path, candidates, overflowed) of the last flat_search_batch: path 0 = exact CUDA-core
-        scan, 1 = mma.sync candidate pass, 2 = tcgen05 + TMA candidate pass."""
+        """(path, candidates, overflowed) of the last flat search: path 0 = exact CUDA-core
+        scan, 1 = mma.sync candidate pass, 2 = tcgen05 + TMA candidate pass. After a device-entry
+        call, waits for that call to complete."""
         import ctypes as C
         path, cand, ovf = C.c_int32(0), C.c_uint64(0), C.c_uint32(0)
         check(self._lib.sdb_flat_last_stats(self._h, C.byref(path), C.byref(cand), C.byref(ovf)))
