@@ -188,6 +188,10 @@ int sdb_flat_search_batch_filters(sdb_index* ix, uint32_t B, const float* querie
  * route scored (ids of deleted points included). All 0 after an unfiltered call. */
 int sdb_flat_last_filter_stats(sdb_index* ix, uint32_t* gathered_filters, uint32_t* scanned_filters,
                                uint64_t* gathered_pairs);
+/* Memory the handle keeps for staging filtered calls: page-locked host bytes (both staging slots and
+ * their gather work items) and device bytes (the device copy of a slot). Grow-only; a filter that
+ * takes the range scan stages only its ids, offsets and request rows. */
+int sdb_filter_staging_bytes(sdb_index* ix, uint64_t* pinned_bytes, uint64_t* device_bytes);
 
 /* Unfiltered flat search with device-resident queries and outputs (the flat twin of
  * sdb_search_batch_device): enqueues everything on `stream` (cudaStream_t) and returns without
@@ -340,6 +344,37 @@ int sdb_search_batch_gather_device(sdb_index* ix, uint32_t B, const float* d_que
 int sdb_flat_search_batch_gather_device(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k,
                                         uint64_t* d_out_ids, float* d_out_dists, uint32_t* d_out_counts,
                                         const sdb_peer_gather* peers, void* stream);
+/* Filtered shard search with device-resident queries and outputs, enqueued on `stream`.
+ * The filter arguments are those of sdb_search_batch_filters / sdb_flat_search_batch_filters, in
+ * host memory; they are copied before the call returns, so the caller may free or reuse them at
+ * once (cgo: Go memory is not retained). Filters are shard-local ids: each shard gets its own lists.
+ * A request filtered on one shard must be filtered on every shard (its list there may be empty);
+ * the library cannot check this across shards.
+ *   - Row b of the outputs equals row b of the matching host filter entry, byte for byte, on every
+ *     store each serves (beam search: f32 L2 / dot / cosine, haversine, binary, PQ; flat search:
+ *     the same stores, on both routes). n_filters == 0 gives the bytes of sdb_search_batch_device /
+ *     sdb_flat_search_batch_device (with peers: of the _gather_device entry).
+ *   - peers == NULL: no exchange. Otherwise every query's final list also goes into slot
+ *     [shard][query] of every peer's buffer, with the bytes the _gather_device entries store
+ *     (tagged ids, id 0 / +inf past the count, count clamped to per_shard_limit).
+ *   - Checks, in order: those of the host filter entry and their error codes (unsorted ids, a
+ *     query_filter index >= n_filters, missing seeds = SDB_ERR_NOTFOUND for the beam search,
+ *     searchSize < k, k outside 1..75 for flat search); then those of the _gather_device entry on
+ *     `peers`; then its SDB_ERR_STATE refusal after a timed-out barrier. A failed call enqueues
+ *     nothing.
+ *   - No host synchronisation: the filters go to the device through one of two page-locked
+ *     staging slots of the handle; the host waits only before refilling a slot whose copy (two
+ *     filtered calls ago) has not run yet. A filtered call on any stream waits, on the device, for
+ *     the previous filtered call on the handle to finish reading the lists it overwrites. The
+ *     first call of a larger shape allocates scratch, which synchronises the device. */
+int sdb_search_batch_filters_device(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, uint32_t search_size,
+                                    uint32_t n_filters, const uint64_t* filter_ids, const uint64_t* filter_offsets,
+                                    const int32_t* query_filter, uint64_t* d_out_ids, float* d_out_dists,
+                                    uint32_t* d_out_counts, const sdb_peer_gather* peers, void* stream);
+int sdb_flat_search_batch_filters_device(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k,
+                                         uint32_t n_filters, const uint64_t* filter_ids, const uint64_t* filter_offsets,
+                                         const int32_t* query_filter, uint64_t* d_out_ids, float* d_out_dists,
+                                         uint32_t* d_out_counts, const sdb_peer_gather* peers, void* stream);
 int sdb_peer_barrier_device(int32_t device, uint32_t n_peers, uint32_t me, uint32_t* const* peer_flags, uint32_t epoch,
                             void* stream);
 /* A peer that never arrives is given ~20 s; the barrier kernel then records the timeout in a

@@ -77,6 +77,9 @@ _SIGS = {
                                           C.c_void_p, C.c_void_p]),
     "sdb_search_batch_gather_device": (C.c_int, [H, C.c_uint32, C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p,
                                                  C.c_void_p, C.POINTER(SdbPeerGather), C.c_void_p]),
+    "sdb_search_batch_filters_device": (C.c_int, [H, C.c_uint32, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, u64p, u64p,
+                                                  i32p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(SdbPeerGather),
+                                                  C.c_void_p]),
     "sdb_peer_barrier_device": (C.c_int, [C.c_int32, C.c_uint32, C.c_uint32, C.POINTER(C.c_void_p), C.c_uint32,
                                           C.c_void_p]),
     "sdb_peer_barrier_check": (C.c_int, [C.c_int32, C.c_int32]),
@@ -90,10 +93,14 @@ _SIGS = {
                                                C.c_void_p]),
     "sdb_flat_search_batch_gather_device": (C.c_int, [H, C.c_uint32, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p,
                                                       C.c_void_p, C.POINTER(SdbPeerGather), C.c_void_p]),
+    "sdb_flat_search_batch_filters_device": (C.c_int, [H, C.c_uint32, C.c_void_p, C.c_uint32, C.c_uint32, u64p, u64p, i32p,
+                                                       C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(SdbPeerGather),
+                                                       C.c_void_p]),
     "sdb_flat_last_stats": (C.c_int, [H, i32p, u64p, u32p]),
     "sdb_flat_search_batch_filters": (C.c_int, [H, C.c_uint32, f32p, C.c_uint32, C.c_uint32, u64p, u64p, i32p, u64p, f32p,
                                                 u32p]),
     "sdb_flat_last_filter_stats": (C.c_int, [H, u32p, u32p, u64p]),
+    "sdb_filter_staging_bytes": (C.c_int, [H, u64p, u64p]),
     "sdb_insert_batch": (C.c_int, [H, C.c_uint64, u64p, f32p]),
     "sdb_insert_batch_device": (C.c_int, [H, C.c_uint64, u64p, C.c_void_p]),
     "sdb_insert_truncated": (C.c_uint64, [H]),

@@ -416,107 +416,127 @@ constexpr uint32_t FLAT_GATHER_CHUNK = 1024;  // ids per gather work item (one w
 
 namespace {
 
-// rows list[0..n) of the batch through `run` on a compacted copy of their queries, results
+// rows d_list[0..n) of the batch through `run` on a compacted copy of their queries, results
 // scattered back into the batch's outputs
 template <class Run>
-int run_subset(sdb_index* ix, const std::vector<uint32_t>& list, const float* d_queries, uint32_t k, uint64_t* d_out_ids,
+int run_subset(sdb_index* ix, const uint32_t* d_list, uint32_t n, const float* d_queries, uint32_t k, uint64_t* d_out_ids,
                float* d_out_dists, uint32_t* d_out_counts, cudaStream_t stream, Run run) {
-  const uint32_t n = uint32_t(list.size()), dim = ix->p.dim;
+  const uint32_t dim = ix->p.dim;
   int rc;
-  if ((rc = ix->d_fsub_list.ensure(n)) || (rc = ix->d_fsub_q.ensure(size_t(n) * dim)) || (rc = ix->d_fsub_ids.ensure(size_t(n) * k)) ||
+  if ((rc = ix->d_fsub_q.ensure(size_t(n) * dim)) || (rc = ix->d_fsub_ids.ensure(size_t(n) * k)) ||
       (rc = ix->d_fsub_d.ensure(size_t(n) * k)) || (rc = ix->d_fsub_cnt.ensure(n)))
     return rc;
-  SDB_CUDA(cudaMemcpyAsync(ix->d_fsub_list.p, list.data(), size_t(n) * 4, cudaMemcpyHostToDevice, stream));
-  gather_queries_kernel<<<n, 128, 0, stream>>>(ix->d_fsub_list.p, n, d_queries, dim, ix->d_fsub_q.p);
+  gather_queries_kernel<<<n, 128, 0, stream>>>(d_list, n, d_queries, dim, ix->d_fsub_q.p);
   ix->launches++;
   SDB_CUDA(cudaGetLastError());
   if ((rc = run(n, ix->d_fsub_q.p, ix->d_fsub_ids.p, ix->d_fsub_d.p, ix->d_fsub_cnt.p))) return rc;
-  scatter_results_kernel<<<n, 128, 0, stream>>>(ix->d_fsub_list.p, n, k, ix->d_fsub_ids.p, ix->d_fsub_d.p, ix->d_fsub_cnt.p,
+  scatter_results_kernel<<<n, 128, 0, stream>>>(d_list, n, k, ix->d_fsub_ids.p, ix->d_fsub_d.p, ix->d_fsub_cnt.p,
                                                 d_out_ids, d_out_dists, d_out_counts);
   ix->launches++;
   SDB_CUDA(cudaGetLastError());
-  // the next subset reuses the scratch: list is pageable host memory, consumed by the copy above
   return SDB_OK;
 }
 
 }  // namespace
 
-int launch_flat_filtered(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, uint32_t n_filters,
-                         const uint32_t* h_off, const int32_t* query_filter, const uint32_t* d_ids, uint64_t* d_out_ids,
-                         float* d_out_dists, uint32_t* d_out_counts, cudaStream_t stream) {
-  const uint32_t end_id = std::max<uint32_t>(2, ix->max_node_id + 1), npts = end_id - 2;
+int flat_plan(sdb_index* ix, uint32_t s, uint32_t B, uint32_t n_filters, const uint32_t* h_off, const int32_t* query_filter,
+              uint32_t npts, uint8_t* slot, size_t at, FlatFilterPlan* p) {
   auto filter_of = [&](uint32_t b) -> int32_t { return query_filter ? query_filter[b] : 0; };
   // requests per filter, grouped by filter (counting sort, batch order within a filter)
-  std::vector<uint32_t> first(size_t(n_filters) + 1, 0), by_filter, plain;
+  auto& first = p->first;
+  first.assign(size_t(n_filters) + 1, 0);
   for (uint32_t b = 0; b < B; ++b)
     if (filter_of(b) >= 0) first[filter_of(b) + 1]++;
   for (uint32_t f = 0; f < n_filters; ++f) first[f + 1] += first[f];
-  by_filter.resize(first[n_filters]);
-  {
-    std::vector<uint32_t> fill(first.begin(), first.end() - 1);
-    for (uint32_t b = 0; b < B; ++b) {
-      if (filter_of(b) >= 0) by_filter[fill[filter_of(b)]++] = b;
-      else plain.push_back(b);
-    }
-  }
   const bool scan_all = getenv("SDB_FLAT_EXACT") != nullptr;  // tests: every filter through the range scan
-  std::vector<uint8_t> gather(n_filters, 0);
-  ix->flat_last_gathered = ix->flat_last_scanned = 0;
-  ix->flat_last_pairs = 0;
+  p->gather.assign(n_filters, 0);
+  p->n_scanned = 0;
+  p->pairs = 0;
+  for (uint32_t f = 0; f < n_filters; ++f) {
+    const uint64_t nf = first[f + 1] - first[f], mf = h_off[f + 1] - h_off[f];
+    if (nf == 0) continue;
+    p->gather[f] = !scan_all && double(nf) * double(mf) < FLAT_GATHER_PAIRS_PER_POINT * double((nf + FQ - 1) / FQ) * npts;
+    if (p->gather[f]) p->pairs += nf * mf;
+    else p->n_scanned++;
+  }
+  // ---- gather route: work items (request, chunk of its filter's ids) in batch order
+  uint64_t n_items = 0;
+  uint32_t n_req = 0;
+  for (uint32_t b = 0; b < B; ++b) {
+    const int32_t f = filter_of(b);
+    if (f < 0 || !p->gather[f]) continue;
+    n_req++;
+    n_items += (h_off[f + 1] - h_off[f] + FLAT_GATHER_CHUNK - 1) / FLAT_GATHER_CHUNK;
+  }
+  if (n_items >= (uint64_t(1) << 32)) return fail(SDB_ERR_INVALID, "filters: too many ids in one batch");
+  p->n_items = uint32_t(n_items);
+  p->n_req = n_req;
+  p->req_at = at;
+  p->rows_at = p->req_at + align16((size_t(n_req) * 2 + 1) * 4);
+  p->items_at = p->rows_at + align16(size_t(B) * 4);
+  int rc;
+  if ((rc = ix->h_stage_items[s].ensure(n_items))) return rc;
+  uint4* items = ix->h_stage_items[s].p;
+  uint32_t* req = reinterpret_cast<uint32_t*>(slot + p->req_at);  // [n_req] batch rows, then [n_req + 1] first items
+  uint32_t* rows = reinterpret_cast<uint32_t*>(slot + p->rows_at);
+  uint32_t it = 0, r = 0, plain = first[n_filters];
+  for (uint32_t b = 0; b < B; ++b) {
+    const int32_t f = filter_of(b);
+    if (f < 0) { rows[plain++] = b; continue; }
+    rows[first[f]++] = b;  // first[f] becomes the end of f's requests: restored below
+    if (!p->gather[f]) continue;
+    req[r] = b;
+    req[n_req + r++] = it;
+    for (uint32_t s = h_off[f]; s < h_off[f + 1]; s += FLAT_GATHER_CHUNK)
+      items[it++] = make_uint4(b, s, std::min(h_off[f + 1], s + FLAT_GATHER_CHUNK), 0);
+  }
+  req[2 * n_req] = it;
+  for (uint32_t f = n_filters; f > 0; --f) first[f] = first[f - 1];
+  first[0] = 0;
+  p->n_plain = plain - first[n_filters];
+  return SDB_OK;
+}
+
+int launch_flat_filtered(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, const FilterStage& fs,
+                         uint64_t* d_out_ids, float* d_out_dists, uint32_t* d_out_counts, cudaStream_t stream) {
+  const uint32_t end_id = std::max<uint32_t>(2, ix->max_node_id + 1);
+  const FlatFilterPlan& p = fs.flat;
+  const uint32_t n_filters = uint32_t(p.gather.size());
+  const uint32_t* h_off = fs.h_off;
+  const uint32_t* d_ids = fs.sf.ids;
+  const uint8_t* d = ix->d_fstage.p;
+  const uint32_t* d_rows = reinterpret_cast<const uint32_t*>(d + p.rows_at);
+  ix->flat_last_scanned = p.n_scanned;
+  ix->flat_last_gathered = 0;
+  for (uint32_t f = 0; f < n_filters; ++f) ix->flat_last_gathered += p.gather[f];
+  ix->flat_last_pairs = p.pairs;
   ix->flat_last_path = 0;
   ix->flat_last_candidates = 0;
   ix->flat_last_overflow = 0;
   ix->flat_stats_pending = false;
-  for (uint32_t f = 0; f < n_filters; ++f) {
-    const uint64_t nf = first[f + 1] - first[f], mf = h_off[f + 1] - h_off[f];
-    if (nf == 0) continue;
-    gather[f] = !scan_all && double(nf) * double(mf) < FLAT_GATHER_PAIRS_PER_POINT * double((nf + FQ - 1) / FQ) * npts;
-    if (gather[f]) { ix->flat_last_gathered++; ix->flat_last_pairs += nf * mf; }
-    else ix->flat_last_scanned++;
-  }
   int rc;
-  // ---- gather route: work items (request, chunk of its filter's ids) in batch order
-  auto& items = ix->h_fg_items;
-  auto& req = ix->h_fg_req;  // [n_req] batch rows, then [n_req + 1] first item of each request
-  items.clear();
-  req.clear();
-  std::vector<uint32_t> req_items;
-  for (uint32_t b = 0; b < B; ++b) {
-    const int32_t f = filter_of(b);
-    if (f < 0 || !gather[f]) continue;
-    req.push_back(b);
-    req_items.push_back(uint32_t(items.size()));
-    for (uint32_t s = h_off[f]; s < h_off[f + 1]; s += FLAT_GATHER_CHUNK)
-      items.push_back(make_uint4(b, s, std::min(h_off[f + 1], s + FLAT_GATHER_CHUNK), 0));
-  }
-  const uint32_t n_req = uint32_t(req.size());
-  if (n_req) {
-    if (items.size() >= (size_t(1) << 32)) return fail(SDB_ERR_INVALID, "filters: too many ids in one batch");
-    req_items.push_back(uint32_t(items.size()));
-    req.insert(req.end(), req_items.begin(), req_items.end());
-    if ((rc = ix->d_fg_items.ensure(items.size() + 1)) || (rc = ix->d_fg_req.ensure(req.size()))) return rc;
-    SDB_CUDA(cudaMemcpyAsync(ix->d_fg_items.p, items.data(), items.size() * sizeof(uint4), cudaMemcpyHostToDevice, stream));
-    SDB_CUDA(cudaMemcpyAsync(ix->d_fg_req.p, req.data(), req.size() * 4, cudaMemcpyHostToDevice, stream));
-    if ((rc = launch_flat_gather(ix, B, d_queries, k, d_ids, uint32_t(items.size()), ix->d_fg_items.p, n_req, ix->d_fg_req.p,
-                                 ix->d_fg_req.p + n_req, d_out_ids, d_out_dists, d_out_counts, stream)))
+  // ---- gather route
+  if (p.n_req) {
+    const uint32_t* d_req = reinterpret_cast<const uint32_t*>(d + p.req_at);
+    if ((rc = launch_flat_gather(ix, B, d_queries, k, d_ids, p.n_items, reinterpret_cast<const uint4*>(d + p.items_at), p.n_req,
+                                 d_req, d_req + p.n_req, d_out_ids, d_out_dists, d_out_counts, stream)))
       return rc;
   }
   // ---- scan route: the range scan with the filter's bitmap over the filter's requests
   for (uint32_t f = 0; f < n_filters; ++f) {
-    if (first[f + 1] == first[f] || gather[f]) continue;
+    if (p.first[f + 1] == p.first[f] || p.gather[f]) continue;
     if ((rc = ix->d_filter_bits.ensure((size_t(ix->rows) + 31) / 32 + 1))) return rc;
     if ((rc = launch_filter_bits(ix, d_ids + h_off[f], h_off[f + 1] - h_off[f], ix->d_filter_bits.p, stream))) return rc;
-    const std::vector<uint32_t> list(by_filter.begin() + first[f], by_filter.begin() + first[f + 1]);
-    rc = run_subset(ix, list, d_queries, k, d_out_ids, d_out_dists, d_out_counts, stream,
-                    [&](uint32_t n, const float* q, uint64_t* oi, float* od, uint32_t* oc) {
+    rc = run_subset(ix, d_rows + p.first[f], p.first[f + 1] - p.first[f], d_queries, k, d_out_ids, d_out_dists, d_out_counts,
+                    stream, [&](uint32_t n, const float* q, uint64_t* oi, float* od, uint32_t* oc) {
                       return launch_flat_exact(ix, n, q, k, ix->d_filter_bits.p, oi, od, oc, stream, 2, end_id);
                     });
     if (rc) return rc;
   }
   // ---- unfiltered requests: the unfiltered pass (tensor-core form where eligible) over their subset
-  if (plain.size() == B) return launch_flat(ix, B, d_queries, k, nullptr, d_out_ids, d_out_dists, d_out_counts, stream);
-  if (!plain.empty())
-    return run_subset(ix, plain, d_queries, k, d_out_ids, d_out_dists, d_out_counts, stream,
+  if (p.n_plain == B) return launch_flat(ix, B, d_queries, k, nullptr, d_out_ids, d_out_dists, d_out_counts, stream);
+  if (p.n_plain)
+    return run_subset(ix, d_rows + p.first[n_filters], p.n_plain, d_queries, k, d_out_ids, d_out_dists, d_out_counts, stream,
                       [&](uint32_t n, const float* q, uint64_t* oi, float* od, uint32_t* oc) {
                         return launch_flat(ix, n, q, k, nullptr, oi, od, oc, stream);
                       });

@@ -233,6 +233,11 @@ int sdb_index_create(const sdb_params* params, sdb_index** out) {
     delete ix;
     return cuda_fail(e, "cudaStreamCreate");
   }
+  for (cudaEvent_t* ev : {&ix->fstage_ev[0], &ix->fstage_ev[1], &ix->filter_done_ev})
+    if ((e = cudaEventCreateWithFlags(ev, cudaEventDisableTiming)) != cudaSuccess) {
+      sdb_index_destroy(ix);
+      return cuda_fail(e, "cudaEventCreate");
+    }
   ix->vec_pitch = (p.dim + 3) / 4 * 4;
   ix->words = (p.dim + 63) / 64;
   ix->bits_pitch = (ix->words + 1) / 2 * 2;
@@ -284,11 +289,17 @@ void sdb_index_destroy(sdb_index* ix) {
   cudaFree(ix->d_pq_cdist);
   cudaFree(ix->d_ins_stats);
   ix->d_q.release(); ix->d_oid.release(); ix->d_od.release(); ix->d_oc.release(); ix->d_hops.release();
-  ix->d_ndist.release(); ix->d_work.release(); ix->d_adc.release(); ix->d_filter_ids.release(); ix->d_filter_off.release();
-  ix->d_filter_bits.release(); ix->d_qmap.release(); ix->d_query_filter.release(); ix->d_retry_bitmap.release(); ix->d_vis_ids.release(); ix->d_vis_len.release(); ix->d_vis_d.release();
-  ix->d_ids64.release(); ix->d_tmp32.release(); ix->d_tmpf.release(); ix->d_tmp8.release(); ix->h_stage.release();
+  ix->d_ndist.release(); ix->d_work.release(); ix->d_adc.release(); ix->d_fstage.release();
+  ix->d_filter_bits.release(); ix->d_retry_bitmap.release(); ix->d_vis_ids.release(); ix->d_vis_len.release(); ix->d_vis_d.release();
+  ix->d_ids64.release(); ix->d_tmp32.release(); ix->d_tmpf.release(); ix->d_tmp8.release();
+  ix->d_fg_part32.release(); ix->d_fsub_cnt.release(); ix->d_fg_partf.release(); ix->d_fsub_q.release(); ix->d_fsub_d.release();
+  ix->d_fsub_ids.release();
+  for (auto& h : ix->h_stage) h.release();
+  for (auto& h : ix->h_stage_items) h.release();
   ix->h_flat_misc.release();
   if (ix->flat_stats_ev) cudaEventDestroy(ix->flat_stats_ev);
+  for (cudaEvent_t e : {ix->fstage_ev[0], ix->fstage_ev[1], ix->filter_done_ev})
+    if (e) cudaEventDestroy(e);
   for (auto& e : ix->prof_ev)
     if (e) cudaEventDestroy(e);
   if (ix->stream) cudaStreamDestroy(ix->stream);
@@ -488,7 +499,11 @@ int sdb_index_delete(sdb_index* ix, uint64_t n, const uint64_t* ids) {
 
 // ---- search -------------------------------------------------------------------------
 
-static int check_search_args(sdb_index* ix, uint32_t k, uint32_t L) {
+}  // extern "C"
+
+namespace sdb {
+
+int check_search_args(sdb_index* ix, uint32_t k, uint32_t L) {
   if (k < 1 || k > 75) return fail(SDB_ERR_INVALID, "invalid limit for vector query, expected 1-75");  // models/search.go:291
   if (L > 75 || L < 1 || (!ix->p.relaxed && L < 25)) return fail(SDB_ERR_INVALID, "invalid searchSize for vector query, expected 25-75");
   if (L < k) return fail(SDB_ERR_SEARCHSIZE, "searchSize (" + std::to_string(L) + ") must be greater than k (" + std::to_string(k) + ")");
@@ -504,29 +519,47 @@ static int ensure_out_scratch(sdb_index* ix, uint32_t B, uint32_t k) {
   return SDB_OK;
 }
 
-// Host staging of a batch's filters (search.go:33-51,93-95; one roaring bitmap per request,
+// Staging of a batch's filters (search.go:33-51,93-95; one roaring bitmap per request,
 // shard/index/search.go:59-85) into the device form of SearchFilters: concatenated ascending u32
 // id lists + offsets, the per-query filter index, the batch positions of the filtered and of the
-// unfiltered requests, and — for a single shared filter — a dense bitmask over rows.
-// filter f = filter_ids[filter_offsets[f] .. filter_offsets[f+1]); query_filter[b] < 0 = request b
-// is not filtered (nullptr: every request uses filter 0). An EMPTY list is still a filter: the
-// reference then seeds nothing and returns no result (search.go:33-51 with an empty bitmap).
-// Ids below min_id are dropped like ids beyond the store (flat search: 2, the scan's first id);
-// h_off, if given, receives the staged offsets.
-static int stage_filters(sdb_index* ix, uint32_t B, uint32_t n_filters, const uint64_t* filter_ids,
-                         const uint64_t* filter_offsets, const int32_t* query_filter, uint32_t L, bool want_bits,
-                         SearchFilters* out, uint64_t min_id = 0, std::vector<uint32_t>* h_off = nullptr) {
+// unfiltered requests, and — for a single shared filter — a dense bitmask over rows, built on the
+// device. filter f = filter_ids[filter_offsets[f] .. filter_offsets[f+1]); query_filter[b] < 0 =
+// request b is not filtered (nullptr: every request uses filter 0). An EMPTY list is still a
+// filter: the reference then seeds nothing and returns no result (search.go:33-51 with an empty
+// bitmap). Flat search drops ids below 2 (the scan's first id) like ids beyond the store.
+// Everything goes into one page-locked slot (and, for the gather route's work items, its item
+// buffer), moved to the device by one copy each (commit_filters), so a filtered call enqueues its
+// staging without a host synchronisation.
+int stage_filters(sdb_index* ix, uint32_t B, uint32_t n_filters, const uint64_t* filter_ids, const uint64_t* filter_offsets,
+                  const int32_t* query_filter, uint32_t L, bool flat, FilterStage* out) {
   if (n_filters == 0 || !filter_offsets) return fail(SDB_ERR_INVALID, "filters: need at least one filter and its offsets");
-  std::vector<uint32_t> ids, off(size_t(n_filters) + 1, 0), qf_plain, qf_filtered;
-  std::vector<int32_t> qfil;
   for (uint32_t f = 0; f < n_filters; ++f)
     if (filter_offsets[f + 1] < filter_offsets[f]) return fail(SDB_ERR_INVALID, "filters: offsets must ascend");
-  if (filter_offsets[n_filters] - filter_offsets[0] >= (uint64_t(1) << 32)) return fail(SDB_ERR_INVALID, "filters: too many ids in one batch");
-  ids.reserve(size_t(filter_offsets[n_filters] - filter_offsets[0]));
+  const uint64_t n_raw = filter_offsets[n_filters] - filter_offsets[0];
+  if (n_raw >= (uint64_t(1) << 32)) return fail(SDB_ERR_INVALID, "filters: too many ids in one batch");
+  // slot layout: ids | offsets | query filter | qmap | flat: request rows and gather requests (all
+  // bounded by the id count and B; the gather work items are sized by flat_plan once routed)
+  FilterStage& fs = *out;
+  fs.ids_at = 0;
+  fs.off_at = align16(size_t(n_raw) * 4 + 4);
+  fs.qf_at = fs.off_at + align16((size_t(n_filters) + 1) * 4);
+  fs.qmap_at = fs.qf_at + (query_filter ? align16(size_t(B) * 4) : 0);
+  const size_t flat_at = fs.qmap_at + (query_filter ? align16(size_t(B) * 4 + 4) : 0);
+  const size_t bytes = flat_at + (flat ? flat_plan_bytes(B) : 0);
+  // the slot is refilled once the copy out of it two filtered calls ago has run
+  const uint32_t s = ix->fstage_next;
+  SDB_CUDA(cudaEventSynchronize(ix->fstage_ev[s]));
+  int rc;
+  if ((rc = ix->h_stage[s].ensure(bytes))) return rc;
+  uint8_t* h = ix->h_stage[s].p;
+  uint32_t* ids = reinterpret_cast<uint32_t*>(h + fs.ids_at);
+  uint32_t* off = reinterpret_cast<uint32_t*>(h + fs.off_at);
+  const uint64_t min_id = flat ? 2 : 0;
+  uint32_t n = 0;
   for (uint32_t f = 0; f < n_filters; ++f) {
     const uint64_t b0 = filter_offsets[f], b1 = filter_offsets[f + 1];
-    if (b1 < b0 || (b1 > b0 && !filter_ids)) return fail(SDB_ERR_INVALID, "filters: offsets must ascend");
-    off[f] = uint32_t(ids.size());
+    if (b1 > b0 && !filter_ids) return fail(SDB_ERR_INVALID, "filters: offsets must ascend");
+    off[f] = n;
     uint64_t prev = 0;
     for (uint64_t i = b0; i < b1; ++i) {
       const uint64_t id = filter_ids[i];
@@ -534,54 +567,80 @@ static int stage_filters(sdb_index* ix, uint32_t B, uint32_t n_filters, const ui
       prev = id;
       if (i - b0 < L && (id == 0 || id >= ix->rows || !ix->h_exists[id]))
         return fail(SDB_ERR_NOTFOUND, "failed to get filter points");  // GetMany of the seeds, search.go:45-48
-      if (id < ix->rows && id >= min_id) ids.push_back(uint32_t(id));  // ids beyond the store can never be expanded
+      if (id < ix->rows && id >= min_id) ids[n++] = uint32_t(id);  // ids beyond the store can never be expanded
     }
   }
-  off[n_filters] = uint32_t(ids.size());
-  if (ids.size() >= (size_t(1) << 32)) return fail(SDB_ERR_INVALID, "filters: too many ids in one batch");
+  off[n_filters] = n;
+  fs.n_ids = n;
+  fs.h_off = off;
+  fs.shared_bits = !flat && n_filters == 1 && !query_filter;
+  fs.per_request = query_filter != nullptr;
+  fs.is_flat = flat;
+  fs.sf = SearchFilters{};
+  fs.sf.n_filtered = B;
   if (query_filter) {
-    qfil.assign(query_filter, query_filter + B);
+    uint32_t n_filtered = 0;
     for (uint32_t b = 0; b < B; ++b) {
-      if (qfil[b] >= int32_t(n_filters)) return fail(SDB_ERR_INVALID, "filters: query_filter index out of range");
-      if (qfil[b] < 0) { qf_plain.push_back(b); qfil[b] = 0; }
-      else qf_filtered.push_back(b);
+      if (query_filter[b] >= int32_t(n_filters)) return fail(SDB_ERR_INVALID, "filters: query_filter index out of range");
+      n_filtered += query_filter[b] >= 0;
     }
+    int32_t* qf = reinterpret_cast<int32_t*>(h + fs.qf_at);
+    uint32_t* qmap = reinterpret_cast<uint32_t*>(h + fs.qmap_at);  // filtered positions, then unfiltered ones
+    uint32_t nf = 0, np = n_filtered;
+    for (uint32_t b = 0; b < B; ++b) {
+      qf[b] = query_filter[b] < 0 ? 0 : query_filter[b];
+      qmap[query_filter[b] < 0 ? np++ : nf++] = b;
+    }
+    fs.sf.n_filtered = n_filtered;
+    fs.sf.n_plain = B - n_filtered;
   }
-  int rc;
-  if ((rc = ix->d_filter_ids.ensure(ids.size() + 1))) return rc;
-  if ((rc = ix->d_filter_off.ensure(off.size()))) return rc;
-  SDB_CUDA(cudaMemcpyAsync(ix->d_filter_ids.p, ids.data(), ids.size() * 4, cudaMemcpyHostToDevice, ix->stream));
-  SDB_CUDA(cudaMemcpyAsync(ix->d_filter_off.p, off.data(), off.size() * 4, cudaMemcpyHostToDevice, ix->stream));
-  *out = SearchFilters{};
-  out->ids = ix->d_filter_ids.p;
-  out->off = ix->d_filter_off.p;
-  out->n_filtered = B;
-  std::vector<uint32_t> bits;
-  if (want_bits && n_filters == 1 && !query_filter) {
-    bits.assign((size_t(ix->rows) + 31) / 32, 0);
-    for (uint32_t id : ids) bits[id >> 5] |= 1u << (id & 31);
-    if ((rc = ix->d_filter_bits.ensure(bits.size() + 1))) return rc;
-    SDB_CUDA(cudaMemcpyAsync(ix->d_filter_bits.p, bits.data(), bits.size() * 4, cudaMemcpyHostToDevice, ix->stream));
-    out->bits = ix->d_filter_bits.p;
+  if (flat) {
+    const uint32_t npts = std::max<uint32_t>(2, ix->max_node_id + 1) - 2;
+    if ((rc = flat_plan(ix, s, B, n_filters, off, query_filter, npts, h, flat_at, &fs.flat))) return rc;
+    fs.bytes = fs.flat.items_at;
+  } else {
+    fs.bytes = flat_at;
   }
-  if (query_filter) {
-    if ((rc = ix->d_query_filter.ensure(B))) return rc;
-    if ((rc = ix->d_qmap.ensure(size_t(B) + 1))) return rc;
-    SDB_CUDA(cudaMemcpyAsync(ix->d_query_filter.p, qfil.data(), size_t(B) * 4, cudaMemcpyHostToDevice, ix->stream));
-    if (!qf_filtered.empty())
-      SDB_CUDA(cudaMemcpyAsync(ix->d_qmap.p, qf_filtered.data(), qf_filtered.size() * 4, cudaMemcpyHostToDevice, ix->stream));
-    if (!qf_plain.empty())
-      SDB_CUDA(cudaMemcpyAsync(ix->d_qmap.p + qf_filtered.size(), qf_plain.data(), qf_plain.size() * 4, cudaMemcpyHostToDevice, ix->stream));
-    out->query_filter = ix->d_query_filter.p;
-    out->qmap_filtered = ix->d_qmap.p;
-    out->n_filtered = uint32_t(qf_filtered.size());
-    out->qmap_plain = ix->d_qmap.p + qf_filtered.size();
-    out->n_plain = uint32_t(qf_plain.size());
-  }
-  SDB_CUDA(cudaStreamSynchronize(ix->stream));  // host vectors go out of scope
-  if (h_off) *h_off = std::move(off);
+  fs.slot = s;
   return SDB_OK;
 }
+
+int commit_filters(sdb_index* ix, FilterStage* fs, cudaStream_t stream) {
+  int rc;
+  // before the copy occupies the stream: the beam search's visited-table step-up reads an idle stream
+  if (!fs->is_flat && (rc = retry_check(ix))) return rc;
+  const size_t item_bytes = fs->is_flat ? size_t(fs->flat.n_items) * sizeof(uint4) : 0;
+  if ((rc = ix->d_fstage.ensure(fs->bytes + item_bytes))) return rc;
+  if (fs->shared_bits && (rc = ix->d_filter_bits.ensure((size_t(ix->rows) + 31) / 32 + 1))) return rc;
+  // the previous filtered call, on whichever stream, has read its lists, bitmap and scratch
+  SDB_CUDA(cudaStreamWaitEvent(stream, ix->filter_done_ev, 0));
+  SDB_CUDA(cudaMemcpyAsync(ix->d_fstage.p, ix->h_stage[fs->slot].p, fs->bytes, cudaMemcpyHostToDevice, stream));
+  if (item_bytes)
+    SDB_CUDA(cudaMemcpyAsync(ix->d_fstage.p + fs->flat.items_at, ix->h_stage_items[fs->slot].p, item_bytes, cudaMemcpyHostToDevice,
+                             stream));
+  SDB_CUDA(cudaEventRecord(ix->fstage_ev[fs->slot], stream));
+  ix->fstage_next = fs->slot ^ 1;
+  uint8_t* d = ix->d_fstage.p;
+  SearchFilters& sf = fs->sf;
+  sf.ids = reinterpret_cast<const uint32_t*>(d + fs->ids_at);
+  sf.off = reinterpret_cast<const uint32_t*>(d + fs->off_at);
+  if (fs->per_request) {
+    sf.query_filter = reinterpret_cast<const int32_t*>(d + fs->qf_at);
+    sf.qmap_filtered = reinterpret_cast<const uint32_t*>(d + fs->qmap_at);
+    sf.qmap_plain = sf.qmap_filtered + sf.n_filtered;
+  }
+  if (fs->shared_bits) {
+    if ((rc = launch_filter_bits(ix, sf.ids, fs->n_ids, ix->d_filter_bits.p, stream))) return rc;
+    sf.bits = ix->d_filter_bits.p;
+  }
+  return SDB_OK;
+}
+
+void filters_done(sdb_index* ix, cudaStream_t stream) { cudaEventRecord(ix->filter_done_ev, stream); }
+
+}  // namespace sdb
+
+extern "C" {
 
 static int search_batch_locked(sdb_index* ix, uint32_t B, const float* queries, uint32_t k, uint32_t search_size,
                                const SearchFilters* filters, uint64_t* out_ids, float* out_dists, uint32_t* out_counts) {
@@ -608,6 +667,7 @@ static int search_batch_locked(sdb_index* ix, uint32_t B, const float* queries, 
   if ((rc = ensure_out_scratch(ix, B, k))) return rc;
   rc = launch_search(ix, B, q_dev, k, search_size, oid_dev ? oid_dev : ix->d_oid.p, od_dev ? od_dev : ix->d_od.p,
                      oc_dev ? oc_dev : ix->d_oc.p, nullptr, nullptr, nullptr, 0, filters, ix->stream);
+  if (filters) filters_done(ix, ix->stream);
   if (rc) return rc;
   if (!oid_dev) SDB_CUDA(cudaMemcpyAsync(out_ids, ix->d_oid.p, size_t(B) * k * sizeof(uint64_t), cudaMemcpyDeviceToHost, ix->stream));
   if (!od_dev) SDB_CUDA(cudaMemcpyAsync(out_dists, ix->d_od.p, size_t(B) * k * sizeof(float), cudaMemcpyDeviceToHost, ix->stream));
@@ -628,13 +688,15 @@ int sdb_search_batch(sdb_index* ix, uint32_t B, const float* queries, uint32_t k
   if (rc) return rc;
   // filter_ids != NULL = filtered, even with n_filter == 0 (an empty bitmap filters everything out);
   // callers whose empty container has a NULL data pointer use sdb_search_batch_filters
-  SearchFilters sf;
+  FilterStage fs;
   const bool filtered = filter_ids != nullptr;
   if (filtered) {
     const uint64_t offs[2] = {0, n_filter};
-    if ((rc = stage_filters(ix, B, 1, filter_ids, offs, nullptr, search_size, true, &sf))) return rc;
+    if ((rc = stage_filters(ix, B, 1, filter_ids, offs, nullptr, search_size, false, &fs)) ||
+        (rc = commit_filters(ix, &fs, ix->stream)))
+      return rc;
   }
-  return search_batch_locked(ix, B, queries, k, search_size, filtered ? &sf : nullptr, out_ids, out_dists, out_counts);
+  return search_batch_locked(ix, B, queries, k, search_size, filtered ? &fs.sf : nullptr, out_ids, out_dists, out_counts);
 }
 
 int sdb_search_batch_filters(sdb_index* ix, uint32_t B, const float* queries, uint32_t k, uint32_t search_size,
@@ -648,9 +710,11 @@ int sdb_search_batch_filters(sdb_index* ix, uint32_t B, const float* queries, ui
   int rc = check_search_args(ix, k, search_size);
   if (rc) return rc;
   if (n_filters == 0) return search_batch_locked(ix, B, queries, k, search_size, nullptr, out_ids, out_dists, out_counts);
-  SearchFilters sf;
-  if ((rc = stage_filters(ix, B, n_filters, filter_ids, filter_offsets, query_filter, search_size, true, &sf))) return rc;
-  return search_batch_locked(ix, B, queries, k, search_size, &sf, out_ids, out_dists, out_counts);
+  FilterStage fs;
+  if ((rc = stage_filters(ix, B, n_filters, filter_ids, filter_offsets, query_filter, search_size, false, &fs)) ||
+      (rc = commit_filters(ix, &fs, ix->stream)))
+    return rc;
+  return search_batch_locked(ix, B, queries, k, search_size, &fs.sf, out_ids, out_dists, out_counts);
 }
 
 int sdb_search_batch_device(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, uint32_t search_size,
@@ -751,17 +815,16 @@ static int flat_batch_locked(sdb_index* ix, uint32_t B, const float* queries, ui
                              const uint64_t* filter_ids, const uint64_t* filter_offsets, const int32_t* query_filter,
                              uint64_t* out_ids, float* out_dists, uint32_t* out_counts) {
   int rc;
-  SearchFilters sf;
-  std::vector<uint32_t> h_off;
+  FilterStage fs;
   // flat search has no GetMany of seeds (L = 0): ids that are not stored are simply never matched
-  if (n_filters && (rc = stage_filters(ix, B, n_filters, filter_ids, filter_offsets, query_filter, 0, false, &sf, 2, &h_off)))
-    return rc;
+  if (n_filters && (rc = stage_filters(ix, B, n_filters, filter_ids, filter_offsets, query_filter, 0, true, &fs))) return rc;
   if ((rc = ix->d_q.ensure(size_t(B) * ix->p.dim))) return rc;
   if ((rc = ensure_out_scratch(ix, B, k))) return rc;
   SDB_CUDA(cudaMemcpyAsync(ix->d_q.p, queries, size_t(B) * ix->p.dim * sizeof(float), cudaMemcpyHostToDevice, ix->stream));
   if (n_filters) {
-    rc = launch_flat_filtered(ix, B, ix->d_q.p, k, n_filters, h_off.data(), query_filter, sf.ids, ix->d_oid.p, ix->d_od.p,
-                              ix->d_oc.p, ix->stream);
+    if ((rc = commit_filters(ix, &fs, ix->stream))) return rc;
+    rc = launch_flat_filtered(ix, B, ix->d_q.p, k, fs, ix->d_oid.p, ix->d_od.p, ix->d_oc.p, ix->stream);
+    filters_done(ix, ix->stream);
     if (rc) return rc;
   } else {
     rc = flat_device_locked(ix, B, ix->d_q.p, k, ix->d_oid.p, ix->d_od.p, ix->d_oc.p, ix->stream);
@@ -822,6 +885,16 @@ int sdb_flat_last_filter_stats(sdb_index* ix, uint32_t* gathered_filters, uint32
   if (gathered_filters) *gathered_filters = ix->flat_last_gathered;
   if (scanned_filters) *scanned_filters = ix->flat_last_scanned;
   if (gathered_pairs) *gathered_pairs = ix->flat_last_pairs;
+  return SDB_OK;
+}
+
+int sdb_filter_staging_bytes(sdb_index* ix, uint64_t* pinned_bytes, uint64_t* device_bytes) {
+  if (!ix) return fail(SDB_ERR_INVALID, "null index");
+  std::lock_guard<std::mutex> g(ix->mu);
+  uint64_t pinned = 0;
+  for (int s = 0; s < 2; ++s) pinned += ix->h_stage[s].n + ix->h_stage_items[s].n * sizeof(uint4);
+  if (pinned_bytes) *pinned_bytes = pinned;
+  if (device_bytes) *device_bytes = ix->d_fstage.n;
   return SDB_OK;
 }
 

@@ -126,15 +126,25 @@ struct sdb_index {
   sdb::DevBuf<uint32_t> d_retry_bitmap;  // RETRY launch: [retry_slots][rows/32] exact visited bitmaps
   uint32_t retry_slots = 1;
   sdb::DevBuf<float> d_adc;
-  sdb::DevBuf<uint32_t> d_filter_ids, d_filter_off, d_filter_bits, d_qmap;
-  sdb::DevBuf<int32_t> d_query_filter;
+  // Filtered calls (index.cu stage_filters): the host pass writes a batch's filters (and, for flat
+  // search, launch_flat_filtered's work lists) into one of two page-locked slots, and a copy moves
+  // the slot (and its gather work items) into d_fstage. fstage_ev[s] is recorded behind the copy out of slot s: the host waits
+  // on it only before refilling s. filter_done_ev is recorded behind the last kernel of a filtered
+  // call that reads d_fstage, d_filter_bits or the filtered-flat scratch; the next filtered call's
+  // stream waits on it before overwriting them, whichever stream either call runs on.
+  sdb::PinBuf<uint8_t> h_stage[2];
+  sdb::PinBuf<uint4> h_stage_items[2];  // flat search: the gather route's work items of slot s
+  cudaEvent_t fstage_ev[2] = {nullptr, nullptr};
+  uint32_t fstage_next = 0;
+  cudaEvent_t filter_done_ev = nullptr;
+  sdb::DevBuf<uint8_t> d_fstage;
+  sdb::DevBuf<uint32_t> d_filter_bits;
   sdb::DevBuf<uint32_t> d_vis_ids, d_vis_len;
   sdb::DevBuf<float> d_vis_d;
   sdb::DevBuf<uint64_t> d_ids64;
   sdb::DevBuf<uint32_t> d_tmp32;
   sdb::DevBuf<float> d_tmpf;
   sdb::DevBuf<uint8_t> d_tmp8;
-  sdb::PinBuf<uint8_t> h_stage;
   // tensor-core flat scan (flat_tc.cu): bf16 shadow of the store + per-call scratch
   uint64_t flat_last_candidates = 0;  // tensor-core flat scan: candidates kept by the last level, all queries
   uint32_t flat_last_overflow = 0;    // ... and queries that fell back to the exact scan
@@ -145,13 +155,10 @@ struct sdb_index {
   cudaEvent_t flat_stats_ev = nullptr;
   bool flat_stats_pending = false;
   // filtered flat search (flat.cu launch_flat_filtered, flat_filter.cu): routes of the last flat call
-  // (sdb_flat_last_filter_stats), host staging of the gather route's work, device scratch of both routes
+  // (sdb_flat_last_filter_stats), device scratch of both routes
   uint32_t flat_last_gathered = 0, flat_last_scanned = 0;  // filters that took each route
   uint64_t flat_last_pairs = 0;                             // (request, id) pairs the gather route scored
-  std::vector<uint4> h_fg_items;
-  std::vector<uint32_t> h_fg_req;
-  sdb::DevBuf<uint4> d_fg_items;
-  sdb::DevBuf<uint32_t> d_fg_req, d_fg_part32, d_fsub_list, d_fsub_cnt;
+  sdb::DevBuf<uint32_t> d_fg_part32, d_fsub_cnt;
   sdb::DevBuf<float> d_fg_partf, d_fsub_q, d_fsub_d;
   sdb::DevBuf<uint64_t> d_fsub_ids;
   uint64_t vec_epoch = 1, tc_epoch = 0;  // vec_epoch: bumped by every change to vec / exists
@@ -210,6 +217,9 @@ struct SearchFilters {
   const uint32_t* qmap_plain = nullptr;
   uint32_t n_plain = 0;
 };
+// the visited-table step-up of launch_search after a search that sent queries to the RETRY launch
+// (search.cu); reads the previous search's retry count only if its stream is idle
+int retry_check(sdb_index* ix);
 int launch_search(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, uint32_t L, uint64_t* d_out_ids,
                   float* d_out_dists, uint32_t* d_out_counts, uint32_t* d_vis_ids, float* d_vis_dists,
                   uint32_t* d_vis_len, uint32_t vis_cap, const SearchFilters* filters, cudaStream_t stream);
@@ -229,13 +239,59 @@ int flat_stats_settle(sdb_index* ix);
 // unfiltered flat search, device queries and outputs, enqueued on `stream` (index.cu)
 int flat_device_locked(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, uint64_t* d_out_ids, float* d_out_dists,
                        uint32_t* d_out_counts, cudaStream_t stream);
-// Flat search of a batch whose requests carry filters (staged as by the Vamana search: ascending
-// u32 ids in d_ids, filter f = [h_off[f], h_off[f+1]), ids 0 and 1 and ids >= rows dropped);
-// query_filter[b] < 0 = request b unfiltered, nullptr = every request uses filter 0. Routes each
-// filter to the gather kernel or to the range scan and the unfiltered requests to launch_flat.
-int launch_flat_filtered(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, uint32_t n_filters,
-                         const uint32_t* h_off, const int32_t* query_filter, const uint32_t* d_ids, uint64_t* d_out_ids,
-                         float* d_out_dists, uint32_t* d_out_counts, cudaStream_t stream);
+// byte offsets of the regions of a staging slot and of its device copy
+inline size_t align16(size_t x) { return (x + 15) & ~size_t(15); }
+// Work lists of launch_flat_filtered, planned on the host (flat_plan) into a filtered call's staging
+// slot: route of each filter, the batch rows grouped by filter (batch order within a filter)
+// followed by the unfiltered rows, and the gather route's requests and work items (x = batch row,
+// [y, z) = range of the staged ids). The work items go into the slot's own item buffer
+// (h_stage_items), sized once the routes are known: a filter on the range scan stages none.
+// *_at: byte offsets in the slot and in its device copy (items: in the device copy, after the
+// slot's bytes); first / gather stay on the host.
+struct FlatFilterPlan {
+  std::vector<uint32_t> first;  // [n_filters + 1] start of filter f's requests in the row list
+  std::vector<uint8_t> gather;  // [n_filters] 1 = gather route, 0 = range scan
+  uint32_t n_items = 0, n_req = 0, n_plain = 0, n_scanned = 0;
+  uint64_t pairs = 0;
+  size_t req_at = 0;    // u32 [n_req] batch rows, then [n_req + 1] first item of each request
+  size_t rows_at = 0;   // u32 [first[n_filters]] rows grouped by filter, then [n_plain] unfiltered rows
+  size_t items_at = 0;  // uint4 [n_items], device copy only: the end of the slot's bytes
+};
+// slot bytes flat_plan writes for a batch of B requests (its rows and requests; the items go apart)
+inline size_t flat_plan_bytes(uint32_t B) { return align16((size_t(B) * 2 + 1) * 4) + align16(size_t(B) * 4); }
+// plans launch_flat_filtered for the staged offsets h_off into slot + at and the work items into
+// ix->h_stage_items[s]; query_filter as the caller gave it
+int flat_plan(sdb_index* ix, uint32_t s, uint32_t B, uint32_t n_filters, const uint32_t* h_off, const int32_t* query_filter,
+              uint32_t npts, uint8_t* slot, size_t at, FlatFilterPlan* p);
+// A batch's filters, staged: `sf` points into the device copy once commit_filters has run; h_off is
+// the staged offsets in the host slot (valid until the call returns).
+struct FilterStage {
+  SearchFilters sf;
+  const uint32_t* h_off = nullptr;
+  uint32_t n_ids = 0, slot = 0;
+  size_t bytes = 0, ids_at = 0, off_at = 0, qf_at = 0, qmap_at = 0;  // bytes: of the slot (items excluded)
+  bool shared_bits = false;  // one filter shared by the batch: build its row bitmap on the device
+  bool per_request = false;  // query_filter given: per-query filter index and qmap staged
+  bool is_flat = false;
+  FlatFilterPlan flat;
+};
+// Host pass of a filtered call (index.cu): validates the filters (the error codes of the host filter
+// entries) and writes their device form into the next staging slot, nothing enqueued yet. flat: flat
+// search rules (no seeds, ids below 2 dropped, no shared bitmap) plus its work lists.
+int stage_filters(sdb_index* ix, uint32_t B, uint32_t n_filters, const uint64_t* filter_ids, const uint64_t* filter_offsets,
+                  const int32_t* query_filter, uint32_t L, bool flat, FilterStage* out);
+// enqueues a staged call's copy on `stream` behind the previous filtered call's readers, and the
+// shared filter's bitmap; fills out->sf
+int commit_filters(sdb_index* ix, FilterStage* fs, cudaStream_t stream);
+// after the last kernel of a filtered call that reads the filter buffers
+void filters_done(sdb_index* ix, cudaStream_t stream);
+// k / searchSize / start-node checks of the beam-search entries
+int check_search_args(sdb_index* ix, uint32_t k, uint32_t L);
+// Flat search of a batch whose requests carry filters, staged and committed by stage_filters /
+// commit_filters (flat rules). Routes each filter to the gather kernel or to the range scan and
+// the unfiltered requests to launch_flat.
+int launch_flat_filtered(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, const FilterStage& fs,
+                         uint64_t* d_out_ids, float* d_out_dists, uint32_t* d_out_counts, cudaStream_t stream);
 // flat_filter.cu: score each work item's ids (x = batch row, [y, z) = range of d_ids) and merge a
 // request's items (d_req_items[r] .. d_req_items[r+1]) into output row d_req_rows[r]
 int launch_flat_gather(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, const uint32_t* d_ids,

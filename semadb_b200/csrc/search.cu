@@ -38,10 +38,8 @@ static uint32_t geo_vt_slots(const sdb_index* ix) {
 
 static int dispatch_search(sdb_index* ix, const SearchArgs& a, bool filtered, cudaStream_t stream);
 
-int launch_search(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, uint32_t L, uint64_t* d_out_ids,
-                  float* d_out_dists, uint32_t* d_out_counts, uint32_t* d_vis_ids, float* d_vis_dists,
-                  uint32_t* d_vis_len, uint32_t vis_cap, const SearchFilters* filters, cudaStream_t stream) {
-  // Visited-table size for this launch: start at 5888 slots; if the previous search on this
+int retry_check(sdb_index* ix) {
+  // Visited-table size for the next launch: start at 5888 slots; if the previous search on this
   // handle sent more than 0.1 % of its queries to the RETRY launch (they visited more nodes than
   // 87.5 % of the table), step up. Read only when the stream is idle: never adds a sync.
   if (ix->retry_check_pending && cudaStreamQuery(ix->last_search_stream) == cudaSuccess) {
@@ -53,7 +51,14 @@ int launch_search(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k,
     if ((uint64_t(h_retry) * 1000 > ix->last_B || (h_retry > 0 && ix->last_B <= 2000)) && ix->vt_level < 2) ix->vt_level++;
     ix->retry_check_pending = false;
   }
+  return SDB_OK;
+}
+
+int launch_search(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, uint32_t L, uint64_t* d_out_ids,
+                  float* d_out_dists, uint32_t* d_out_counts, uint32_t* d_vis_ids, float* d_vis_dists,
+                  uint32_t* d_vis_len, uint32_t vis_cap, const SearchFilters* filters, cudaStream_t stream) {
   int rc;
+  if ((rc = retry_check(ix))) return rc;
   if ((rc = ix->d_hops.ensure(B))) return rc;
   if ((rc = ix->d_ndist.ensure(B))) return rc;
   if ((rc = ix->d_work.ensure(4 + size_t(B)))) return rc;
@@ -192,6 +197,15 @@ __global__ void flat_publish_kernel(PeerGather g, uint32_t B, uint32_t k, const 
   }
 }
 
+static int launch_flat_publish(sdb_index* ix, const PeerGather& g, uint32_t B, uint32_t k, const uint64_t* ids,
+                               const float* dists, const uint32_t* counts, cudaStream_t stream) {
+  const uint64_t n = uint64_t(B) * k;
+  flat_publish_kernel<<<uint32_t((n + 255) / 256), 256, 0, stream>>>(g, B, k, ids, dists, counts);
+  ix->launches++;
+  SDB_CUDA(cudaGetLastError());
+  return SDB_OK;
+}
+
 }  // namespace sdb
 
 using namespace sdb;
@@ -230,9 +244,60 @@ extern "C" int sdb_flat_search_batch_gather_device(sdb_index* ix, uint32_t B, co
   const cudaStream_t st = static_cast<cudaStream_t>(stream);
   int rc = flat_device_locked(ix, B, d_queries, k, d_out_ids, d_out_dists, d_out_counts, st);
   if (rc) return rc;
-  const uint64_t n = uint64_t(B) * k;
-  flat_publish_kernel<<<uint32_t((n + 255) / 256), 256, 0, st>>>(g, B, k, d_out_ids, d_out_dists, d_out_counts);
-  ix->launches++;
-  SDB_CUDA(cudaGetLastError());
-  return SDB_OK;
+  return launch_flat_publish(ix, g, B, k, d_out_ids, d_out_dists, d_out_counts, st);
+}
+
+extern "C" int sdb_search_batch_filters_device(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k,
+                                               uint32_t search_size, uint32_t n_filters, const uint64_t* filter_ids,
+                                               const uint64_t* filter_offsets, const int32_t* query_filter,
+                                               uint64_t* d_out_ids, float* d_out_dists, uint32_t* d_out_counts,
+                                               const sdb_peer_gather* peers, void* stream) {
+  if (!ix) return fail(SDB_ERR_INVALID, "null index");
+  if (B == 0) return SDB_OK;
+  if (!d_queries || !d_out_ids || !d_out_dists || !d_out_counts) return fail(SDB_ERR_INVALID, "null argument");
+  std::lock_guard<std::mutex> lk(ix->mu);
+  SDB_CUDA(cudaSetDevice(ix->device));
+  int rc = check_search_args(ix, k, search_size);
+  if (rc) return rc;
+  FilterStage fs;
+  if (n_filters && (rc = stage_filters(ix, B, n_filters, filter_ids, filter_offsets, query_filter, search_size, false, &fs)))
+    return rc;
+  PeerGather g;
+  if (peers && ((rc = peer_gather_args(peers, k, &g)) || (rc = peer_barrier_poisoned(ix->device)))) return rc;
+  const cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (n_filters && (rc = commit_filters(ix, &fs, st))) return rc;
+  ix->gather = peers ? &g : nullptr;  // the beam-search epilogue publishes every query's list
+  rc = launch_search(ix, B, d_queries, k, search_size, d_out_ids, d_out_dists, d_out_counts, nullptr, nullptr, nullptr, 0,
+                     n_filters ? &fs.sf : nullptr, st);
+  ix->gather = nullptr;
+  if (n_filters) filters_done(ix, st);
+  return rc;
+}
+
+extern "C" int sdb_flat_search_batch_filters_device(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k,
+                                                    uint32_t n_filters, const uint64_t* filter_ids,
+                                                    const uint64_t* filter_offsets, const int32_t* query_filter,
+                                                    uint64_t* d_out_ids, float* d_out_dists, uint32_t* d_out_counts,
+                                                    const sdb_peer_gather* peers, void* stream) {
+  if (!ix) return fail(SDB_ERR_INVALID, "null index");
+  if (B == 0) return SDB_OK;
+  if (!d_queries || !d_out_ids || !d_out_dists || !d_out_counts) return fail(SDB_ERR_INVALID, "null argument");
+  if (k < 1 || k > 75) return fail(SDB_ERR_INVALID, "invalid limit for vector query, expected 1-75");  // models/search.go:329
+  std::lock_guard<std::mutex> lk(ix->mu);
+  SDB_CUDA(cudaSetDevice(ix->device));
+  int rc;
+  FilterStage fs;
+  if (n_filters && (rc = stage_filters(ix, B, n_filters, filter_ids, filter_offsets, query_filter, 0, true, &fs))) return rc;
+  PeerGather g;
+  if (peers && ((rc = peer_gather_args(peers, k, &g)) || (rc = peer_barrier_poisoned(ix->device)))) return rc;
+  const cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (n_filters) {
+    if ((rc = commit_filters(ix, &fs, st))) return rc;
+    rc = launch_flat_filtered(ix, B, d_queries, k, fs, d_out_ids, d_out_dists, d_out_counts, st);
+    filters_done(ix, st);
+  } else {
+    rc = flat_device_locked(ix, B, d_queries, k, d_out_ids, d_out_dists, d_out_counts, st);
+  }
+  if (rc || !peers) return rc;
+  return launch_flat_publish(ix, g, B, k, d_out_ids, d_out_dists, d_out_counts, st);
 }

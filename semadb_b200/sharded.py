@@ -182,12 +182,19 @@ class ShardedSearcher:
                       torch.zeros((B, k), dtype=torch.float32, device=device),
                       torch.zeros((B,), dtype=torch.int32, device=device))
 
-    def _search_shard(self, q, k: int, search_size, l_ids, l_d, l_c, stream, pg=None):
+    def _search_shard(self, q, k: int, search_size, l_ids, l_d, l_c, stream, pg=None, filters=None, query_filter=None):
         """This rank's shard search of the [B, dim] query tensor q (device or page-locked) into l_*
         and, with pg, into slot [rank] of every peer's gather buffer: the flat entries for an
-        IndexFlat, the beam-search entries otherwise. Enqueued on `stream`, no synchronisation."""
+        IndexFlat, the beam-search entries otherwise, their filtered forms when `filters` is given.
+        Enqueued on `stream`, no synchronisation."""
         B = int(q.shape[0])
         L = None if self._flat else (self.index.L if search_size is None else int(search_size))
+        if filters is not None:
+            if self._flat:
+                self.index.flat_search_batch_filters_device(q, filters, query_filter, k, l_ids, l_d, l_c, stream, pg)
+            else:
+                self.index.search_batch_filters_device(q, filters, query_filter, k, L, l_ids, l_d, l_c, stream, pg)
+            return
         if pg is None:
             if self._flat:
                 self.index.flat_search_batch_device(q, k, l_ids, l_d, l_c, stream)
@@ -203,12 +210,13 @@ class ShardedSearcher:
         _capi.check(rc)
 
     def search_batch_pinned(self, h_queries, k: int, search_size: Optional[int], h_ids, h_dists, h_counts, device,
-                            max_search_limit: int = 75):
+                            max_search_limit: int = 75, filters=None, query_filter=None):
         """Host-facing twin of search_batch_device for page-locked (pinned) torch CPU tensors:
         pinned memory is mapped into the device address space, so K1 reads the broadcast query
         batch straight from host memory (no staging copy in front of the kernel); the merged
         lists come back with one small copy. Falls back to explicit copies when the fused
-        exchange is not active. Synchronises before returning."""
+        exchange is not active. Synchronises before returning. filters / query_filter: as in
+        search_batch_device."""
         import torch
         B = int(h_queries.shape[0])
         stream = torch.cuda.current_stream(device).cuda_stream
@@ -217,7 +225,7 @@ class ShardedSearcher:
             h_dists.is_pinned() and h_counts.is_pinned()
         if not fused:
             r_ids, r_d, r_c = self.search_batch_device(h_queries.to(device, non_blocking=True), k, search_size,
-                                                       max_search_limit)
+                                                       max_search_limit, filters, query_filter)
             h_ids.copy_(r_ids, non_blocking=True)
             h_dists.copy_(r_d, non_blocking=True)
             h_counts.copy_(r_c, non_blocking=True)
@@ -232,7 +240,7 @@ class ShardedSearcher:
         pg.per_shard_limit = shard_limit(k, self.world, max_search_limit)
         lib = _capi.lib()
         di = device.index or 0
-        self._search_shard(h_queries, k, search_size, l_ids, l_d, l_c, stream, pg)
+        self._search_shard(h_queries, k, search_size, l_ids, l_d, l_c, stream, pg, filters, query_filter)
         _capi.check(lib.sdb_peer_barrier_device(di, self.world, self.rank, pb._flags, pb.epoch, stream))
         g_i, g_dd, g_cc = pb.local(par)
         # The merge is a short kernel: its 300 k small stores would sit exposed on PCIe if they went
@@ -248,10 +256,28 @@ class ShardedSearcher:
         # the step is complete on this GPU: a barrier that gave up on a peer makes it an error
         _capi.check(lib.sdb_peer_barrier_check(di, 0))
 
-    def search_batch_device(self, d_queries, k: int, search_size: Optional[int], max_search_limit: int = 75):
+    def search_batch_device(self, d_queries, k: int, search_size: Optional[int], max_search_limit: int = 75,
+                            filters=None, query_filter=None):
         """d_queries: [B, dim] f32 CUDA tensor, identical on every rank (broadcast by the
         caller). Returns merged (global ids [B,k] int64, dists [B,k], counts [B]) on every rank.
-        search_size: the beam width of a Vamana shard (None = the index's); unused for a flat one."""
+        search_size: the beam width of a Vamana shard (None = the index's); unused for a flat one.
+
+        filters: this rank's shard-local id lists (as in IndexVamana.search_batch_filters: the
+        reference evaluates a request's filter on every shard against that shard's own points,
+        shard/index/search.go:59-85); query_filter[b]: the list request b uses on this rank, -1 for
+        none (None: every request uses filters[0]). A request filtered on one rank must be filtered
+        on every rank — its list there may be empty — or the merged list mixes filtered and
+        unfiltered shard results; the library cannot check this across ranks. The filters are
+        copied before the call returns. A vamana.PackedFilters (which carries its query_filter) may
+        stand for the lists.
+
+        A filter error is local to the rank whose lists it finds (unsorted ids, a query_filter index
+        out of range, a missing seed): that rank raises before it reaches the step's barrier, and with
+        the fused exchange its peers' barrier of that step times out (~20 s), after which their
+        exchange calls fail with SDB_ERR_STATE until sdb_peer_barrier_check(clear) (semadb_b200.h).
+        The epoch has advanced on every rank, so the ranks stay in step once cleared. Callers that
+        cannot rule such errors out check each rank's lists first (the host filter entries apply the
+        same checks)."""
         import torch
         B = int(d_queries.shape[0])
         dev = d_queries.device
@@ -281,7 +307,7 @@ class ShardedSearcher:
                 par = pb.epoch % pb.NBUF
                 pg = pb._pg[par]
                 pg.per_shard_limit = per_shard
-                self._search_shard(d_queries, k, search_size, l_ids, l_d, l_c, stream, pg)
+                self._search_shard(d_queries, k, search_size, l_ids, l_d, l_c, stream, pg, filters, query_filter)
                 _capi.check(lib.sdb_peer_barrier_device(di, self.world, self.rank, pb._flags, pb.epoch, stream))
                 g_i, g_dd, g_cc = pb.local(par)
                 _capi.check(lib.sdb_merge_topk_device(di, self.world, B, k, g_i, g_dd, g_cc, m_ids.data_ptr(),
@@ -304,7 +330,7 @@ class ShardedSearcher:
                 main.wait_event(self._bar_done[(e - 2) % pb.NBUF])
             pg = pb._pg[par]
             pg.per_shard_limit = per_shard
-            self._search_shard(d_queries, k, search_size, l_ids, l_d, l_c, main.cuda_stream, pg)
+            self._search_shard(d_queries, k, search_size, l_ids, l_d, l_c, main.cuda_stream, pg, filters, query_filter)
             self._k1_done.record(main)
             side.wait_event(self._k1_done)
             o_ids, o_d, o_c = self._pipe_out[par]
@@ -315,7 +341,7 @@ class ShardedSearcher:
                                                   o_d.data_ptr(), o_c.data_ptr(), side.cuda_stream))
             self._pending = True
             return o_ids, o_d, o_c
-        self._search_shard(d_queries, k, search_size, l_ids, l_d, l_c, stream)
+        self._search_shard(d_queries, k, search_size, l_ids, l_d, l_c, stream, None, filters, query_filter)
         if per_shard < k:
             l_c.clamp_(max=per_shard)
         if self.world == 1:

@@ -142,6 +142,41 @@ def _ptr(a, t):
     return None if a is None else a.ctypes.data_as(t)
 
 
+class PackedFilters:
+    """Per-request filters in the C form of sdb_search_batch_filters: `filters` is a list of id
+    collections (each sorted and de-duplicated here; an empty one filters everything out),
+    query_filter[b] the filter index of request b or -1 for none (None: every request uses
+    filters[0]). Every filtered entry takes either the lists or one of these; packing once serves
+    callers that search with the same large filters step after step."""
+
+    def __init__(self, filters, query_filter=None):
+        lists = [np.unique(_u64(f)) for f in filters]
+        off = np.zeros(len(lists) + 1, dtype=np.uint64)
+        off[1:] = np.cumsum([len(x) for x in lists])
+        self._set(np.concatenate(lists) if lists and off[-1] else np.zeros(0, dtype=np.uint64), off, query_filter)
+
+    @classmethod
+    def from_csr(cls, ids, offsets, query_filter=None):
+        """Already packed: filter f = ids[offsets[f]:offsets[f+1]], each strictly ascending (the
+        library checks)."""
+        self = cls.__new__(cls)
+        self._set(_u64(ids), _u64(offsets), query_filter)
+        return self
+
+    def _set(self, ids, off, query_filter):
+        self.n, self.ids, self.off = len(off) - 1, ids, off
+        self.qf = None if query_filter is None else np.ascontiguousarray(query_filter, dtype=np.int32)
+
+    @staticmethod
+    def of(filters, query_filter=None) -> "PackedFilters":
+        return filters if isinstance(filters, PackedFilters) else PackedFilters(filters, query_filter)
+
+    def args(self):
+        """(n_filters, filter_ids, filter_offsets, query_filter) as ctypes arguments."""
+        return (self.n, _ptr(self.ids, u64p) if len(self.ids) else None, _ptr(self.off, u64p),
+                None if self.qf is None else _ptr(self.qf, _capi.i32p))
+
+
 class _DeviceIndex:
     """Owns an sdb_index handle; shared by IndexVamana and IndexFlat."""
 
@@ -302,23 +337,17 @@ class _DeviceIndex:
     def search_batch_filters(self, queries, filters, query_filter=None, k: int = 10, search_size: Optional[int] = None):
         """One filter per request (shard/index/search.go:59-85): `filters` is a list of id
         collections (an empty one filters everything out), query_filter[b] the filter index of
-        request b or -1 for none (None: every request uses filters[0])."""
+        request b or -1 for none (None: every request uses filters[0]); or a PackedFilters."""
         q = _f32(queries)
         if q.ndim != 2 or q.shape[1] != self.dim:
             raise SdbError(_capi.ERR_INVALID, "queries must be [B, dim]")
         B = q.shape[0]
         L = self.L if search_size is None else int(search_size)
-        lists = [np.unique(_u64(f)) for f in filters]
-        off = np.zeros(len(lists) + 1, dtype=np.uint64)
-        off[1:] = np.cumsum([len(x) for x in lists])
-        flat = np.concatenate(lists) if lists and off[-1] else np.zeros(0, dtype=np.uint64)
-        qf = None if query_filter is None else np.ascontiguousarray(query_filter, dtype=np.int32)
+        f = PackedFilters.of(filters, query_filter)
         ids = np.zeros((B, k), dtype=np.uint64)
         d = np.zeros((B, k), dtype=np.float32)
         cnt = np.zeros(B, dtype=np.uint32)
-        check(self._lib.sdb_search_batch_filters(self._h, B, _ptr(q, f32p), k, L, len(lists),
-                                                 _ptr(flat, u64p) if len(flat) else None, _ptr(off, u64p),
-                                                 None if qf is None else _ptr(qf, _capi.i32p), _ptr(ids, u64p),
+        check(self._lib.sdb_search_batch_filters(self._h, B, _ptr(q, f32p), k, L, *f.args(), _ptr(ids, u64p),
                                                  _ptr(d, f32p), _ptr(cnt, u32p)))
         return ids, d, cnt
 
@@ -330,6 +359,18 @@ class _DeviceIndex:
         check(self._lib.sdb_search_batch_device(self._h, B, d_queries.data_ptr(), k, search_size,
                                                 d_out_ids.data_ptr(), d_out_dists.data_ptr(),
                                                 d_out_counts.data_ptr(), stream))
+
+    def search_batch_filters_device(self, d_queries, filters, query_filter, k: int, search_size: int, d_out_ids,
+                                    d_out_dists, d_out_counts, stream: int = 0, peers=None):
+        """Filtered twin of search_batch_device (sdb_search_batch_filters_device): `filters` and
+        query_filter as in search_batch_filters, host-side and copied before the call returns. peers
+        (an SdbPeerGather) also stores every final list into slot [shard][query] of every peer's
+        gather buffer. Enqueues on `stream` without synchronising; row b equals
+        search_batch_filters' row b."""
+        f = PackedFilters.of(filters, query_filter)
+        check(self._lib.sdb_search_batch_filters_device(
+            self._h, int(d_queries.shape[0]), d_queries.data_ptr(), k, search_size, *f.args(), d_out_ids.data_ptr(),
+            d_out_dists.data_ptr(), d_out_counts.data_ptr(), None if peers is None else C.byref(peers), stream))
 
     def last_search_stats(self, B: int):
         hops = np.zeros(B, dtype=np.uint32)
@@ -391,19 +432,25 @@ class _DeviceIndex:
         if q.ndim != 2 or q.shape[1] != self.dim:
             raise SdbError(_capi.ERR_INVALID, "queries must be [B, dim]")
         B = q.shape[0]
-        lists = [np.unique(_u64(f)) for f in filters]
-        off = np.zeros(len(lists) + 1, dtype=np.uint64)
-        off[1:] = np.cumsum([len(x) for x in lists])
-        flat = np.concatenate(lists) if lists and off[-1] else np.zeros(0, dtype=np.uint64)
-        qf = None if query_filter is None else np.ascontiguousarray(query_filter, dtype=np.int32)
+        f = PackedFilters.of(filters, query_filter)
         ids = np.zeros((B, k), dtype=np.uint64)
         d = np.zeros((B, k), dtype=np.float32)
         cnt = np.zeros(B, dtype=np.uint32)
-        check(self._lib.sdb_flat_search_batch_filters(self._h, B, _ptr(q, f32p), k, len(lists),
-                                                      _ptr(flat, u64p) if len(flat) else None, _ptr(off, u64p),
-                                                      None if qf is None else _ptr(qf, _capi.i32p), _ptr(ids, u64p),
+        check(self._lib.sdb_flat_search_batch_filters(self._h, B, _ptr(q, f32p), k, *f.args(), _ptr(ids, u64p),
                                                       _ptr(d, f32p), _ptr(cnt, u32p)))
         return ids, d, cnt
+
+    def flat_search_batch_filters_device(self, d_queries, filters, query_filter, k: int, d_out_ids, d_out_dists,
+                                         d_out_counts, stream: int = 0, peers=None):
+        """Filtered twin of flat_search_batch_device (sdb_flat_search_batch_filters_device): `filters`
+        and query_filter as in flat_search_batch_filters, host-side and copied before the call
+        returns. peers (an SdbPeerGather) also stores every final list into slot [shard][query] of
+        every peer's gather buffer. Enqueues on `stream` without synchronising; row b equals
+        flat_search_batch_filters' row b."""
+        f = PackedFilters.of(filters, query_filter)
+        check(self._lib.sdb_flat_search_batch_filters_device(
+            self._h, int(d_queries.shape[0]), d_queries.data_ptr(), k, *f.args(), d_out_ids.data_ptr(),
+            d_out_dists.data_ptr(), d_out_counts.data_ptr(), None if peers is None else C.byref(peers), stream))
 
     def flat_last_filter_stats(self):
         """(gathered_filters, scanned_filters, gathered_pairs) of the last flat search: filters that
@@ -412,6 +459,12 @@ class _DeviceIndex:
         g, s, p = C.c_uint32(0), C.c_uint32(0), C.c_uint64(0)
         check(self._lib.sdb_flat_last_filter_stats(self._h, C.byref(g), C.byref(s), C.byref(p)))
         return g.value, s.value, p.value
+
+    def filter_staging_bytes(self):
+        """(page-locked host bytes, device bytes) the handle keeps for staging filtered calls."""
+        pinned, device = C.c_uint64(0), C.c_uint64(0)
+        check(self._lib.sdb_filter_staging_bytes(self._h, C.byref(pinned), C.byref(device)))
+        return pinned.value, device.value
 
     def flat_last_stats(self):
         """(path, candidates, overflowed) of the last flat search: path 0 = exact CUDA-core
