@@ -375,6 +375,54 @@ int sdb_flat_search_batch_filters_device(sdb_index* ix, uint32_t B, const float*
                                          uint32_t n_filters, const uint64_t* filter_ids, const uint64_t* filter_offsets,
                                          const int32_t* query_filter, uint64_t* d_out_ids, float* d_out_dists,
                                          uint32_t* d_out_counts, const sdb_peer_gather* peers, void* stream);
+/* ---- per-request parameters: the reference gives every request its own Limit and SearchSize
+ * (models/search.go:268-314) as it gives every request its own filter. One batch serves any mix.
+ *   - Outputs are B x k_stride: row b holds out_counts[b] <= req[b].limit results, every other slot
+ *     is id 0 / +inf. Row b equals, byte for byte, the row the matching filter entry returns for
+ *     request b alone with k = req[b].limit, search_size = req[b].search_size and b's filter
+ *     (slots past the limit padded). A req array whose entries share one (limit, search_size), with
+ *     k_stride = limit, gives the bytes of the filter entry on the same batch.
+ *   - filter = index into the filters (sdb_search_batch_filters' filter_ids / filter_offsets), -1 =
+ *     unfiltered; n_filters may be 0 when no request is filtered.
+ *   - Checks, before anything is enqueued: every limit is 1..75, every search_size 25..75 (1..75 on a
+ *     `relaxed` index; ignored by flat search), limit > search_size = SDB_ERR_SEARCHSIZE, limit >
+ *     k_stride or k_stride > 75 = SDB_ERR_INVALID, then the checks of the filter entries. The seeds
+ *     of a filtered request are the first min(n_f, its search_size) ids of its filter, so requests
+ *     sharing a filter may have different seeds; the existence check of a filter's seeds covers the
+ *     largest search_size of the requests that use it (the batch's largest for a filter none uses).
+ *     A failed call enqueues nothing and leaves the outputs untouched.
+ *   - With peers, slot [shard][b] of every peer buffer (stride k_stride) gets request b's tagged ids,
+ *     count clamped to shard_limit (0 = limit); peers->per_shard_limit is ignored.
+ *   - Flat search runs the batch at k = k_stride and cuts every row to its limit: the exact top-k by
+ *     (distance, id) at a smaller k is a prefix of it.
+ *   - Staging: req travels with the filters through the handle's page-locked slots (an unfiltered
+ *     batch uses a slot too); the _device entries do no host synchronisation and copy req and the
+ *     filters before returning. */
+typedef struct sdb_request {
+  uint32_t limit;        /* k of this request, 1..75 */
+  uint32_t search_size;  /* L of this request (beam search; ignored by flat search) */
+  uint32_t shard_limit;  /* with peers: ranks published into the gather buffers, 0 = limit */
+  int32_t filter;        /* index into the filters, -1 = unfiltered (below -1: SDB_ERR_INVALID) */
+} sdb_request;
+int sdb_search_batch_requests(sdb_index* ix, uint32_t B, const float* queries, const sdb_request* req, uint32_t n_filters,
+                              const uint64_t* filter_ids, const uint64_t* filter_offsets, uint32_t k_stride,
+                              uint64_t* out_ids, float* out_dists, uint32_t* out_counts);
+int sdb_search_batch_requests_device(sdb_index* ix, uint32_t B, const float* d_queries, const sdb_request* req,
+                                     uint32_t n_filters, const uint64_t* filter_ids, const uint64_t* filter_offsets,
+                                     uint32_t k_stride, uint64_t* d_out_ids, float* d_out_dists, uint32_t* d_out_counts,
+                                     const sdb_peer_gather* peers, void* stream);
+int sdb_flat_search_batch_requests(sdb_index* ix, uint32_t B, const float* queries, const sdb_request* req,
+                                   uint32_t n_filters, const uint64_t* filter_ids, const uint64_t* filter_offsets,
+                                   uint32_t k_stride, uint64_t* out_ids, float* out_dists, uint32_t* out_counts);
+int sdb_flat_search_batch_requests_device(sdb_index* ix, uint32_t B, const float* d_queries, const sdb_request* req,
+                                          uint32_t n_filters, const uint64_t* filter_ids, const uint64_t* filter_offsets,
+                                          uint32_t k_stride, uint64_t* d_out_ids, float* d_out_dists,
+                                          uint32_t* d_out_counts, const sdb_peer_gather* peers, void* stream);
+/* sdb_merge_topk_device with one output limit per request: d_limits[b] (device, 1..k_stride) bounds
+ * row b's merged list; inputs S x B x k_stride, outputs B x k_stride padded with id 0 / +inf. */
+int sdb_merge_topk_requests_device(int32_t device, uint32_t S, uint32_t B, uint32_t k_stride, const uint32_t* d_limits,
+                                   const uint64_t* d_in_ids, const float* d_in_dists, const uint32_t* d_in_counts,
+                                   uint64_t* d_out_ids, float* d_out_dists, uint32_t* d_out_counts, void* stream);
 int sdb_peer_barrier_device(int32_t device, uint32_t n_peers, uint32_t me, uint32_t* const* peer_flags, uint32_t epoch,
                             void* stream);
 /* A peer that never arrives is given ~20 s; the barrier kernel then records the timeout in a

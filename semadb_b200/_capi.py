@@ -47,6 +47,11 @@ class SdbPeerGather(C.Structure):
     ]
 
 
+class SdbRequest(C.Structure):
+    """sdb_request (include/semadb_b200.h): one request's limit, searchSize, shard limit and filter."""
+    _fields_ = [("limit", C.c_uint32), ("search_size", C.c_uint32), ("shard_limit", C.c_uint32), ("filter", C.c_int32)]
+
+
 f32p = C.POINTER(C.c_float)
 u64p = C.POINTER(C.c_uint64)
 u32p = C.POINTER(C.c_uint32)
@@ -80,6 +85,19 @@ _SIGS = {
     "sdb_search_batch_filters_device": (C.c_int, [H, C.c_uint32, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, u64p, u64p,
                                                   i32p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(SdbPeerGather),
                                                   C.c_void_p]),
+    "sdb_search_batch_requests": (C.c_int, [H, C.c_uint32, f32p, C.POINTER(SdbRequest), C.c_uint32, u64p, u64p,
+                                            C.c_uint32, u64p, f32p, u32p]),
+    "sdb_search_batch_requests_device": (C.c_int, [H, C.c_uint32, C.c_void_p, C.POINTER(SdbRequest), C.c_uint32, u64p,
+                                                   u64p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                   C.POINTER(SdbPeerGather), C.c_void_p]),
+    "sdb_flat_search_batch_requests": (C.c_int, [H, C.c_uint32, f32p, C.POINTER(SdbRequest), C.c_uint32, u64p, u64p,
+                                                 C.c_uint32, u64p, f32p, u32p]),
+    "sdb_flat_search_batch_requests_device": (C.c_int, [H, C.c_uint32, C.c_void_p, C.POINTER(SdbRequest), C.c_uint32,
+                                                        u64p, u64p, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                        C.POINTER(SdbPeerGather), C.c_void_p]),
+    "sdb_merge_topk_requests_device": (C.c_int, [C.c_int32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p,
+                                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                 C.c_void_p]),
     "sdb_peer_barrier_device": (C.c_int, [C.c_int32, C.c_uint32, C.c_uint32, C.POINTER(C.c_void_p), C.c_uint32,
                                           C.c_void_p]),
     "sdb_peer_barrier_check": (C.c_int, [C.c_int32, C.c_int32]),

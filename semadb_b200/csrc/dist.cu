@@ -133,14 +133,17 @@ __global__ void point_dists_sdc_kernel(const uint8_t* codes, uint32_t pitch, con
 }
 
 // K6: one thread per query merges S sorted lists; stable by (dist asc, shard asc, rank asc).
+// k is the row stride of inputs and outputs; row b keeps limits[b] results (nullptr: k).
 __global__ void merge_topk_kernel(uint32_t S, uint32_t B, uint32_t k, const uint64_t* in_ids, const float* in_d,
-                                  const uint32_t* in_c, uint64_t* out_ids, float* out_d, uint32_t* out_c) {
+                                  const uint32_t* in_c, uint64_t* out_ids, float* out_d, uint32_t* out_c,
+                                  const uint32_t* limits) {
   uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
   uint32_t heads[64];  // S <= 64 (checked by launch_merge)
   for (uint32_t s = 0; s < S; ++s) heads[s] = 0;
+  const uint32_t lim = limits ? min(limits[b], k) : k;
   uint32_t n = 0;
-  for (; n < k; ++n) {
+  for (; n < lim; ++n) {
     int best = -1;
     float bd = 0.0f;
     for (uint32_t s = 0; s < S; ++s) {
@@ -295,9 +298,9 @@ int launch_adc_tables(sdb_index* ix, uint32_t B, const float* d_queries, float* 
 }
 
 int launch_merge(uint32_t S, uint32_t B, uint32_t k, const uint64_t* in_ids, const float* in_d, const uint32_t* in_c,
-                 uint64_t* out_ids, float* out_d, uint32_t* out_c, cudaStream_t stream) {
+                 uint64_t* out_ids, float* out_d, uint32_t* out_c, cudaStream_t stream, const uint32_t* limits) {
   if (S == 0 || S > 64) return fail(SDB_ERR_INVALID, "merge supports 1..64 shards");
-  merge_topk_kernel<<<(B + 127) / 128, 128, 0, stream>>>(S, B, k, in_ids, in_d, in_c, out_ids, out_d, out_c);
+  merge_topk_kernel<<<(B + 127) / 128, 128, 0, stream>>>(S, B, k, in_ids, in_d, in_c, out_ids, out_d, out_c, limits);
   SDB_CUDA(cudaGetLastError());
   return SDB_OK;
 }
@@ -523,6 +526,20 @@ int sdb_merge_topk_device(int32_t device, uint32_t S, uint32_t B, uint32_t k, co
   if (rc) return rc;
   if ((rc = peer_barrier_poisoned(device))) return rc;  // an earlier cross-GPU barrier on this device timed out
   return launch_merge(S, B, k, d_in_ids, d_in_dists, d_in_counts, d_out_ids, d_out_dists, d_out_counts, static_cast<cudaStream_t>(stream));
+}
+
+int sdb_merge_topk_requests_device(int32_t device, uint32_t S, uint32_t B, uint32_t k_stride, const uint32_t* d_limits,
+                                   const uint64_t* d_in_ids, const float* d_in_dists, const uint32_t* d_in_counts,
+                                   uint64_t* d_out_ids, float* d_out_dists, uint32_t* d_out_counts, void* stream) {
+  if (B == 0) return SDB_OK;
+  if (!d_limits || !d_in_ids || !d_in_dists || !d_in_counts || !d_out_ids || !d_out_dists || !d_out_counts)
+    return fail(SDB_ERR_INVALID, "null argument");
+  if (k_stride < 1 || k_stride > 75) return fail(SDB_ERR_INVALID, "invalid limit");
+  int rc = set_device_checked(device);
+  if (rc) return rc;
+  if ((rc = peer_barrier_poisoned(device))) return rc;
+  return launch_merge(S, B, k_stride, d_in_ids, d_in_dists, d_in_counts, d_out_ids, d_out_dists, d_out_counts,
+                      static_cast<cudaStream_t>(stream), d_limits);
 }
 
 int sdb_merge_topk(int32_t device, uint32_t S, uint32_t B, uint32_t k, const uint64_t* in_ids, const float* in_dists,

@@ -511,6 +511,25 @@ int check_search_args(sdb_index* ix, uint32_t k, uint32_t L) {
   return SDB_OK;
 }
 
+int check_requests(sdb_index* ix, uint32_t B, const sdb_request* req, uint32_t n_filters, uint32_t k_stride, bool flat) {
+  if (!req) return fail(SDB_ERR_INVALID, "null argument");
+  for (uint32_t b = 0; b < B; ++b) {
+    const sdb_request& r = req[b];
+    if (r.limit < 1 || r.limit > 75) return fail(SDB_ERR_INVALID, "invalid limit for vector query, expected 1-75");  // models/search.go:291
+    if (!flat) {
+      const uint32_t L = r.search_size;
+      if (L > 75 || L < 1 || (!ix->p.relaxed && L < 25)) return fail(SDB_ERR_INVALID, "invalid searchSize for vector query, expected 25-75");
+      if (L < r.limit)
+        return fail(SDB_ERR_SEARCHSIZE, "searchSize (" + std::to_string(L) + ") must be greater than k (" + std::to_string(r.limit) + ")");
+    }
+    if (r.limit > k_stride || k_stride > 75) return fail(SDB_ERR_INVALID, "requests: k_stride must be 1..75 and at least every limit");
+    if (r.filter < -1 || (r.filter >= 0 && uint32_t(r.filter) >= n_filters))
+      return fail(SDB_ERR_INVALID, "requests: filter must be -1 or a filter index");
+  }
+  if (!flat && (ix->rows <= START_ID || !ix->h_exists[START_ID])) return fail(SDB_ERR_STATE, "failed to get start point");
+  return SDB_OK;
+}
+
 static int ensure_out_scratch(sdb_index* ix, uint32_t B, uint32_t k) {
   int rc;
   if ((rc = ix->d_oid.ensure(size_t(B) * k))) return rc;
@@ -529,13 +548,31 @@ static int ensure_out_scratch(sdb_index* ix, uint32_t B, uint32_t k) {
 // bitmap). Flat search drops ids below 2 (the scan's first id) like ids beyond the store.
 // Everything goes into one page-locked slot (and, for the gather route's work items, its item
 // buffer), moved to the device by one copy each (commit_filters), so a filtered call enqueues its
-// staging without a host synchronisation.
+// staging without a host synchronisation. A request batch (req) also stages every request's
+// parameters, and takes a slot even when nobody is filtered.
 int stage_filters(sdb_index* ix, uint32_t B, uint32_t n_filters, const uint64_t* filter_ids, const uint64_t* filter_offsets,
-                  const int32_t* query_filter, uint32_t L, bool flat, FilterStage* out) {
-  if (n_filters == 0 || !filter_offsets) return fail(SDB_ERR_INVALID, "filters: need at least one filter and its offsets");
+                  const int32_t* query_filter, uint32_t L, bool flat, FilterStage* out, const sdb_request* req) {
+  if ((!req && n_filters == 0) || (n_filters && !filter_offsets))
+    return fail(SDB_ERR_INVALID, "filters: need at least one filter and its offsets");
   for (uint32_t f = 0; f < n_filters; ++f)
     if (filter_offsets[f + 1] < filter_offsets[f]) return fail(SDB_ERR_INVALID, "filters: offsets must ascend");
-  const uint64_t n_raw = filter_offsets[n_filters] - filter_offsets[0];
+  const uint64_t n_raw = n_filters ? filter_offsets[n_filters] - filter_offsets[0] : 0;
+  // request batch: per-request filter index, and per filter the seeds its requests read (the largest
+  // search_size among them; the batch's largest for a filter no request uses)
+  std::vector<int32_t> req_qf;
+  std::vector<uint32_t> seed_L;
+  if (req) {
+    req_qf.resize(B);
+    seed_L.assign(n_filters, 0);
+    uint32_t L_max = 0;
+    for (uint32_t b = 0; b < B; ++b) {
+      req_qf[b] = req[b].filter < 0 ? -1 : req[b].filter;
+      L_max = std::max(L_max, req[b].search_size);
+      if (req[b].filter >= 0) seed_L[req[b].filter] = std::max(seed_L[req[b].filter], req[b].search_size);
+    }
+    for (uint32_t& x : seed_L) x = flat ? 0 : (x ? x : L_max);
+    query_filter = req_qf.data();
+  }
   if (n_raw >= (uint64_t(1) << 32)) return fail(SDB_ERR_INVALID, "filters: too many ids in one batch");
   // slot layout: ids | offsets | query filter | qmap | flat: request rows and gather requests (all
   // bounded by the id count and B; the gather work items are sized by flat_plan once routed)
@@ -544,8 +581,9 @@ int stage_filters(sdb_index* ix, uint32_t B, uint32_t n_filters, const uint64_t*
   fs.off_at = align16(size_t(n_raw) * 4 + 4);
   fs.qf_at = fs.off_at + align16((size_t(n_filters) + 1) * 4);
   fs.qmap_at = fs.qf_at + (query_filter ? align16(size_t(B) * 4) : 0);
-  const size_t flat_at = fs.qmap_at + (query_filter ? align16(size_t(B) * 4 + 4) : 0);
-  const size_t bytes = flat_at + (flat ? flat_plan_bytes(B) : 0);
+  fs.req_at = fs.qmap_at + (query_filter ? align16(size_t(B) * 4 + 4) : 0);
+  const size_t flat_at = fs.req_at + (req ? align16(size_t(B) * sizeof(uint4)) : 0);
+  const size_t bytes = flat_at + (flat && n_filters ? flat_plan_bytes(B) : 0);
   // the slot is refilled once the copy out of it two filtered calls ago has run
   const uint32_t s = ix->fstage_next;
   SDB_CUDA(cudaEventSynchronize(ix->fstage_ev[s]));
@@ -560,12 +598,13 @@ int stage_filters(sdb_index* ix, uint32_t B, uint32_t n_filters, const uint64_t*
     const uint64_t b0 = filter_offsets[f], b1 = filter_offsets[f + 1];
     if (b1 > b0 && !filter_ids) return fail(SDB_ERR_INVALID, "filters: offsets must ascend");
     off[f] = n;
+    const uint64_t seeds = req ? seed_L[f] : L;
     uint64_t prev = 0;
     for (uint64_t i = b0; i < b1; ++i) {
       const uint64_t id = filter_ids[i];
       if (i > b0 && id <= prev) return fail(SDB_ERR_INVALID, "filter ids must be strictly ascending");
       prev = id;
-      if (i - b0 < L && (id == 0 || id >= ix->rows || !ix->h_exists[id]))
+      if (i - b0 < seeds && (id == 0 || id >= ix->rows || !ix->h_exists[id]))
         return fail(SDB_ERR_NOTFOUND, "failed to get filter points");  // GetMany of the seeds, search.go:45-48
       if (id < ix->rows && id >= min_id) ids[n++] = uint32_t(id);  // ids beyond the store can never be expanded
     }
@@ -573,8 +612,11 @@ int stage_filters(sdb_index* ix, uint32_t B, uint32_t n_filters, const uint64_t*
   off[n_filters] = n;
   fs.n_ids = n;
   fs.h_off = off;
-  fs.shared_bits = !flat && n_filters == 1 && !query_filter;
+  // one filter shared by every request: the dense bitmap (a request batch: every request uses filter 0)
+  const bool all_first = req && std::all_of(req, req + B, [](const sdb_request& r) { return r.filter == 0; });
+  fs.shared_bits = !flat && n_filters == 1 && (!query_filter || all_first);
   fs.per_request = query_filter != nullptr;
+  fs.has_req = req != nullptr;
   fs.is_flat = flat;
   fs.sf = SearchFilters{};
   fs.sf.n_filtered = B;
@@ -594,7 +636,16 @@ int stage_filters(sdb_index* ix, uint32_t B, uint32_t n_filters, const uint64_t*
     fs.sf.n_filtered = n_filtered;
     fs.sf.n_plain = B - n_filtered;
   }
-  if (flat) {
+  if (req) {
+    uint4* rq = reinterpret_cast<uint4*>(h + fs.req_at);
+    for (uint32_t b = 0; b < B; ++b) {
+      const sdb_request& r = req[b];
+      const uint32_t plim = r.shard_limit == 0 || r.shard_limit > r.limit ? r.limit : r.shard_limit;
+      rq[b] = make_uint4(r.search_size, r.limit, plim, 0);
+    }
+  }
+  fs.flat = FlatFilterPlan{};
+  if (flat && n_filters) {
     const uint32_t npts = std::max<uint32_t>(2, ix->max_node_id + 1) - 2;
     if ((rc = flat_plan(ix, s, B, n_filters, off, query_filter, npts, h, flat_at, &fs.flat))) return rc;
     fs.bytes = fs.flat.items_at;
@@ -629,6 +680,7 @@ int commit_filters(sdb_index* ix, FilterStage* fs, cudaStream_t stream) {
     sf.qmap_filtered = reinterpret_cast<const uint32_t*>(d + fs->qmap_at);
     sf.qmap_plain = sf.qmap_filtered + sf.n_filtered;
   }
+  if (fs->has_req) sf.req = reinterpret_cast<const uint4*>(d + fs->req_at);
   if (fs->shared_bits) {
     if ((rc = launch_filter_bits(ix, sf.ids, fs->n_ids, ix->d_filter_bits.p, stream))) return rc;
     sf.bits = ix->d_filter_bits.p;
@@ -715,6 +767,23 @@ int sdb_search_batch_filters(sdb_index* ix, uint32_t B, const float* queries, ui
       (rc = commit_filters(ix, &fs, ix->stream)))
     return rc;
   return search_batch_locked(ix, B, queries, k, search_size, &fs.sf, out_ids, out_dists, out_counts);
+}
+
+int sdb_search_batch_requests(sdb_index* ix, uint32_t B, const float* queries, const sdb_request* req, uint32_t n_filters,
+                              const uint64_t* filter_ids, const uint64_t* filter_offsets, uint32_t k_stride,
+                              uint64_t* out_ids, float* out_dists, uint32_t* out_counts) {
+  if (!ix) return fail(SDB_ERR_INVALID, "null index");
+  if (B == 0) return SDB_OK;
+  if (!queries || !out_ids || !out_dists || !out_counts) return fail(SDB_ERR_INVALID, "null argument");
+  std::lock_guard<std::mutex> g(ix->mu);
+  SDB_CUDA(cudaSetDevice(ix->device));
+  int rc = check_requests(ix, B, req, n_filters, k_stride, false);
+  if (rc) return rc;
+  FilterStage fs;
+  if ((rc = stage_filters(ix, B, n_filters, filter_ids, filter_offsets, nullptr, 0, false, &fs, req)) ||
+      (rc = commit_filters(ix, &fs, ix->stream)))
+    return rc;
+  return search_batch_locked(ix, B, queries, k_stride, 75, &fs.sf, out_ids, out_dists, out_counts);
 }
 
 int sdb_search_batch_device(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, uint32_t search_size,
@@ -866,6 +935,33 @@ int sdb_flat_search_batch_filters(sdb_index* ix, uint32_t B, const float* querie
   SDB_CUDA(cudaSetDevice(ix->device));
   return flat_batch_locked(ix, B, queries, k, n_filters, filter_ids, filter_offsets, query_filter, out_ids, out_dists,
                            out_counts);
+}
+
+int sdb_flat_search_batch_requests(sdb_index* ix, uint32_t B, const float* queries, const sdb_request* req,
+                                   uint32_t n_filters, const uint64_t* filter_ids, const uint64_t* filter_offsets,
+                                   uint32_t k_stride, uint64_t* out_ids, float* out_dists, uint32_t* out_counts) {
+  if (!ix) return fail(SDB_ERR_INVALID, "null index");
+  if (B == 0) return SDB_OK;
+  if (!queries || !out_ids || !out_dists || !out_counts) return fail(SDB_ERR_INVALID, "null argument");
+  std::lock_guard<std::mutex> g(ix->mu);
+  SDB_CUDA(cudaSetDevice(ix->device));
+  int rc = check_requests(ix, B, req, n_filters, k_stride, true);
+  if (rc) return rc;
+  FilterStage fs;
+  if ((rc = stage_filters(ix, B, n_filters, filter_ids, filter_offsets, nullptr, 0, true, &fs, req))) return rc;
+  if ((rc = ix->d_q.ensure(size_t(B) * ix->p.dim))) return rc;
+  if ((rc = ensure_out_scratch(ix, B, k_stride))) return rc;
+  SDB_CUDA(cudaMemcpyAsync(ix->d_q.p, queries, size_t(B) * ix->p.dim * sizeof(float), cudaMemcpyHostToDevice, ix->stream));
+  if ((rc = commit_filters(ix, &fs, ix->stream))) return rc;
+  if ((rc = flat_requests_locked(ix, B, ix->d_q.p, n_filters, fs, k_stride, ix->d_oid.p, ix->d_od.p, ix->d_oc.p, nullptr,
+                                 ix->stream)))
+    return rc;
+  const size_t n = size_t(B) * k_stride;
+  SDB_CUDA(cudaMemcpyAsync(out_ids, ix->d_oid.p, n * sizeof(uint64_t), cudaMemcpyDeviceToHost, ix->stream));
+  SDB_CUDA(cudaMemcpyAsync(out_dists, ix->d_od.p, n * sizeof(float), cudaMemcpyDeviceToHost, ix->stream));
+  SDB_CUDA(cudaMemcpyAsync(out_counts, ix->d_oc.p, size_t(B) * sizeof(uint32_t), cudaMemcpyDeviceToHost, ix->stream));
+  SDB_CUDA(cudaStreamSynchronize(ix->stream));
+  return flat_stats_settle(ix);
 }
 
 int sdb_flat_search_batch_device(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, uint64_t* d_out_ids,

@@ -216,6 +216,9 @@ struct SearchFilters {
   uint32_t n_filtered = 0;
   const uint32_t* qmap_plain = nullptr;
   uint32_t n_plain = 0;
+  // per-request parameters {L, k, gather count limit, 0} of a request batch (sdb_request), nullptr
+  // otherwise (SearchArgs::req)
+  const uint4* req = nullptr;
 };
 // the visited-table step-up of launch_search after a search that sent queries to the RETRY launch
 // (search.cu); reads the previous search's retry count only if its stream is idle
@@ -269,17 +272,23 @@ struct FilterStage {
   SearchFilters sf;
   const uint32_t* h_off = nullptr;
   uint32_t n_ids = 0, slot = 0;
-  size_t bytes = 0, ids_at = 0, off_at = 0, qf_at = 0, qmap_at = 0;  // bytes: of the slot (items excluded)
+  size_t bytes = 0, ids_at = 0, off_at = 0, qf_at = 0, qmap_at = 0, req_at = 0;  // bytes: of the slot (items excluded)
   bool shared_bits = false;  // one filter shared by the batch: build its row bitmap on the device
   bool per_request = false;  // query_filter given: per-query filter index and qmap staged
+  bool has_req = false;      // a request batch: per-request parameters staged at req_at
   bool is_flat = false;
   FlatFilterPlan flat;
 };
 // Host pass of a filtered call (index.cu): validates the filters (the error codes of the host filter
 // entries) and writes their device form into the next staging slot, nothing enqueued yet. flat: flat
 // search rules (no seeds, ids below 2 dropped, no shared bitmap) plus its work lists.
+// req (a request batch, already checked by check_requests; nullptr otherwise): the filter of request b
+// is req[b].filter, the seed check of a filter covers the largest search_size of its requests (L
+// and query_filter are ignored), n_filters may be 0, and the parameters are staged too.
 int stage_filters(sdb_index* ix, uint32_t B, uint32_t n_filters, const uint64_t* filter_ids, const uint64_t* filter_offsets,
-                  const int32_t* query_filter, uint32_t L, bool flat, FilterStage* out);
+                  const int32_t* query_filter, uint32_t L, bool flat, FilterStage* out, const sdb_request* req = nullptr);
+// limit / searchSize / stride checks of the request entries (flat: search_size ignored, no start node)
+int check_requests(sdb_index* ix, uint32_t B, const sdb_request* req, uint32_t n_filters, uint32_t k_stride, bool flat);
 // enqueues a staged call's copy on `stream` behind the previous filtered call's readers, and the
 // shared filter's bitmap; fills out->sf
 int commit_filters(sdb_index* ix, FilterStage* fs, cudaStream_t stream);
@@ -292,6 +301,12 @@ int check_search_args(sdb_index* ix, uint32_t k, uint32_t L);
 // the unfiltered requests to launch_flat.
 int launch_flat_filtered(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, const FilterStage& fs,
                          uint64_t* d_out_ids, float* d_out_dists, uint32_t* d_out_counts, cudaStream_t stream);
+// Flat search of a request batch staged and committed by stage_filters / commit_filters (req): the
+// batch runs at k_stride (filtered or not), then every row is cut to its request's limit and, with g,
+// published into the peers' gather buffers (search.cu)
+int flat_requests_locked(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t n_filters, const FilterStage& fs,
+                         uint32_t k_stride, uint64_t* d_out_ids, float* d_out_dists, uint32_t* d_out_counts,
+                         const PeerGather* g, cudaStream_t stream);
 // flat_filter.cu: score each work item's ids (x = batch row, [y, z) = range of d_ids) and merge a
 // request's items (d_req_items[r] .. d_req_items[r+1]) into output row d_req_rows[r]
 int launch_flat_gather(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k, const uint32_t* d_ids,
@@ -309,8 +324,9 @@ int launch_flat_tc(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k
                    uint32_t* d_out_counts, cudaStream_t stream);
 int launch_encode_rows(sdb_index* ix, uint32_t n, const uint32_t* d_ids, cudaStream_t stream);
 int launch_adc_tables(sdb_index* ix, uint32_t B, const float* d_queries, float* d_out, cudaStream_t stream);
+// limits: per-row output limit (device, <= k), nullptr = k for every row
 int launch_merge(uint32_t S, uint32_t B, uint32_t k, const uint64_t* in_ids, const float* in_d, const uint32_t* in_c,
-                 uint64_t* out_ids, float* out_d, uint32_t* out_c, cudaStream_t stream);
+                 uint64_t* out_ids, float* out_d, uint32_t* out_c, cudaStream_t stream, const uint32_t* limits = nullptr);
 // reinsert: ids already exist (update path, vamana.go:249-253): rows are overwritten, one point per mini-batch
 int insert_batch_locked(sdb_index* ix, uint64_t n, const uint64_t* ids, const float* vectors, bool reinsert = false,
                         bool vectors_on_device = false);

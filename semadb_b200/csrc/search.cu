@@ -89,6 +89,7 @@ int launch_search(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t k,
   a.B = B;
   a.L = L;
   a.k = k;
+  a.req = filters ? filters->req : nullptr;
   a.out_ids = d_out_ids;
   a.out_dists = d_out_dists;
   a.out_counts = d_out_counts;
@@ -206,6 +207,54 @@ static int launch_flat_publish(sdb_index* ix, const PeerGather& g, uint32_t B, u
   return SDB_OK;
 }
 
+// Request batches: the final lists of a flat search run at k_stride, cut to every request's limit.
+// One warp per request: slots past min(count, limit) get id 0 / +inf, the count is clamped, and
+// with peers every rank goes into slot [shard][q] of every peer's buffer with the bytes
+// flat_publish_kernel stores, the count clamped to the request's shard limit.
+__global__ void request_rows_kernel(PeerGather g, uint32_t B, uint32_t k, const uint4* req, uint64_t* ids, float* dists,
+                                    uint32_t* counts) {
+  const uint32_t q = (blockIdx.x * blockDim.x + threadIdx.x) / 32, lane = threadIdx.x & 31;
+  if (q >= B) return;
+  const uint4 r = req[q];
+  const uint32_t cnt = min(counts[q], r.y);
+  __syncwarp();
+  for (uint32_t j = lane; j < k; j += 32) {
+    const size_t t = size_t(q) * k + j;
+    const bool have = j < cnt;
+    if (!have) {
+      ids[t] = 0;
+      dists[t] = __int_as_float(0x7f800000);
+    }
+    if (g.n) {
+      const uint64_t id = have ? (ids[t] | g.tag) : 0;
+      const float d = have ? dists[t] : __int_as_float(0x7f800000);
+      const size_t o = (size_t(g.shard) * B + q) * k + j;
+      for (uint32_t s = 0; s < g.n; ++s) {
+        g.ids[s][o] = id;
+        g.dists[s][o] = d;
+      }
+    }
+  }
+  if (lane == 0) counts[q] = cnt;
+  if (lane < g.n) g.counts[lane][size_t(g.shard) * B + q] = min(cnt, r.z);
+}
+
+int flat_requests_locked(sdb_index* ix, uint32_t B, const float* d_queries, uint32_t n_filters, const FilterStage& fs,
+                         uint32_t k_stride, uint64_t* d_out_ids, float* d_out_dists, uint32_t* d_out_counts,
+                         const PeerGather* g, cudaStream_t stream) {
+  int rc = n_filters ? launch_flat_filtered(ix, B, d_queries, k_stride, fs, d_out_ids, d_out_dists, d_out_counts, stream)
+                     : flat_device_locked(ix, B, d_queries, k_stride, d_out_ids, d_out_dists, d_out_counts, stream);
+  if (!rc) {
+    const PeerGather none{};
+    request_rows_kernel<<<(B + 7) / 8, 256, 0, stream>>>(g ? *g : none, B, k_stride, fs.sf.req, d_out_ids, d_out_dists,
+                                                         d_out_counts);
+    ix->launches++;
+    if (cudaError_t e = cudaGetLastError(); e != cudaSuccess) rc = cuda_fail(e, "request_rows_kernel");
+  }
+  filters_done(ix, stream);  // the last reader of the staged parameters
+  return rc;
+}
+
 }  // namespace sdb
 
 using namespace sdb;
@@ -300,4 +349,51 @@ extern "C" int sdb_flat_search_batch_filters_device(sdb_index* ix, uint32_t B, c
   }
   if (rc || !peers) return rc;
   return launch_flat_publish(ix, g, B, k, d_out_ids, d_out_dists, d_out_counts, st);
+}
+
+extern "C" int sdb_search_batch_requests_device(sdb_index* ix, uint32_t B, const float* d_queries, const sdb_request* req,
+                                                uint32_t n_filters, const uint64_t* filter_ids, const uint64_t* filter_offsets,
+                                                uint32_t k_stride, uint64_t* d_out_ids, float* d_out_dists,
+                                                uint32_t* d_out_counts, const sdb_peer_gather* peers, void* stream) {
+  if (!ix) return fail(SDB_ERR_INVALID, "null index");
+  if (B == 0) return SDB_OK;
+  if (!d_queries || !d_out_ids || !d_out_dists || !d_out_counts) return fail(SDB_ERR_INVALID, "null argument");
+  std::lock_guard<std::mutex> lk(ix->mu);
+  SDB_CUDA(cudaSetDevice(ix->device));
+  int rc = check_requests(ix, B, req, n_filters, k_stride, false);
+  if (rc) return rc;
+  FilterStage fs;
+  if ((rc = stage_filters(ix, B, n_filters, filter_ids, filter_offsets, nullptr, 0, false, &fs, req))) return rc;
+  PeerGather g;
+  if (peers && ((rc = peer_gather_args(peers, k_stride, &g)) || (rc = peer_barrier_poisoned(ix->device)))) return rc;
+  const cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if ((rc = commit_filters(ix, &fs, st))) return rc;
+  ix->gather = peers ? &g : nullptr;  // the epilogue publishes every query's list, count clamped per request
+  rc = launch_search(ix, B, d_queries, k_stride, 75, d_out_ids, d_out_dists, d_out_counts, nullptr, nullptr, nullptr, 0, &fs.sf,
+                     st);
+  ix->gather = nullptr;
+  filters_done(ix, st);
+  return rc;
+}
+
+extern "C" int sdb_flat_search_batch_requests_device(sdb_index* ix, uint32_t B, const float* d_queries,
+                                                     const sdb_request* req, uint32_t n_filters, const uint64_t* filter_ids,
+                                                     const uint64_t* filter_offsets, uint32_t k_stride, uint64_t* d_out_ids,
+                                                     float* d_out_dists, uint32_t* d_out_counts, const sdb_peer_gather* peers,
+                                                     void* stream) {
+  if (!ix) return fail(SDB_ERR_INVALID, "null index");
+  if (B == 0) return SDB_OK;
+  if (!d_queries || !d_out_ids || !d_out_dists || !d_out_counts) return fail(SDB_ERR_INVALID, "null argument");
+  std::lock_guard<std::mutex> lk(ix->mu);
+  SDB_CUDA(cudaSetDevice(ix->device));
+  int rc = check_requests(ix, B, req, n_filters, k_stride, true);
+  if (rc) return rc;
+  FilterStage fs;
+  if ((rc = stage_filters(ix, B, n_filters, filter_ids, filter_offsets, nullptr, 0, true, &fs, req))) return rc;
+  PeerGather g;
+  if (peers && ((rc = peer_gather_args(peers, k_stride, &g)) || (rc = peer_barrier_poisoned(ix->device)))) return rc;
+  const cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if ((rc = commit_filters(ix, &fs, st))) return rc;
+  return flat_requests_locked(ix, B, d_queries, n_filters, fs, k_stride, d_out_ids, d_out_dists, d_out_counts,
+                              peers ? &g : nullptr, st);
 }

@@ -103,6 +103,10 @@ struct SearchArgs {
   uint32_t* work_counter;
   uint32_t* retry_list;
   uint32_t* retry_count;
+  // optional per-query parameters {L, k, gather count limit, 0} (sdb_request), read by the REQ
+  // variants only: nullptr = L, k and pg.limit for every query. With them, k is the stride of the
+  // outputs and of the gather slots.
+  const uint4* req;
 };
 
 // ---- exact visited set, compact form with a launch-time slot count ------------------------
@@ -1026,8 +1030,10 @@ __host__ __device__ constexpr size_t warp_smem_bytes(uint32_t qfloats, uint32_t 
 // SETS: FloatEvalFixed pipeline depth; MERGE_MIN > 0: use the batch form of AddWithLimit
 // (CandList::merge) when at least that many candidates survive.
 // XTRA: the start node has edges beyond R (a.start_extra) — compiled in only when it does.
+// REQ: per-query L / k / gather limit from a.req (request batches); false = the launch-wide values,
+// compiled without a trace of the per-query path.
 template <int KIND, int METRIC, int TRIPS, int SETS, int MERGE_MIN, class VT, bool FILTER, bool RETRY, int MINB,
-          bool XTRA, bool PF>
+          bool XTRA, bool PF, bool REQ>
 __global__ void __launch_bounds__(32, MINB) beam_search_kernel(SearchArgs a, uint32_t qfloats, uint32_t qwords) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int lane = threadIdx.x & 31;
@@ -1114,10 +1120,10 @@ __global__ void __launch_bounds__(32, MINB) beam_search_kernel(SearchArgs a, uin
     auto evaluate = [&](int n) { evaluate_h(n, no_hook); };
 
     list.len = 0;
-    list.cap = int(a.L);
+    list.cap = int(REQ ? __ldg(&a.req[qi].x) : a.L);
     list.nan_seen = false;
     res.len = 0;
-    res.cap = int(a.k);
+    res.cap = int(REQ ? __ldg(&a.req[qi].y) : a.k);
     res.nan_seen = false;
     uint32_t hops = 0, ndist = 0, nvisited = 0;
     bool overflow = false;
@@ -1157,7 +1163,8 @@ __global__ void __launch_bounds__(32, MINB) beam_search_kernel(SearchArgs a, uin
       return t0 + __popc(b1);
     };
 
-    // this query's filter: ascending ids fl[0..fn), the first min(fn, L) of them are the seeds
+    // this query's filter: ascending ids fl[0..fn), the first min(fn, L) of them are the seeds (L of
+    // this query: list.cap)
     const uint32_t* fl = nullptr;
     uint32_t fn = 0;
     if (FILTER) {
@@ -1169,7 +1176,7 @@ __global__ void __launch_bounds__(32, MINB) beam_search_kernel(SearchArgs a, uin
     if (FILTER) {
       // searchSet.Add(filterPoints...) (plain append, search.go:49) and
       // resultSet.AddWithLimit(filterPoints...) (search.go:50)
-      const int nf = int(min(fn, a.L));
+      const int nf = int(min(fn, REQ ? uint32_t(list.cap) : a.L));
       for (int b0 = 0; b0 < nf; b0 += CAND_SLOTS) {
         const int n = min(CAND_SLOTS, nf - b0);
         uint32_t i0 = lane < n ? __ldg(fl + b0 + lane) : 0;
@@ -1207,7 +1214,7 @@ __global__ void __launch_bounds__(32, MINB) beam_search_kernel(SearchArgs a, uin
     // one hop early; used if that candidate is indeed expanded next.
     uint32_t pf_id = INVALID_ID, pf_n0 = INVALID_ID, pf_n1 = INVALID_ID;
     for (; !overflow;) {
-      const int lim = min(list.len, int(a.L));
+      const int lim = min(list.len, REQ ? list.cap : int(a.L));
       int pos = -1, pos2 = -1, pos3 = -1;
 #pragma unroll
       for (int j = 0; j < 3; ++j) {
@@ -1326,7 +1333,7 @@ __global__ void __launch_bounds__(32, MINB) beam_search_kernel(SearchArgs a, uin
         if (in_filter) {
           // the seeds are already in resultSet (search.go:50): ascending list => e is a seed
           // iff it is not above the last seed
-          const uint32_t ns = min(fn, a.L);
+          const uint32_t ns = min(fn, REQ ? uint32_t(list.cap) : a.L);
           const bool seeded = ns > 0 && e <= __ldg(fl + ns - 1);
           if (!seeded) {
             if (lane == 0) { cid[0] = e; cdist[0] = edist; }
@@ -1347,6 +1354,8 @@ __global__ void __launch_bounds__(32, MINB) beam_search_kernel(SearchArgs a, uin
         if (!RETRY) a.retry_list[atomicAdd(a.retry_count, 1u)] = qi;
       }
     } else {
+      // this query's k; a.k is the row stride
+      const int qk = REQ ? res.cap : int(a.k);
       int written = 0;
 #pragma unroll
       for (int j = 0; j < 3; ++j) {
@@ -1355,7 +1364,7 @@ __global__ void __launch_bounds__(32, MINB) beam_search_kernel(SearchArgs a, uin
         bool keep = (p < out.len) && (nid != START_ID);
         uint32_t b = __ballot_sync(SDB_FULL, keep);
         int r = written + __popc(b & lt);
-        if (keep && r < int(a.k)) {
+        if (keep && r < qk) {
           const float dd = out.dist[p];
           a.out_ids[size_t(qi) * a.k + r] = uint64_t(nid);
           a.out_dists[size_t(qi) * a.k + r] = dd;
@@ -1369,7 +1378,7 @@ __global__ void __launch_bounds__(32, MINB) beam_search_kernel(SearchArgs a, uin
         }
         written += __popc(b);
       }
-      int cnt = min(written, int(a.k));
+      int cnt = min(written, qk);
       for (int r = cnt + lane; r < int(a.k); r += 32) {
         a.out_ids[size_t(qi) * a.k + r] = 0;
         a.out_dists[size_t(qi) * a.k + r] = __int_as_float(0x7f800000);
@@ -1381,7 +1390,10 @@ __global__ void __launch_bounds__(32, MINB) beam_search_kernel(SearchArgs a, uin
           }
         }
       }
-      if (a.pg.n && lane < int(a.pg.n)) a.pg.counts[lane][size_t(a.pg.shard) * a.B + qi] = uint32_t(min(cnt, int(a.pg.limit)));
+      if (a.pg.n && lane < int(a.pg.n)) {
+        const int plim = REQ ? int(__ldg(&a.req[qi].z)) : int(a.pg.limit);
+        a.pg.counts[lane][size_t(a.pg.shard) * a.B + qi] = uint32_t(min(cnt, plim));
+      }
       if (lane == 0) {
         a.out_counts[qi] = uint32_t(cnt);
         a.out_hops[qi] = hops;

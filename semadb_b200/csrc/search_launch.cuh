@@ -15,9 +15,9 @@ namespace sdb {
 namespace launch {
 
 template <int KIND, int METRIC, int TRIPS, int SETS, int MERGE_MIN, class VT, bool FILTER, bool RETRY, int MINB, bool XTRA,
-          bool PF = false>
+          bool PF, bool REQ>
 int launch_variant_x(sdb_index* ix, const SearchArgs& a, cudaStream_t stream) {
-  auto kern = beam_search_kernel<KIND, METRIC, TRIPS, SETS, MERGE_MIN, VT, FILTER, RETRY, MINB, XTRA, PF>;
+  auto kern = beam_search_kernel<KIND, METRIC, TRIPS, SETS, MERGE_MIN, VT, FILTER, RETRY, MINB, XTRA, PF, REQ>;
   // FloatEvalFixed keeps short queries (<= 4 float4 per lane) in registers: no shared copy
   constexpr bool QREG = (KIND == EVAL_FLOAT_FIXED) && TRIPS <= 4;
   const uint32_t qfloats = (KIND == EVAL_ADC || KIND == EVAL_ADC_SMEM || KIND == EVAL_BITS || KIND == EVAL_GEO || QREG) ? 0 : (a.dim + 3) / 4 * 4;
@@ -59,14 +59,22 @@ int launch_variant_x(sdb_index* ix, const SearchArgs& a, cudaStream_t stream) {
 
 // the start node's overflow edges (after deletes; normally none) get their own instantiation so
 // the common case pays nothing for them (the extra loop cost 5 % on C2)
-template <int KIND, int METRIC, int TRIPS, int SETS, int MERGE_MIN, class VT, bool FILTER, bool RETRY, int MINB>
-int launch_variant(sdb_index* ix, const SearchArgs& a, cudaStream_t stream) {
+template <int KIND, int METRIC, int TRIPS, int SETS, int MERGE_MIN, class VT, bool FILTER, bool RETRY, int MINB, bool REQ>
+int launch_variant_r(sdb_index* ix, const SearchArgs& a, cudaStream_t stream) {
   if (a.n_start_extra != 0)
-    return launch_variant_x<KIND, METRIC, TRIPS, SETS, MERGE_MIN, VT, FILTER, RETRY, MINB, true>(ix, a, stream);
+    return launch_variant_x<KIND, METRIC, TRIPS, SETS, MERGE_MIN, VT, FILTER, RETRY, MINB, true, false, REQ>(ix, a, stream);
   // speculative row prefetch (small-row evaluators, unfiltered first pass)
   // (PQ kernels: +1.6 %; bit rows: -1.6 %, the probes cost more than the L2 hits save — off there)
   constexpr bool PF = !FILTER && !RETRY && (KIND == EVAL_ADC_SMEM || KIND == EVAL_ADC || KIND == EVAL_ADC_FLY);
-  return launch_variant_x<KIND, METRIC, TRIPS, SETS, MERGE_MIN, VT, FILTER, RETRY, MINB, false, PF>(ix, a, stream);
+  return launch_variant_x<KIND, METRIC, TRIPS, SETS, MERGE_MIN, VT, FILTER, RETRY, MINB, false, PF, REQ>(ix, a, stream);
+}
+
+// request batches (per-query L / k, a.req) get instantiations of their own, so the kernels every other
+// entry launches are compiled exactly as without them
+template <int KIND, int METRIC, int TRIPS, int SETS, int MERGE_MIN, class VT, bool FILTER, bool RETRY, int MINB>
+int launch_variant(sdb_index* ix, const SearchArgs& a, cudaStream_t stream) {
+  if (a.req != nullptr) return launch_variant_r<KIND, METRIC, TRIPS, SETS, MERGE_MIN, VT, FILTER, RETRY, MINB, true>(ix, a, stream);
+  return launch_variant_r<KIND, METRIC, TRIPS, SETS, MERGE_MIN, VT, FILTER, RETRY, MINB, false>(ix, a, stream);
 }
 
 template <int KIND, int METRIC, int TRIPS, int SETS, int MERGE_MIN, bool FILTER, int MINB>

@@ -2,8 +2,8 @@
 // IndexVamana.Search with ONE vector under a read lock: shard/index/search.go:67-85,
 // shard/cache/manager.go:151-182) into the batches the GPU kernels need (SURVEY.md §8f-1).
 // Callers block in Search(); a single batcher thread collects requests until `max_batch` are
-// waiting or the oldest has waited `window`, runs one sdb_search_batch for all requests that
-// share (limit, searchSize) — each with its own optional filter bitmap, like
+// waiting or the oldest has waited `window`, runs one sdb_search_batch_requests for all of them —
+// each with its own limit, searchSize (models/search.go:268-314) and optional filter bitmap, like
 // shard/index/search.go:59-85 — and hands every caller its own slice of the result.
 #pragma once
 #include <chrono>
@@ -42,6 +42,8 @@ class SearchCoalescer {
                std::vector<uint64_t>* result_set, std::vector<models::SearchResult>* results) {
     if (query.Vector.size() != ix_->Parameters().VectorSize)
       return Error("could not perform graph search: query vector length mismatch");
+    // an invalid request fails alone, before it can fail the batch it would have joined
+    if (Error e = query.Validate()) return e;
     Request r;
     r.q = &query;
     r.filter = filter;
@@ -87,7 +89,7 @@ class SearchCoalescer {
     std::vector<float> qbuf;
     std::vector<uint64_t> ids;
     std::vector<float> dists;
-    std::vector<uint32_t> counts;
+    std::vector<uint32_t> counts, limits, sizes;
     std::unique_lock<std::mutex> g(mu_);
     for (;;) {
       cv_.wait(g, [&] { return stop_ || !queue_.empty(); });
@@ -98,22 +100,24 @@ class SearchCoalescer {
       // let the batch fill up, but never hold the oldest request longer than `window`
       const auto deadline = std::chrono::steady_clock::now() + window_;
       cv_.wait_until(g, deadline, [&] { return stop_ || queue_.size() >= max_batch_; });
-      // take every waiting request that shares the head's (limit, searchSize)
-      const int k = queue_.front()->q->Limit, L = queue_.front()->q->SearchSize;
+      // take the waiting requests in arrival order, whatever their (limit, searchSize)
       std::vector<Request*> batch;
-      for (auto it = queue_.begin(); it != queue_.end() && batch.size() < max_batch_;) {
-        if ((*it)->q->Limit == k && (*it)->q->SearchSize == L) {
-          batch.push_back(*it);
-          it = queue_.erase(it);
-        } else {
-          ++it;
-        }
+      while (!queue_.empty() && batch.size() < max_batch_) {
+        batch.push_back(queue_.front());
+        queue_.pop_front();
       }
       g.unlock();
       const uint32_t B = uint32_t(batch.size());
       qbuf.resize(size_t(B) * dim);
-      for (uint32_t b = 0; b < B; ++b) std::copy(batch[b]->q->Vector.begin(), batch[b]->q->Vector.end(), qbuf.begin() + size_t(b) * dim);
-      const uint32_t kk = uint32_t(k > 0 ? k : 1);
+      limits.resize(B);
+      sizes.resize(B);
+      uint32_t kk = 1;  // row stride: the largest limit of the batch
+      for (uint32_t b = 0; b < B; ++b) {
+        std::copy(batch[b]->q->Vector.begin(), batch[b]->q->Vector.end(), qbuf.begin() + size_t(b) * dim);
+        limits[b] = uint32_t(batch[b]->q->Limit);
+        sizes[b] = uint32_t(batch[b]->q->SearchSize);
+        kk = std::max(kk, limits[b]);
+      }
       ids.assign(size_t(B) * kk, 0);
       dists.assign(size_t(B) * kk, 0.0f);
       counts.assign(B, 0);
@@ -123,17 +127,17 @@ class SearchCoalescer {
         filters[b] = batch[b]->filter;
         any_filter |= batch[b]->filter != nullptr;
       }
+      if (!any_filter) filters.clear();
       std::vector<Error> errs(B);
-      Error err = any_filter ? ix_->SearchBatchFilters(qbuf.data(), B, uint32_t(k), uint32_t(L), filters, ids.data(),
-                                                       dists.data(), counts.data())
-                             : ix_->SearchBatch(qbuf.data(), B, uint32_t(k), uint32_t(L), ids.data(), dists.data(), counts.data());
+      Error err = ix_->SearchBatchRequests(qbuf.data(), B, limits.data(), sizes.data(), filters, kk, ids.data(), dists.data(),
+                                           counts.data());
       if (err && any_filter && B > 1) {
         // a request whose filter names a missing point fails alone in the reference (search.go:45-48):
         // re-run the batch request by request so only the offender gets the error
         for (uint32_t b = 0; b < B; ++b) {
           std::vector<const std::vector<uint64_t>*> one(1, filters[b]);
-          errs[b] = ix_->SearchBatchFilters(qbuf.data() + size_t(b) * dim, 1, uint32_t(k), uint32_t(L), one,
-                                            ids.data() + size_t(b) * kk, dists.data() + size_t(b) * kk, counts.data() + b);
+          errs[b] = ix_->SearchBatchRequests(qbuf.data() + size_t(b) * dim, 1, &limits[b], &sizes[b], one, limits[b],
+                                             ids.data() + size_t(b) * kk, dists.data() + size_t(b) * kk, counts.data() + b);
         }
       } else {
         for (uint32_t b = 0; b < B; ++b) errs[b] = err;

@@ -203,6 +203,33 @@ class IndexVamana {
                 "could not perform graph search");
   }
 
+  // B requests, each with its own limit and searchSize (models/search.go:268-314) and optional filter
+  // (filters empty = nobody is filtered; else one slot per request as in SearchBatchFilters), in one
+  // call: outputs B x k_stride, row b holds out_counts[b] <= limits[b] results and equals the request
+  // served alone.
+  Error SearchBatchRequests(const float* queries, uint32_t B, const uint32_t* limits, const uint32_t* search_sizes,
+                            const std::vector<const std::vector<uint64_t>*>& filters, uint32_t k_stride, uint64_t* out_ids,
+                            float* out_dists, uint32_t* out_counts) {
+    if (!filters.empty() && filters.size() != B)
+      return Error("could not perform graph search: one filter slot per request expected");
+    std::vector<uint64_t> flat, off(1, 0), f;
+    std::vector<sdb_request> req(B);
+    for (uint32_t b = 0; b < B; ++b) {
+      req[b] = sdb_request{limits[b], search_sizes[b], 0, -1};
+      if (filters.empty() || !filters[b]) continue;
+      f = *filters[b];
+      std::sort(f.begin(), f.end());
+      f.erase(std::unique(f.begin(), f.end()), f.end());
+      req[b].filter = int32_t(off.size() - 1);
+      flat.insert(flat.end(), f.begin(), f.end());
+      off.push_back(flat.size());
+    }
+    const uint32_t nf = uint32_t(off.size() - 1);
+    return CErr(sdb_search_batch_requests(h_, B, queries, req.data(), nf, flat.data(), off.data(), k_stride, out_ids,
+                                          out_dists, out_counts),
+                "could not perform graph search");
+  }
+
   // flush (vamana.go:265-276): vecStore.Flush, nodeStore.Flush, MAXNODEIDKEY.
   Error Flush() {
     if (bucket_ == nullptr || bucket_->IsReadOnly()) return Ok();

@@ -182,12 +182,46 @@ class ShardedSearcher:
                       torch.zeros((B, k), dtype=torch.float32, device=device),
                       torch.zeros((B,), dtype=torch.int32, device=device))
 
-    def _search_shard(self, q, k: int, search_size, l_ids, l_d, l_c, stream, pg=None, filters=None, query_filter=None):
+    def _requests(self, B: int, k: int, limits, search_sizes, filters, query_filter, max_search_limit: int, dev):
+        """Per-request parameters of a step with `limits`: (PackedRequests, device limits for the
+        merge, device shard limits), or None without them. Each request publishes
+        sdb_shard_limit(limit_b, S, max_search_limit) ranks; k is the row stride."""
+        if limits is None:
+            return None
+        import torch
+        from .vamana import PackedRequests
+        lim = np.broadcast_to(np.asarray(limits, dtype=np.int64), (B,))
+        if B and int(lim.max()) > k:
+            raise _capi.SdbError(_capi.ERR_INVALID, "limits must not exceed k, the row stride")
+        shard = np.array([shard_limit(int(x), self.world, max_search_limit) for x in lim], dtype=np.int64)
+        rq = PackedRequests(B, lim, search_sizes, filters, query_filter, shard, default_L=self.index.L)
+        # page-locked, copied without blocking the host: a pipelined step does not wait for the last one
+        d_lim = torch.from_numpy(lim.astype(np.int32)).pin_memory().to(dev, non_blocking=True)
+        d_shard = torch.from_numpy(np.minimum(shard, lim).astype(np.int32)).pin_memory().to(dev, non_blocking=True)
+        return rq, d_lim, d_shard
+
+    def _merge(self, di: int, B: int, k: int, g_i, g_d, g_c, o_ids, o_d, o_c, stream, rq=None):
+        """K6 over the gathered shard lists: per-request output limits when the step has them."""
+        lib = _capi.lib()
+        outs = (o_ids.data_ptr(), o_d.data_ptr(), o_c.data_ptr())
+        if rq is None:
+            _capi.check(lib.sdb_merge_topk_device(di, self.world, B, k, g_i, g_d, g_c, *outs, stream))
+        else:
+            _capi.check(lib.sdb_merge_topk_requests_device(di, self.world, B, k, rq[1].data_ptr(), g_i, g_d, g_c, *outs,
+                                                           stream))
+
+    def _search_shard(self, q, k: int, search_size, l_ids, l_d, l_c, stream, pg=None, filters=None, query_filter=None,
+                      rq=None):
         """This rank's shard search of the [B, dim] query tensor q (device or page-locked) into l_*
         and, with pg, into slot [rank] of every peer's gather buffer: the flat entries for an
-        IndexFlat, the beam-search entries otherwise, their filtered forms when `filters` is given.
+        IndexFlat, the beam-search entries otherwise, their filtered forms when `filters` is given,
+        their request forms when the step has per-request parameters (rq, from _requests).
         Enqueued on `stream`, no synchronisation."""
         B = int(q.shape[0])
+        if rq is not None:
+            entry = self.index.flat_search_batch_requests_device if self._flat else self.index.search_batch_requests_device
+            entry(q, rq[0], k, l_ids, l_d, l_c, stream, pg)
+            return
         L = None if self._flat else (self.index.L if search_size is None else int(search_size))
         if filters is not None:
             if self._flat:
@@ -210,13 +244,13 @@ class ShardedSearcher:
         _capi.check(rc)
 
     def search_batch_pinned(self, h_queries, k: int, search_size: Optional[int], h_ids, h_dists, h_counts, device,
-                            max_search_limit: int = 75, filters=None, query_filter=None):
+                            max_search_limit: int = 75, filters=None, query_filter=None, limits=None, search_sizes=None):
         """Host-facing twin of search_batch_device for page-locked (pinned) torch CPU tensors:
         pinned memory is mapped into the device address space, so K1 reads the broadcast query
         batch straight from host memory (no staging copy in front of the kernel); the merged
         lists come back with one small copy. Falls back to explicit copies when the fused
-        exchange is not active. Synchronises before returning. filters / query_filter: as in
-        search_batch_device."""
+        exchange is not active. Synchronises before returning. filters / query_filter, limits /
+        search_sizes: as in search_batch_device."""
         import torch
         B = int(h_queries.shape[0])
         stream = torch.cuda.current_stream(device).cuda_stream
@@ -225,7 +259,7 @@ class ShardedSearcher:
             h_dists.is_pinned() and h_counts.is_pinned()
         if not fused:
             r_ids, r_d, r_c = self.search_batch_device(h_queries.to(device, non_blocking=True), k, search_size,
-                                                       max_search_limit, filters, query_filter)
+                                                       max_search_limit, filters, query_filter, limits, search_sizes)
             h_ids.copy_(r_ids, non_blocking=True)
             h_dists.copy_(r_d, non_blocking=True)
             h_counts.copy_(r_c, non_blocking=True)
@@ -240,15 +274,15 @@ class ShardedSearcher:
         pg.per_shard_limit = shard_limit(k, self.world, max_search_limit)
         lib = _capi.lib()
         di = device.index or 0
-        self._search_shard(h_queries, k, search_size, l_ids, l_d, l_c, stream, pg, filters, query_filter)
+        rq = self._requests(B, k, limits, search_sizes, filters, query_filter, max_search_limit, device)
+        self._search_shard(h_queries, k, search_size, l_ids, l_d, l_c, stream, pg, filters, query_filter, rq)
         _capi.check(lib.sdb_peer_barrier_device(di, self.world, self.rank, pb._flags, pb.epoch, stream))
         g_i, g_dd, g_cc = pb.local(par)
         # The merge is a short kernel: its 300 k small stores would sit exposed on PCIe if they went
         # to mapped host memory (measured: +0.3 ms per step at B = 10 k), so it writes device buffers
         # and one 1.24 MB copy brings the lists back. K1's query reads stay zero-copy.
         m_ids, m_d, m_c = self._bufs[3], self._bufs[4], self._bufs[5]
-        _capi.check(lib.sdb_merge_topk_device(di, self.world, B, k, g_i, g_dd, g_cc, m_ids.data_ptr(), m_d.data_ptr(),
-                                              m_c.data_ptr(), stream))
+        self._merge(di, B, k, g_i, g_dd, g_cc, m_ids, m_d, m_c, stream, rq)
         h_ids.copy_(m_ids, non_blocking=True)
         h_dists.copy_(m_d, non_blocking=True)
         h_counts.copy_(m_c, non_blocking=True)
@@ -257,7 +291,7 @@ class ShardedSearcher:
         _capi.check(lib.sdb_peer_barrier_check(di, 0))
 
     def search_batch_device(self, d_queries, k: int, search_size: Optional[int], max_search_limit: int = 75,
-                            filters=None, query_filter=None):
+                            filters=None, query_filter=None, limits=None, search_sizes=None):
         """d_queries: [B, dim] f32 CUDA tensor, identical on every rank (broadcast by the
         caller). Returns merged (global ids [B,k] int64, dists [B,k], counts [B]) on every rank.
         search_size: the beam width of a Vamana shard (None = the index's); unused for a flat one.
@@ -277,11 +311,20 @@ class ShardedSearcher:
         exchange calls fail with SDB_ERR_STATE until sdb_peer_barrier_check(clear) (semadb_b200.h).
         The epoch has advanced on every rank, so the ranks stay in step once cleared. Callers that
         cannot rule such errors out check each rank's lists first (the host filter entries apply the
-        same checks)."""
+        same checks).
+
+        limits / search_sizes: every request's own limit and searchSize (models/search.go:268-314),
+        one value per request or one for all (search_sizes None: search_size, else the index's). k is
+        then the row stride of the results and must be at least every limit; row b holds at most
+        limits[b] results, each shard contributing sdb_shard_limit(limits[b], S, max_search_limit)
+        of them, and is padded with id 0 / +inf. The limits are the same on every rank."""
         import torch
         B = int(d_queries.shape[0])
         dev = d_queries.device
+        if limits is not None and search_sizes is None and search_size is not None:
+            search_sizes = search_size
         self._ensure(B, k, dev)
+        rq = self._requests(B, k, limits, search_sizes, filters, query_filter, max_search_limit, dev)
         l_ids, l_d, l_c, m_ids, m_d, m_c = self._bufs
         stream = torch.cuda.current_stream(dev).cuda_stream
         # the reference asks each shard for min(k, floor(k/S*1.42+10)) results; the local
@@ -307,11 +350,10 @@ class ShardedSearcher:
                 par = pb.epoch % pb.NBUF
                 pg = pb._pg[par]
                 pg.per_shard_limit = per_shard
-                self._search_shard(d_queries, k, search_size, l_ids, l_d, l_c, stream, pg, filters, query_filter)
+                self._search_shard(d_queries, k, search_size, l_ids, l_d, l_c, stream, pg, filters, query_filter, rq)
                 _capi.check(lib.sdb_peer_barrier_device(di, self.world, self.rank, pb._flags, pb.epoch, stream))
                 g_i, g_dd, g_cc = pb.local(par)
-                _capi.check(lib.sdb_merge_topk_device(di, self.world, B, k, g_i, g_dd, g_cc, m_ids.data_ptr(),
-                                                      m_d.data_ptr(), m_c.data_ptr(), stream))
+                self._merge(di, B, k, g_i, g_dd, g_cc, m_ids, m_d, m_c, stream, rq)
                 return m_ids, m_d, m_c
             # Pipelined steps: the search of step e runs on the caller's stream; its barrier and merge
             # run on a side stream, so the search of step e+1 starts without waiting for the slowest
@@ -330,26 +372,28 @@ class ShardedSearcher:
                 main.wait_event(self._bar_done[(e - 2) % pb.NBUF])
             pg = pb._pg[par]
             pg.per_shard_limit = per_shard
-            self._search_shard(d_queries, k, search_size, l_ids, l_d, l_c, main.cuda_stream, pg, filters, query_filter)
+            self._search_shard(d_queries, k, search_size, l_ids, l_d, l_c, main.cuda_stream, pg, filters, query_filter, rq)
             self._k1_done.record(main)
             side.wait_event(self._k1_done)
             o_ids, o_d, o_c = self._pipe_out[par]
             _capi.check(lib.sdb_peer_barrier_device(di, self.world, self.rank, pb._flags, e, side.cuda_stream))
             self._bar_done[par].record(side)
             g_i, g_dd, g_cc = pb.local(par)
-            _capi.check(lib.sdb_merge_topk_device(di, self.world, B, k, g_i, g_dd, g_cc, o_ids.data_ptr(),
-                                                  o_d.data_ptr(), o_c.data_ptr(), side.cuda_stream))
+            if rq is not None:  # the side stream reads the step's limits: keep them alive until it has
+                self._pipe_rq = getattr(self, "_pipe_rq", [None] * pb.NBUF)
+                self._pipe_rq[par] = rq
+            self._merge(di, B, k, g_i, g_dd, g_cc, o_ids, o_d, o_c, side.cuda_stream, rq)
             self._pending = True
             return o_ids, o_d, o_c
-        self._search_shard(d_queries, k, search_size, l_ids, l_d, l_c, stream, None, filters, query_filter)
-        if per_shard < k:
+        self._search_shard(d_queries, k, search_size, l_ids, l_d, l_c, stream, None, filters, query_filter, rq)
+        if rq is not None:
+            torch.minimum(l_c, rq[2], out=l_c)
+        elif per_shard < k:
             l_c.clamp_(max=per_shard)
         if self.world == 1:
             return l_ids, l_d, l_c
         g_ids, g_d, g_c = exchange_topk(pack_global_ids(l_ids, self.rank), l_d, l_c, self.group)
-        _capi.check(_capi.lib().sdb_merge_topk_device(dev.index or 0, self.world, B, k, g_ids.data_ptr(),
-                                                      g_d.data_ptr(), g_c.data_ptr(), m_ids.data_ptr(),
-                                                      m_d.data_ptr(), m_c.data_ptr(), stream))
+        self._merge(dev.index or 0, B, k, g_ids.data_ptr(), g_d.data_ptr(), g_c.data_ptr(), m_ids, m_d, m_c, stream, rq)
         return m_ids, m_d, m_c
 
 

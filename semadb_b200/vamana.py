@@ -177,6 +177,42 @@ class PackedFilters:
                 None if self.qf is None else _ptr(self.qf, _capi.i32p))
 
 
+_REQUEST_DTYPE = np.dtype([("limit", "<u4"), ("search_size", "<u4"), ("shard_limit", "<u4"), ("filter", "<i4")])
+
+
+class PackedRequests:
+    """Per-request parameters in the C form of sdb_search_batch_requests: an array of sdb_request
+    (limit, search_size, shard_limit, filter) and the filters they index. limits, search_sizes and
+    shard_limits are one value per request or one for all (search_sizes None: default_L;
+    shard_limits None: 0 = the limit); filters / query_filter as in PackedFilters (filters None:
+    nobody is filtered)."""
+
+    def __init__(self, B: int, limits, search_sizes=None, filters=None, query_filter=None, shard_limits=None,
+                 default_L: int = 75):
+        def col(v):
+            return np.broadcast_to(np.asarray(v, dtype=np.int64), (B,)).astype(np.uint32)
+        self.req = np.zeros(B, dtype=_REQUEST_DTYPE)
+        self.req["limit"] = col(limits)
+        self.req["search_size"] = col(default_L if search_sizes is None else search_sizes)
+        self.req["shard_limit"] = col(0 if shard_limits is None else shard_limits)
+        self.filters = None if filters is None else PackedFilters.of(filters, query_filter)
+        if self.filters is None:
+            self.req["filter"] = -1
+        else:
+            # query_filter < 0 = unfiltered, as in the filter entries; sdb_request spells that -1
+            self.req["filter"] = 0 if self.filters.qf is None else np.maximum(self.filters.qf, -1)
+        self.B = B
+        self.k_max = int(self.req["limit"].max()) if B else 1
+
+    def args(self):
+        """(req, n_filters, filter_ids, filter_offsets) as ctypes arguments."""
+        r = self.req.ctypes.data_as(C.POINTER(_capi.SdbRequest))
+        if self.filters is None:
+            return r, 0, None, None
+        n, ids, off, _ = self.filters.args()
+        return r, n, ids, off
+
+
 class _DeviceIndex:
     """Owns an sdb_index handle; shared by IndexVamana and IndexFlat."""
 
@@ -371,6 +407,53 @@ class _DeviceIndex:
         check(self._lib.sdb_search_batch_filters_device(
             self._h, int(d_queries.shape[0]), d_queries.data_ptr(), k, search_size, *f.args(), d_out_ids.data_ptr(),
             d_out_dists.data_ptr(), d_out_counts.data_ptr(), None if peers is None else C.byref(peers), stream))
+
+    def _request_batch(self, queries, limits, search_sizes, filters, query_filter, k_stride):
+        q = _f32(queries)
+        if q.ndim != 2 or q.shape[1] != self.dim:
+            raise SdbError(_capi.ERR_INVALID, "queries must be [B, dim]")
+        r = PackedRequests(q.shape[0], limits, search_sizes, filters, query_filter, default_L=self.L)
+        k = r.k_max if k_stride is None else int(k_stride)
+        out = (np.zeros((q.shape[0], k), dtype=np.uint64), np.zeros((q.shape[0], k), dtype=np.float32),
+               np.zeros(q.shape[0], dtype=np.uint32))
+        return q, r, k, out
+
+    def search_batch_requests(self, queries, limits, search_sizes=None, filters=None, query_filter=None, k_stride=None):
+        """Every request with its own limit and searchSize (models/search.go:268-314) and, optionally,
+        its own filter (filters / query_filter as in search_batch_filters). Returns (ids [B, k_stride],
+        dists, counts), k_stride = the largest limit by default: row b equals search_batch_filters of
+        request b alone at its limit and searchSize, padded with id 0 / +inf."""
+        q, r, k, (ids, d, cnt) = self._request_batch(queries, limits, search_sizes, filters, query_filter, k_stride)
+        check(self._lib.sdb_search_batch_requests(self._h, q.shape[0], _ptr(q, f32p), *r.args(), k, _ptr(ids, u64p),
+                                                  _ptr(d, f32p), _ptr(cnt, u32p)))
+        return ids, d, cnt
+
+    def flat_search_batch_requests(self, queries, limits, filters=None, query_filter=None, k_stride=None):
+        """Flat twin of search_batch_requests: row b equals flat_search_batch_filters of request b
+        alone at its limit, padded with id 0 / +inf."""
+        q, r, k, (ids, d, cnt) = self._request_batch(queries, limits, None, filters, query_filter, k_stride)
+        check(self._lib.sdb_flat_search_batch_requests(self._h, q.shape[0], _ptr(q, f32p), *r.args(), k,
+                                                       _ptr(ids, u64p), _ptr(d, f32p), _ptr(cnt, u32p)))
+        return ids, d, cnt
+
+    def search_batch_requests_device(self, d_queries, requests, k_stride: int, d_out_ids, d_out_dists, d_out_counts,
+                                     stream: int = 0, peers=None):
+        """Device twin of search_batch_requests (sdb_search_batch_requests_device): `requests` is a
+        PackedRequests, host-side and copied before the call returns; outputs [B, k_stride]. peers (an
+        SdbPeerGather) also stores every request's list into slot [shard][query] of every peer's
+        gather buffer, its count clamped to the request's shard limit. Enqueues on `stream`."""
+        check(self._lib.sdb_search_batch_requests_device(
+            self._h, int(d_queries.shape[0]), d_queries.data_ptr(), *requests.args(), int(k_stride),
+            d_out_ids.data_ptr(), d_out_dists.data_ptr(), d_out_counts.data_ptr(),
+            None if peers is None else C.byref(peers), stream))
+
+    def flat_search_batch_requests_device(self, d_queries, requests, k_stride: int, d_out_ids, d_out_dists,
+                                          d_out_counts, stream: int = 0, peers=None):
+        """Flat twin of search_batch_requests_device (sdb_flat_search_batch_requests_device)."""
+        check(self._lib.sdb_flat_search_batch_requests_device(
+            self._h, int(d_queries.shape[0]), d_queries.data_ptr(), *requests.args(), int(k_stride),
+            d_out_ids.data_ptr(), d_out_dists.data_ptr(), d_out_counts.data_ptr(),
+            None if peers is None else C.byref(peers), stream))
 
     def last_search_stats(self, B: int):
         hops = np.zeros(B, dtype=np.uint32)
